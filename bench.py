@@ -61,7 +61,16 @@ def parse():
     ap.add_argument("--concurrent-folds", type=int, default=4, help="loso: folds interleaved per GPU on separate CUDA streams (1 = one after another)")
     ap.add_argument("--subjects", type=int, default=15, help="loso / preprocess: number of synthetic subjects")
     ap.add_argument("--minutes", type=float, default=100.0, help="loso / preprocess: recording length (100 = 4.2 M chest samples)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of the train_step workload (--impl ours, the headline path; no other workload "
+                         "takes it), write what the last of them returned (loss, logits, gradient, updated state_dict) as "
+                         "DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "train_step" or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the train_step workload of --impl ours")
+    return args
 
 
 def peaks():
@@ -149,9 +158,10 @@ class _ReferenceStep:
         return loss.item()                                                                                 # trainer.py:152
 
 
-def cpu_reference_run(args, steps, warmup, budget_s):
-    """Time the reference's CPU training step (bounded by ``budget_s`` seconds of CPU work): the unmodified reference
-    ``models.py`` when it is present (kind "reference"), else oracle/cpu_port.py (kind "port")."""
+def cpu_reference_run(args, steps, warmup, budget_s=None):
+    """Time the reference's CPU training step: the unmodified reference ``models.py`` when it is present (kind
+    "reference"), else oracle/cpu_port.py (kind "port").  ``steps`` timed steps after ``warmup`` (the first included),
+    or, with ``budget_s``, as many of them as fit in about that many seconds of CPU work."""
     import torch
     from oracle import ref_harness
     threads = os.cpu_count() or 1
@@ -173,10 +183,10 @@ def cpu_reference_run(args, steps, warmup, budget_s):
     t0 = time.perf_counter()
     step(x, y)
     first = time.perf_counter() - t0
-    warm = max(0, min(warmup - 1, int(0.25 * budget_s / max(first, 1e-3))))
+    warm = max(0, warmup - 1 if budget_s is None else min(warmup - 1, int(0.25 * budget_s / max(first, 1e-3))))
     for _ in range(warm):
         step(x, y)
-    n = max(1, min(steps, int(budget_s / max(first, 1e-3))))
+    n = steps if budget_s is None else max(1, min(steps, int(budget_s / max(first, 1e-3))))
     t0 = time.perf_counter()
     for _ in range(n):
         step(x, y)
@@ -253,7 +263,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    r = cpu_reference_run(args, args.steps, args.warmup, budget_s=60.0)
+    r = cpu_reference_run(args, args.steps, args.warmup)
     line = {"impl": "reference", "metric": "train windows/sec (fwd+bwd+Adam) CnnGruAttention", "value": r["value"],
             "unit": "windows/s", "n_gpus": args.gpus, "steps": r["timed_steps"], "requested_steps": args.steps,
             "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak",
@@ -330,6 +340,8 @@ def run_ours(args):
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_total = float(ms.item())
     loss_after = step.last_loss()
+    if args.dump_outputs:                                 # before the e2e loop below trains the same model further
+        dump_outputs(Path(args.dump_outputs), step, model, f"rank{rank}_" if world > 1 else "")
 
     # ---- e2e: pinned host batch -> H2D -> step -> loss.item() every step ----------------------
     # warm-up of THIS path (copy stream, pinned loss ring, prefetch pipeline): the same loop, untimed
@@ -540,6 +552,19 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, step, model, prefix=""):
+    """What a caller of the fused training step holds after its last call: the loss, the logits, the flat gradient and
+    every state_dict entry (updated parameters, BatchNorm statistics), as float32 (integers as float64).  Independent of
+    T, and of B apart from the logits: about 1 MB at the default configuration."""
+    import numpy as np
+    out_dir.mkdir(parents=True, exist_ok=True)
+    arrays = {"loss": step.loss, "logits": step.logits, "grads": step.opt.grads}
+    arrays.update({f"state.{k}": v for k, v in model.state_dict().items()})
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        np.save(out_dir / f"{prefix}{name}.npy", a.astype(np.float32 if a.dtype.kind == "f" else np.float64))
+
+
 def model_seq_len(T):
     l1 = (T + 6 - 7) // 2 + 1
     p1 = (l1 - 1) // 2 + 1
@@ -603,7 +628,7 @@ def preprocess_measure(args, subjects=None):
     time.sleep(0.4)                                                     # nvidia-smi's start-up (NVML initialisation) stalls launches: keep it out of
     l0 = lib.mms_launch_count()                                         # a region that is ~100 host-enqueued launches per subject
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    reps = max(1, args.steps if args.steps < 50 else 20)      # 15 subjects per pass, ~26 ms per pass
+    reps = args.steps                                                   # 15 subjects per pass, ~26 ms per pass
     e0.record()
     nwin = 0
     for _ in range(reps):

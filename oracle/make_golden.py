@@ -21,7 +21,7 @@ import torch
 ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
 
-from oracle import ref_harness  # noqa: E402
+from oracle import golden_inputs as gi, ref_harness  # noqa: E402
 from multimodalsignal_b200 import synth  # noqa: E402
 
 GOLDEN = ROOT / "tests" / "golden"
@@ -48,6 +48,35 @@ MODEL_CASES = {
 }
 
 
+def _keep(out, name, a):
+    """Output ``name`` in full or, when it is large, the fixed seeded subset of its elements (flat indices under
+    ``idx/<key>``).  A gradient also keeps its largest magnitude: the scale of the tests' tolerance."""
+    a = np.asarray(a)
+    key = name.split("/", 1)[1]
+    if name.startswith("grad/"):
+        out[f"absmax/{name}"] = np.float32(np.abs(a).max() if a.size else 0.0)
+    idx = gi.subset_indices(key, a.size)
+    if idx is None:
+        out[name] = a
+    else:
+        out[f"idx/{key}"] = idx
+        out[name] = a.reshape(-1)[idx]
+
+
+def pack_model_case(meta, x, y, sd, outputs):
+    """A model fixture: the reference's outputs (gradients and post-Adam weights subset by ``_keep``) and the digests of
+    the inputs it ran on, which tests/conftest.py rebuilds from the seeds (oracle/golden_inputs.py)."""
+    digests = {"x": gi.digest(x), "y": gi.digest(y), **{f"sd/{k}": gi.digest(v) for k, v in sd.items()}}
+    out = {}
+    for k, v in outputs.items():
+        if k.startswith(("grad/", "sd_adam/")):
+            _keep(out, k, v)
+        else:
+            out[k] = v
+    out["meta"] = np.frombuffer(json.dumps(dict(meta, inputs="model_case", input_sha256=digests)).encode(), dtype=np.uint8)
+    return out
+
+
 def make_model_case(name, C, nc, B, T, kwargs, adam_steps):
     ref_models = ref_harness.load("models")
     torch.manual_seed(1234 + C)
@@ -56,16 +85,11 @@ def make_model_case(name, C, nc, B, T, kwargs, adam_steps):
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
         model = ref_models.CnnGruAttentionModel(in_channels=C, num_classes=nc, dropout=0.0, **kwargs)
-    # move BN affine params / biases off their trivial init so the test has teeth
-    with torch.no_grad():
-        for k, v in model.named_parameters():
-            if "cnn_encoder.1" in k or "cnn_encoder.5" in k:
-                v.add_(0.1 * torch.randn_like(v))
-    x, y = synth.synthetic_windows(B, C, T, seed=C * 100 + B, num_classes=nc)
+    gi.perturb_batchnorm(model)
+    x, y = gi.model_windows(C, nc, B, T)
     xt, yt = torch.from_numpy(x), torch.from_numpy(y)
-    out = {"x": x, "y": y}
-    for k, v in model.state_dict().items():
-        out[f"sd/{k}"] = v.detach().numpy().copy()
+    sd = {k: v.detach().numpy().copy() for k, v in model.state_dict().items()}
+    out = {}
 
     model.train()
     crit = torch.nn.CrossEntropyLoss()
@@ -99,39 +123,34 @@ def make_model_case(name, C, nc, B, T, kwargs, adam_steps):
         out["adam_steps"] = np.int64(adam_steps)
         for k, v in model.state_dict().items():
             out[f"sd_adam/{k}"] = v.detach().numpy().copy()
-    out["meta"] = np.frombuffer(json.dumps({
-        "C": C, "num_classes": nc, "B": B, "T": T, "kwargs": kwargs, "versions": _versions(),
-        "source": "reference models.py CnnGruAttentionModel, dropout=0.0, float32, CPU"}).encode(), dtype=np.uint8)
-    np.savez_compressed(GOLDEN / f"model_{name}.npz", **out)
+    meta = {"C": C, "num_classes": nc, "B": B, "T": T, "kwargs": kwargs, "versions": _versions(),
+            "source": "reference models.py CnnGruAttentionModel, dropout=0.0, float32, CPU"}
+    np.savez_compressed(GOLDEN / f"model_{name}.npz", **pack_model_case(meta, x, y, sd, out))
     print(f"model_{name}: loss={loss.item():.6f}")
 
 
 # ----------------------------------------------------------------------- preprocess
+def pack_resample_cases(meta, xs, ys):
+    """The resample fixture: the reference's outputs in full, the digests of the inputs (rebuilt from their seed)."""
+    out = {}
+    for i, ((_, _, f0, f1), y) in enumerate(zip(gi.RESAMPLE_CASES, ys)):
+        out[f"y{i}"] = y
+        out[f"fs{i}"] = np.asarray([f0, f1], dtype=np.int64)
+    out["n_cases"] = np.int64(len(ys))
+    digests = {f"x{i}": gi.digest(x) for i, x in enumerate(xs)}
+    out["meta"] = np.frombuffer(json.dumps(dict(meta, inputs="resample_cases", input_sha256=digests)).encode(), dtype=np.uint8)
+    return out
+
+
 def make_resample_cases():
-    """reference ``preprocess.resample_signal`` on short 1-D / 2-D arrays covering
-    down-sampling (700 -> 64/128), up-sampling (4, 32 -> 64), identity (64 -> 64),
-    even and odd lengths."""
+    """reference ``preprocess.resample_signal`` on the short 1-D / 2-D arrays of ``golden_inputs.RESAMPLE_CASES``."""
     with tempfile.TemporaryDirectory() as tmp:
         pp = ref_harness.load("preprocess", scratch_dir=tmp)
-    rng = np.random.default_rng(7)
-    cases = [  # (n, k, original_fs, target_fs)
-        (7137, 1, 700, 64), (7000, 1, 700, 64), (7001, 3, 700, 128), (6999, 1, 700, 64),
-        (240, 1, 4, 64), (241, 1, 4, 64), (1920, 3, 32, 64), (1921, 1, 32, 64),
-        (3840, 1, 64, 64), (3841, 1, 64, 64), (21011, 1, 700, 64), (16384, 1, 700, 64),
-    ]
-    out = {}
-    for i, (n, k, f0, f1) in enumerate(cases):
-        x = rng.standard_normal((n, k)).cumsum(axis=0) * 0.05 + rng.standard_normal((n, k))
-        if k == 1 and i % 2 == 0:
-            x = x[:, 0]
-        y = pp.resample_signal(x, f0, f1)
-        out[f"x{i}"], out[f"y{i}"] = x, y
-        out[f"fs{i}"] = np.asarray([f0, f1], dtype=np.int64)
-    out["n_cases"] = np.int64(len(cases))
-    out["meta"] = np.frombuffer(json.dumps({"versions": _versions(),
-                                            "source": "reference preprocess.resample_signal"}).encode(), dtype=np.uint8)
-    np.savez_compressed(GOLDEN / "resample_cases.npz", **out)
-    print("resample_cases:", len(cases))
+    xs = gi.resample_signals()
+    ys = [pp.resample_signal(x, f0, f1) for x, (_, _, f0, f1) in zip(xs, gi.RESAMPLE_CASES)]
+    meta = {"versions": _versions(), "source": "reference preprocess.resample_signal"}
+    np.savez_compressed(GOLDEN / "resample_cases.npz", **pack_resample_cases(meta, xs, ys))
+    print("resample_cases:", len(xs))
 
 
 def _run_reference_preprocessing(tmp: Path, fs: int, index_probe: bool):

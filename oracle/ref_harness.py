@@ -1,6 +1,9 @@
-"""Import the UNMODIFIED reference modules from ``/root/reference`` (authoring container) or,
-on the GPU box where that tree does not exist, from the byte-identical staging ``baseline/_ref``
-made by ``oracle/build_ref.py`` (git-ignored; it travels with the gpurun snapshot).
+"""Import the UNMODIFIED reference modules (17LiQi/MultimodalSignal: models.py, dataset.py, ...).
+
+Where they are looked for, first match wins: the directory named by ``MMS_REFERENCE_ROOT``; a copy of the
+reference installed under ``oracle/_ref/`` (the tree itself or one directory down); the byte-identical staging
+``baseline/_ref/`` made by ``oracle/build_ref.py``.  Both directories are git-ignored: no reference source enters
+the history.  Without any of them ``available()`` is False and the reference legs of ``bench.py`` say so.
 
 TEST INFRASTRUCTURE ONLY.  Used by ``oracle/make_golden.py`` to produce the
 committed fixtures under ``tests/golden/`` and by ``bench.py --impl reference``
@@ -21,16 +24,25 @@ import sys
 import types
 from pathlib import Path
 
-_STAGED = Path(__file__).resolve().parents[1] / "baseline" / "_ref"     # oracle/build_ref.py (git-ignored, travels to the GPU box)
+_INSTALLED = Path(__file__).resolve().parent / "_ref"
+_STAGED = Path(__file__).resolve().parents[1] / "baseline" / "_ref"     # oracle/build_ref.py
+
+
+def _has_models(d: Path) -> bool:
+    try:
+        return (d / "models.py").is_file()
+    except OSError:                  # a directory this user may not search counts as absent
+        return False
 
 
 def _find_root() -> Path:
     env = os.environ.get("MMS_REFERENCE_ROOT")
     if env:
         return Path(env)
-    if Path("/root/reference/models.py").exists():
-        return Path("/root/reference")
-    return _STAGED
+    candidates = [_INSTALLED]
+    if _INSTALLED.is_dir():
+        candidates += sorted(d for d in _INSTALLED.iterdir() if d.is_dir())
+    return next((d for d in candidates + [_STAGED] if _has_models(d)), _STAGED)
 
 
 REFERENCE_ROOT = _find_root()
@@ -38,7 +50,7 @@ _STUBS = ("matplotlib", "matplotlib.pyplot", "seaborn", "neurokit2")
 
 
 def available() -> bool:
-    return (REFERENCE_ROOT / "models.py").exists()
+    return _has_models(REFERENCE_ROOT)
 
 
 def staged_ok() -> bool:

@@ -58,7 +58,7 @@ def test_two_rank_data_parallel_equals_full_batch(case, splits):
             if v.numel() == 0:
                 continue
             np.testing.assert_allclose(v.float().cpu().numpy(), ref_sd[k].float().cpu().numpy(), atol=2e-5, err_msg=k)
-    if "adam_losses" in z.files:        # and therefore also the reference's own trajectory
+    if "adam_losses" in z:        # and therefore also the reference's own trajectory
         np.testing.assert_allclose(losses[:int(z["adam_steps"])], z["adam_losses"][:3], atol=1e-4)
 
 

@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import MODEL_CASES, golden_state, load_golden
+from conftest import MODEL_CASES, golden_kept, golden_state, load_golden
 from oracle import model_oracle as mo
 
 
@@ -24,11 +24,10 @@ def test_forward_backward_matches_reference(case, prune):
     np.testing.assert_allclose(logits.numpy(), z["train_logits"], atol=2e-5, rtol=1e-4)
     assert abs(loss.item() - float(z["train_loss"])) < 2e-5
     for k in params:
-        ref = z[f"grad/{k}"]
-        got = grads[k].numpy()
+        got, ref = golden_kept(z, f"grad/{k}", grads[k].numpy())
         if ref.size == 0:
             continue
-        scale = max(1e-6, np.abs(ref).max())
+        scale = max(1e-6, float(z[f"absmax/grad/{k}"]))
         assert np.abs(got - ref).max() <= 2e-4 * scale + 1e-7, k
 
 
@@ -82,7 +81,7 @@ def test_adam_trajectory(case):
                 params[k], m[k], v2[k] = mo.adam_step(params[k], grads[k], m[k], v2[k], step)
     np.testing.assert_allclose(losses, z["adam_losses"], atol=5e-5)
     for k in params:
-        np.testing.assert_allclose(params[k].numpy(), z[f"sd_adam/{k}"], atol=3e-5, err_msg=k)
+        np.testing.assert_allclose(*golden_kept(z, f"sd_adam/{k}", params[k].numpy()), atol=3e-5, err_msg=k)
 
 
 def test_cnn_gru_baseline_is_attention_identity():
@@ -122,7 +121,7 @@ def test_cpu_port_matches_reference(case):
     loss.backward()
     for k, v in p.items():
         if v.numel():
-            ref = z[f"grad/{k}"]
-            assert np.abs(v.grad.numpy() - ref).max() <= 2e-4 * max(1e-6, np.abs(ref).max()) + 1e-7, k
+            got, ref = golden_kept(z, f"grad/{k}", v.grad.numpy())
+            assert np.abs(got - ref).max() <= 2e-4 * max(1e-6, float(z[f"absmax/grad/{k}"])) + 1e-7, k
     for k, v in bufs.items():
         np.testing.assert_allclose(v.numpy(), z[f"sd_after_fwd/{k}"], atol=1e-6, rtol=1e-5)
