@@ -80,7 +80,7 @@ typedef struct {
     int32_t seq_len;        /* T  = window samples (3840 @64 Hz, 7680 @128 Hz)          */
     int32_t num_classes;    /* 2 (stress_binary) or 3 (ternary), <= 8                   */
     int32_t cnn_out;        /* cnn_out_channels, models.py:39 (32)                      */
-    int32_t hidden;         /* gru_hidden_size (64 or 32)                               */
+    int32_t hidden;         /* gru_hidden_size: 32, 64 or 128; others are MMS_E_INVALID */
     int32_t layers;         /* gru_num_layers (>= 1)                                    */
     int32_t training;       /* 1: batch-stat BN + dropout (model.train()), 0: eval      */
     int32_t attention;      /* 1: ChannelAttention gate, 0: cnn_gru baseline (SURVEY D3)*/
@@ -321,7 +321,9 @@ int mms_gemm_tn_acc(const float* A, int64_t lda, int32_t a_split, int32_t a_skip
 int mms_dropout_apply(const float* in, float* out, int64_t n, int64_t base_id, float dropout_p,
                       uint64_t rng_seed, uint64_t rng_offset, const int64_t* rng_offset_dev, mms_stream_t stream);
 
-/* The GRU recurrence of one direction (models.py:56-63; gate order r,z,n; h0 = 0).
+/* The GRU recurrence of one direction (models.py:56-63; gate order r,z,n; h0 = 0).  H is 32, 64 or
+ * 128.  At H = 128 every pointer and stride must be 16-byte / 4-float aligned (the shared-memory-ring
+ * kernels are the only ones built for that size) and MMS_GRU_FWD_V2=0 / MMS_GRU_BWD_RING=0 are refused.
  * gi[(b*gi_bs + t*gi_ts) + 0..3H) are the input projections (incl. b_ih).  Runs `nsteps` steps
  * starting at t0 and moving by dt (+1 forward, -1 reverse).  Writes h to hs[b*hs_bs + t*hs_ts + j]
  * and, if stash != NULL, (r,z,n,W_hn h + b_hn) to

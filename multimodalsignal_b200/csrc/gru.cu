@@ -745,10 +745,24 @@ static inline int rows_per_cta(int B, int ndirs) {
     return R;
 }
 
+// Hidden size 128 runs the same kernels as 32 / 64, instantiated at H = 128 (256 threads, one CTA per SM):
+//   gru_fwd_v2_kernel<128>        ptxas: 244 registers, no spill; static shared memory 4 x 3H (ring) + 2 x (H + 8) floats = 7232 bytes
+//   gru_bwd_ring_kernel<128, 8>   ptxas: 255 registers, no spill; 8 x 6H (ring) + 2 x 3 x (H + 16) floats = 28032 bytes
+//   gru_bwd_ring_kernel<128, 4>   ptxas: 255 registers, no spill; 4 x 6H + 2 x 3 x (H + 16) floats = 15744 bytes
+// 256 threads x 255 registers = 65280 of the SM's 65536: one recurrence CTA per SM.  W_hh of one direction (3H x H fp32 =
+// 192 KB) lives entirely in registers, 192 floats per thread.  The multi-row kernels (gru_fwd_kernel / gru_bwd_kernel with
+// R > 1) spill at H = 128 (gru_bwd_kernel<128, 1> already spills 96 bytes), so they are not instantiated: large batches run one
+// row per CTA over several waves, and the register-ring backward (GRU_BWD_RING=0, or operands that are not 16-byte aligned) is
+// refused at this size.
+constexpr int GRU_H_WIDE = 128;
+
 template <int H>
 static int gru_fwd_dispatch(const GruFwdParams& prm, int ndirs, cudaStream_t st) {
-    const int R = rows_per_cta(prm.B, ndirs);
+    const bool wide = H == GRU_H_WIDE;
+    const int R = wide ? 1 : rows_per_cta(prm.B, ndirs);          // hidden size 128: one row per CTA at every batch size
     dim3 grid(cdiv(prm.B, R), ndirs);
+    MMS_REQUIRE(!wide || option_get("GRU_FWD_V2", 1) == 1,
+                "gru_recur_fwd: GRU_FWD_V2=0 selects the multi-row forward, which has no hidden size %d kernel", H);
     if (R == 1 && option_get("GRU_FWD_V2", 1) == 1) {      // experiment (see gru_fwd_v2_kernel)
         MMS_PROF_BEGIN(st);
         auto k2 = gru_fwd_v2_kernel<H>;
@@ -756,14 +770,16 @@ static int gru_fwd_dispatch(const GruFwdParams& prm, int ndirs, cudaStream_t st)
         MMS_LAUNCH_CHECK("gru_fwd_v2_kernel");
         return MMS_OK;
     }
-    MMS_PROF_BEGIN(st);
-    auto k1 = gru_fwd_kernel<H, 1>;
-    auto k2 = gru_fwd_kernel<H, 2>;
-    auto k4 = gru_fwd_kernel<H, 4>;
-    if (R == 1) MMS_LAUNCH(k1, grid, dim3(2 * H), 0, st, prm);
-    else if (R == 2) MMS_LAUNCH(k2, grid, dim3(2 * H), 0, st, prm);
-    else MMS_LAUNCH(k4, grid, dim3(2 * H), 0, st, prm);
-    MMS_LAUNCH_CHECK("gru_fwd_kernel");
+    if constexpr (H != GRU_H_WIDE) {
+        MMS_PROF_BEGIN(st);
+        auto k1 = gru_fwd_kernel<H, 1>;
+        auto k2 = gru_fwd_kernel<H, 2>;
+        auto k4 = gru_fwd_kernel<H, 4>;
+        if (R == 1) MMS_LAUNCH(k1, grid, dim3(2 * H), 0, st, prm);
+        else if (R == 2) MMS_LAUNCH(k2, grid, dim3(2 * H), 0, st, prm);
+        else MMS_LAUNCH(k4, grid, dim3(2 * H), 0, st, prm);
+        MMS_LAUNCH_CHECK("gru_fwd_kernel");
+    }
     return MMS_OK;
 }
 
@@ -780,13 +796,18 @@ static bool bwd_ring_ok(const GruBwdParams& prm, int ndirs) {
 
 template <int H>
 static int gru_bwd_dispatch(const GruBwdParams& prm, int ndirs, cudaStream_t st) {
-    const int R = rows_per_cta(prm.B, ndirs);
+    const int R = H == GRU_H_WIDE ? 1 : rows_per_cta(prm.B, ndirs);   // hidden size 128: one row per CTA at every batch size
     dim3 grid(cdiv(prm.B, R), ndirs);
     // MMS_GRU_BWD_RING / mms_set_option("GRU_BWD_RING", n): shared-memory ring of depth 8 (default) or 4; 0 = the register-ring
     // kernel (gru_bwd_kernel), which also serves R > 1 rows per CTA and operands that are not 16-byte aligned.
     // Measured on a B200 (profiles/r1_ab_gru_bwd_ring.json): 89.6 us (register ring) -> 69.3 us (depth 4) -> 66.7 us (depth 8)
     // per launch; depth 8 is the default since round 2 (the whole GPU suite runs with it).
     const int ring = option_get("GRU_BWD_RING", 8);
+    if (H == GRU_H_WIDE) {
+        MMS_REQUIRE(ring > 0, "gru_recur_bwd: GRU_BWD_RING=0 selects the register-ring backward, which has no hidden size %d kernel", H);
+        MMS_REQUIRE(bwd_ring_ok(prm, ndirs),
+                    "gru_recur_bwd: at hidden size %d stash / hs / dout must be 16-byte aligned with strides that are multiples of 4 floats", H);
+    }
     if (ring > 0 && R == 1 && bwd_ring_ok(prm, ndirs)) {
         // MMS_GRU_BWD_EXCLUSIVE_KB (experiment, default 0): reserve that much dynamic shared memory per CTA so that no
         // other kernel's CTAs (the weight-gradient GEMMs of the side streams) can share an SM with a recurrence CTA
@@ -809,18 +830,20 @@ static int gru_bwd_dispatch(const GruBwdParams& prm, int ndirs, cudaStream_t st)
         MMS_LAUNCH_CHECK("gru_bwd_ring_kernel");
         return MMS_OK;
     }
-    MMS_PROF_BEGIN(st);
-    if (R == 1) gru_bwd_kernel<H, 1><<<grid, 2 * H, 0, st>>>(prm);
-    else if (R == 2) gru_bwd_kernel<H, 2><<<grid, 2 * H, 0, st>>>(prm);
-    else gru_bwd_kernel<H, 4><<<grid, 2 * H, 0, st>>>(prm);
-    MMS_LAUNCH_CHECK("gru_bwd_kernel");
+    if constexpr (H != GRU_H_WIDE) {
+        MMS_PROF_BEGIN(st);
+        if (R == 1) gru_bwd_kernel<H, 1><<<grid, 2 * H, 0, st>>>(prm);
+        else if (R == 2) gru_bwd_kernel<H, 2><<<grid, 2 * H, 0, st>>>(prm);
+        else gru_bwd_kernel<H, 4><<<grid, 2 * H, 0, st>>>(prm);
+        MMS_LAUNCH_CHECK("gru_bwd_kernel");
+    }
     return MMS_OK;
 }
 
 int launch_gru_fwd(const mms_gru_dir_fwd* dirs, int ndirs, int B, int H, float p, uint64_t seed, uint64_t offset,
                    const int64_t* offset_dev, cudaStream_t st) {
     MMS_REQUIRE(ndirs >= 1 && ndirs <= GRU_MAX_DIRS && B > 0, "gru_recur_fwd: bad direction count / batch");
-    MMS_REQUIRE(H == 64 || H == 32, "gru_recur_fwd: hidden size %d not supported (32 or 64)", H);
+    MMS_REQUIRE(H == 32 || H == 64 || H == GRU_H_WIDE, "gru_recur_fwd: hidden size %d not supported (32, 64 or 128)", H);
     GruFwdParams prm;
     for (int i = 0; i < ndirs; ++i) {
         prm.dir[i] = dirs[i];
@@ -831,13 +854,14 @@ int launch_gru_fwd(const mms_gru_dir_fwd* dirs, int ndirs, int B, int H, float p
     }
     for (int i = ndirs; i < GRU_MAX_DIRS; ++i) prm.dir[i] = dirs[0];
     prm.B = B; prm.p = p; prm.seed = seed; prm.offset = offset; prm.offset_dev = offset_dev;
+    if (H == GRU_H_WIDE) return gru_fwd_dispatch<GRU_H_WIDE>(prm, ndirs, st);
     return H == 64 ? gru_fwd_dispatch<64>(prm, ndirs, st) : gru_fwd_dispatch<32>(prm, ndirs, st);
 }
 
 int launch_gru_bwd(const mms_gru_dir_bwd* dirs, int ndirs, int B, int H, float p, uint64_t seed, uint64_t offset,
                    const int64_t* offset_dev, cudaStream_t st) {
     MMS_REQUIRE(ndirs >= 1 && ndirs <= GRU_MAX_DIRS && B > 0, "gru_recur_bwd: bad direction count / batch");
-    MMS_REQUIRE(H == 64 || H == 32, "gru_recur_bwd: hidden size %d not supported (32 or 64)", H);
+    MMS_REQUIRE(H == 32 || H == 64 || H == GRU_H_WIDE, "gru_recur_bwd: hidden size %d not supported (32, 64 or 128)", H);
     GruBwdParams prm;
     for (int i = 0; i < ndirs; ++i) {
         prm.dir[i] = dirs[i];
@@ -847,6 +871,7 @@ int launch_gru_bwd(const mms_gru_dir_bwd* dirs, int ndirs, int B, int H, float p
     }
     for (int i = ndirs; i < GRU_MAX_DIRS; ++i) prm.dir[i] = dirs[0];
     prm.B = B; prm.p = p; prm.seed = seed; prm.offset = offset; prm.offset_dev = offset_dev;
+    if (H == GRU_H_WIDE) return gru_bwd_dispatch<GRU_H_WIDE>(prm, ndirs, st);
     return H == 64 ? gru_bwd_dispatch<64>(prm, ndirs, st) : gru_bwd_dispatch<32>(prm, ndirs, st);
 }
 

@@ -97,11 +97,53 @@ static bool bn_fold() {
     return v == 1;
 }
 
-// Weight-gradient (TN) products: tcgen05 split-K kernel when the shape allows it, fp32 SIMT otherwise.
+// The TN kernel takes at most 256 gradient rows (N1, two UMMA M = 128 tiles) and 224 columns (N2).  At hidden size 128 the
+// gradients have N1 = 3H = 384 rows, and the upper layers' W_ih gradient N2 = 2H = 256 columns: such a problem is cut into
+// row halves (the a_split / a_skip column map of D moved past the rows before the cut) times column halves, and only the
+// first column half adds the bias gradient.  A problem that fits -- every one at hidden size 32 and 64 -- is passed through.
+constexpr int TN_PIECES_MAX = 4;
+static int tn_split(const TnCall& c, TnCall* out) {
+    const int n1_parts = c.N1 > 256 ? 2 : 1, n2_parts = c.N2 > 224 ? 2 : 1;
+    const int n1 = c.N1 / n1_parts, n2 = c.N2 / n2_parts;
+    int n = 0;
+    for (int i = 0; i < n1_parts; ++i) {
+        const int r0 = i * n1;                 // first gradient row of the piece: D column acol(r0)
+        for (int j = 0; j < n2_parts; ++j) {
+            TnCall q = c;
+            q.N1 = n1;
+            if (r0 < c.a_split) { q.A = c.A + r0; q.a_split = c.a_split - r0; }
+            else { q.A = c.A + r0 + c.a_skip; q.a_split = n1; q.a_skip = 0; }
+            q.N2 = n2;
+            q.Bm = c.Bm ? c.Bm + (int64_t)j * n2 : nullptr;
+            q.C = c.C ? c.C + (int64_t)r0 * c.ldc + (int64_t)j * n2 : nullptr;
+            q.bias_grad = c.bias_grad && j == 0 ? c.bias_grad + r0 : nullptr;
+            out[n++] = q;
+        }
+    }
+    return n;
+}
+
+static bool tn_tc_ok(const TnCall& c) {
+    return tc_gemm_tn_supported(c.A, c.lda, c.a_split, c.a_skip, c.N2 > 0 ? c.Bm : nullptr, c.ldb, c.N2 > 0 ? c.C : nullptr, c.ldc,
+                                c.M, c.N1, c.N2);
+}
+
+// Weight-gradient (TN) products: tcgen05 split-K kernel when the shape allows it (after tn_split), fp32 SIMT otherwise.
 static int gemm_tn(const float* A, int64_t lda, int a_split, int a_skip, const float* Bm, int64_t ldb, int shift, int seq, float* C,
                    int64_t ldc, float* bias_grad, int M, int N1, int N2, cudaStream_t st) {
-    if (use_tc() && M >= 1024 && tc_gemm_tn_supported(A, lda, a_split, a_skip, N2 > 0 ? Bm : nullptr, ldb, N2 > 0 ? C : nullptr, ldc, M, N1, N2))
-        return launch_tc_gemm_tn(A, lda, a_split, a_skip, Bm, ldb, shift, seq, C, ldc, bias_grad, M, N1, N2, st);
+    if (use_tc() && M >= 1024) {
+        TnCall piece[TN_PIECES_MAX];
+        const int np = tn_split({A, lda, a_split, a_skip, Bm, ldb, shift, seq, C, ldc, bias_grad, M, N1, N2}, piece);
+        bool ok = true;
+        for (int j = 0; j < np; ++j) ok = ok && tn_tc_ok(piece[j]);
+        for (int j = 0; ok && j < np; ++j) {
+            const TnCall& c = piece[j];
+            const int rc = launch_tc_gemm_tn(c.A, c.lda, c.a_split, c.a_skip, c.Bm, c.ldb, c.shift, c.seq, c.C, c.ldc, c.bias_grad, c.M,
+                                             c.N1, c.N2, st);
+            if (rc) return rc;
+        }
+        if (ok) return MMS_OK;
+    }
     return launch_gemm_tn_acc(A, lda, a_split, a_skip, Bm, ldb, shift, seq, C, ldc, bias_grad, M, N1, N2, st);
 }
 
@@ -109,7 +151,7 @@ int launch_tc_gemm_tn_batch(const TnCall*, int, cudaStream_t);
 
 // Several TN products on one stream: one launch of the batched tensor-core kernel when MMS_TN_BATCH=1 (experiment) and every
 // problem qualifies for it, otherwise one launch each (the default).
-static int gemm_tn_many(const TnCall* c, int n, cudaStream_t st) {
+static int gemm_tn_group(const TnCall* c, int n, cudaStream_t st) {
     bool batch = n > 1 && n <= 4 && use_tc() && option_get("TN_BATCH", 1) == 1;
     for (int j = 0; batch && j < n; ++j)
         batch = c[j].M >= 1024 && c[j].N1 > 0 &&
@@ -119,6 +161,24 @@ static int gemm_tn_many(const TnCall* c, int n, cudaStream_t st) {
     for (int j = 0; j < n; ++j) {
         int rc = gemm_tn(c[j].A, c[j].lda, c[j].a_split, c[j].a_skip, c[j].Bm, c[j].ldb, c[j].shift, c[j].seq, c[j].C, c[j].ldc,
                          c[j].bias_grad, c[j].M, c[j].N1, c[j].N2, st);
+        if (rc) return rc;
+    }
+    return MMS_OK;
+}
+
+// Up to four TN products on one stream, cut to the TN kernel's limits (tn_split; at hidden size 32 / 64 nothing is cut) and run in
+// groups of four.
+static int gemm_tn_many(const TnCall* c, int n, cudaStream_t st) {
+    constexpr int MAX_CALLS = 4;
+    MMS_REQUIRE(n >= 1 && n <= MAX_CALLS, "gemm_tn_many: 1..%d problems", MAX_CALLS);
+    TnCall pieces[MAX_CALLS * TN_PIECES_MAX];
+    int np = 0;
+    for (int j = 0; j < n; ++j) {
+        if (use_tc() && c[j].M >= 1024) np += tn_split(c[j], pieces + np);
+        else pieces[np++] = c[j];
+    }
+    for (int j0 = 0; j0 < np; j0 += 4) {
+        const int rc = gemm_tn_group(pieces + j0, np - j0 < 4 ? np - j0 : 4, st);
         if (rc) return rc;
     }
     return MMS_OK;
@@ -224,7 +284,7 @@ static int make_dims(const mms_cnngru_desc* d, Dims* o) {
     MMS_REQUIRE(o->C >= 1 && o->C <= 16, "in_channels %d outside [1,16]", o->C);
     MMS_REQUIRE(o->nc >= 1 && o->nc <= 8, "num_classes %d outside [1,8]", o->nc);
     MMS_REQUIRE(o->O == 16 || o->O == 32 || o->O == 64, "cnn_out_channels %d not in {16,32,64}", o->O);
-    MMS_REQUIRE(o->H == 32 || o->H == 64, "gru_hidden_size %d not in {32,64}", o->H);
+    MMS_REQUIRE(o->H == 32 || o->H == 64 || o->H == 128, "gru_hidden_size %d not in {32,64,128}", o->H);
     MMS_REQUIRE(o->layers >= 1 && o->layers <= MAX_LAYERS, "gru_num_layers %d outside [1,%d]", o->layers, MAX_LAYERS);
     o->L1c = conv_out_len(o->T, CONV1_K, CONV1_S, CONV1_P);
     MMS_REQUIRE(o->T >= 1 && o->L1c >= 1, "seq_len %d too short", o->T);
