@@ -93,6 +93,11 @@ typedef struct {
     int32_t global_batch;   /* 0 or == batch: single GPU.  > batch: intra-fold data parallelism -- BatchNorm
                                statistics are counted over the global batch (SyncBN) and the BN affine
                                gradients are scaled by batch/global_batch so that a sum all-reduce is exact */
+    const float* class_weight; /* NULL: CrossEntropyLoss().  Else float32 [num_classes] device array, the
+                                  CrossEntropyLoss(weight=w) of mms_cnngru_train_step (fused and unfused head):
+                                  loss = sum_b w[y_b] l_b / sum_b w[y_b], dlogits = w[y_b] (softmax - onehot) / sum_b w[y_b].
+                                  The train step needs global_batch == batch; under data parallelism the BN2 sum
+                                  vector of mms_cnngru_sync_offsets gets one more double for sum_b w[y_b] */
 } mms_cnngru_desc;
 
 /* Flat parameter buffer.  The model's parameters live in ONE float32 buffer so that Adam and
@@ -136,7 +141,10 @@ int mms_cnngru_backward(const mms_cnngru_desc* d, const float* x, const float* p
  *             gradients, stage-1 pool/ReLU backward (+BN1 reductions) | 4 = the rest
  * Between the phases the caller sum-all-reduces the float64 vectors whose byte offsets inside the
  * workspace mms_cnngru_sync_offsets() reports: [0] BN1 sums, [1] BN2 sums (forward), [2] BN1
- * reductions, [3] BN2 reductions (backward); counts are in doubles.  desc.global_batch must be set. */
+ * reductions, [3] BN2 reductions (backward); counts are in doubles.  desc.global_batch must be set.
+ * With desc.class_weight set, vector [1] has 2*cnn_out + 1 doubles: the caller writes the local sum_b w[y_b] into the last
+ * one (mms_class_weight_sum) after forward phase 1 and before the exchange, and the weighted cross entropy reads the sum
+ * from there (mms_cross_entropy_weighted's norm_dev).  Without class weights offsets and counts are unchanged. */
 int mms_cnngru_forward_phase(const mms_cnngru_desc* d, int32_t phases, const float* x, const float* params,
                              float* bn_buffers, int64_t* num_batches_tracked, void* workspace, float* logits,
                              mms_stream_t stream);
@@ -182,6 +190,19 @@ int mms_peer_allreduce_adam(float* params, const void* const* grads_host, void* 
  * this keeps the sum on the device so that a step needs no sync). */
 int mms_cross_entropy(const float* logits, const int64_t* labels, int32_t batch, int32_t num_classes,
                       float* loss_out, float* dlogits, double* loss_sum_accum, mms_stream_t stream);
+/* CrossEntropyLoss(weight=class_weight) (mean reduction), the same kernel as the two calls above:
+ * loss_out[0] = sum_b w[y_b] (lse_b - logit[b, y_b]) / W, dlogits = w[y_b] (softmax - onehot) / W, where W = *norm_dev
+ * (float64; a rank's share of a data-parallel batch passes the summed slot of mms_cnngru_sync_offsets, and the per-rank
+ * losses then add up to the global weighted mean) or, with norm_dev == NULL, sum_b w[y_b] over this batch.  Labels
+ * outside [0, num_classes) make the loss NaN and add no gradient; W == 0 gives NaN, as torch does.  loss_sum_accum
+ * receives += loss * batch.  class_weight == NULL (then norm_dev must be NULL too) is mms_cross_entropy. */
+int mms_cross_entropy_weighted(const float* logits, const int64_t* labels, int32_t batch, int32_t num_classes,
+                               const float* class_weight, const double* norm_dev, float* loss_out, float* dlogits,
+                               double* loss_sum_accum, mms_stream_t stream);
+/* out[0] = sum_b class_weight[labels[b]] over the labels in [0, num_classes) (float64, written, fixed order): the local
+ * normaliser of the weighted cross entropy. */
+int mms_class_weight_sum(const int64_t* labels, int32_t batch, int32_t num_classes, const float* class_weight,
+                         double* out, mms_stream_t stream);
 
 /* trainer.py:68,149 torch.optim.Adam (coupled L2 weight decay) over the flat buffer.
  * step_dev holds the number of steps already taken; the kernel uses step_dev+1 for the bias
@@ -208,6 +229,14 @@ int mms_batch_gather(const float* data, const int64_t* labels, const int64_t* pe
  * preds_out, confusion and loss_sum may each be NULL. */
 int mms_eval_accumulate(const float* logits, const int64_t* labels, int32_t batch, int32_t num_classes,
                         int64_t* preds_out, int64_t* confusion, double* loss_sum, mms_stream_t stream);
+/* The same with CrossEntropyLoss(weight=class_weight): the rows are cut into groups of `group` consecutive rows (the
+ * evaluation loader's batches; group <= 0: one group of `batch` rows, the last group may be shorter) and every group g of
+ * n_g rows adds n_g * sum_{b in g} w[y_b] l_b / sum_{b in g} w[y_b] to *loss_sum (float64, groups in order), as the
+ * reference adds loss.item() * batch per loader batch.  Predictions and confusion counts are those of
+ * mms_eval_accumulate; class_weight == NULL is mms_eval_accumulate. */
+int mms_eval_accumulate_weighted(const float* logits, const int64_t* labels, int32_t batch, int32_t num_classes,
+                                 const float* class_weight, int32_t group, int64_t* preds_out, int64_t* confusion,
+                                 double* loss_sum, mms_stream_t stream);
 
 /* One whole training step, trainer.py:144-149: zero_grad, forward, CE, backward, Adam.
  * (With world_size > 1 the host calls forward/backward/adam separately around its NCCL

@@ -33,7 +33,7 @@ class CnnGruDesc(C.Structure):
         ("cnn_out", c_i32), ("hidden", c_i32), ("layers", c_i32), ("training", c_i32),
         ("attention", c_i32), ("need_grad", c_i32), ("dropout_p", c_f32),
         ("rng_seed", c_u64), ("rng_offset", c_u64), ("rng_offset_dev", C.c_void_p),
-        ("global_batch", c_i32),
+        ("global_batch", c_i32), ("class_weight", C.c_void_p),
     ]
 
 
@@ -91,6 +91,8 @@ _SIGNATURES = {
     "mms_cnngru_backward": (c_i32, [C.POINTER(CnnGruDesc), P, P, P, P, P, P, P, P]),
     "mms_cross_entropy": (c_i32, [P, P, c_i32, c_i32, P, P, P, P]),
     "mms_cross_entropy_partial": (c_i32, [P, P, c_i32, c_i32, c_i32, P, P, P, P]),
+    "mms_cross_entropy_weighted": (c_i32, [P, P, c_i32, c_i32, P, P, P, P, P, P]),
+    "mms_class_weight_sum": (c_i32, [P, c_i32, c_i32, P, P, P]),
     "mms_cnngru_forward_phase": (c_i32, [C.POINTER(CnnGruDesc), c_i32, P, P, P, P, P, P, P]),
     "mms_cnngru_backward_phase": (c_i32, [C.POINTER(CnnGruDesc), c_i32, P, P, P, P, P, P, P]),
     "mms_cnngru_sync_offsets": (c_i32, [C.POINTER(CnnGruDesc), C.POINTER(c_i64), C.POINTER(c_i64)]),
@@ -102,6 +104,7 @@ _SIGNATURES = {
                                       c_f32, c_f32, c_f32, c_f32, P, P, P]),
     "mms_batch_gather": (c_i32, [P, P, P, P, c_i64, c_i64, c_i32, P, P, c_i32, P, P]),
     "mms_eval_accumulate": (c_i32, [P, P, c_i32, c_i32, P, P, P, P]),
+    "mms_eval_accumulate_weighted": (c_i32, [P, P, c_i32, c_i32, P, c_i32, P, P, P, P]),
     "mms_chan_attn_fwd": (c_i32, [P, P, P, c_i32, c_i32, c_i32, P, P, P, P]),
     "mms_chan_attn_bwd": (c_i32, [P, P, P, P, P, P, c_i32, c_i32, c_i32, P, P, P, P, P]),
     "mms_conv1d_fwd": (c_i32, [c_i32, P, P, P, c_i32, c_i32, c_i32, c_i32, P, P, P]),

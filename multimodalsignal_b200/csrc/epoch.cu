@@ -43,41 +43,81 @@ __global__ void __launch_bounds__(256) batch_gather_kernel(const float4* __restr
     }
 }
 
+// Row b's loss term lse - logit[y] (y clamped into [0, nc)), its first arg-max and its clamped label.
+__device__ __forceinline__ float eval_row(const float* __restrict__ logits, const int64_t* __restrict__ labels, int b, int nc,
+                                          int* am_out, int* y_out) {
+    float v[MAX_NC];
+    for (int c = 0; c < nc; ++c) v[c] = logits[(size_t)b * nc + c];
+    float mx = v[0];
+    int am = 0;
+    for (int c = 1; c < nc; ++c)              // first maximum; a NaN counts as the maximum, like torch.argmax
+        if (!(mx != mx) && (v[c] > mx || v[c] != v[c])) { mx = v[c]; am = c; }
+    float m2 = -INFINITY;
+    for (int c = 0; c < nc; ++c) m2 = fmaxf(m2, v[c]);
+    float se = 0.f;
+    for (int c = 0; c < nc; ++c) se += expf(v[c] - m2);
+    const float lse = m2 + logf(se);
+    int y = (int)labels[b];
+    y = y < 0 ? 0 : (y >= nc ? nc - 1 : y);
+    *am_out = am;
+    *y_out = y;
+    return lse - v[y];
+}
+
 // Single CTA.  For every row: loss_sum += lse - logit[y] (float64), pred = first arg-max of the logits
 // (== torch.argmax(softmax(logits)), ties to the lowest index), conf[y * nc + pred] += 1.
+// With class_weight (CrossEntropyLoss(weight=w)) the loss is the reference's per-loader-batch accumulation instead: the rows
+// are taken in groups of `group` consecutive rows, each reduced over the block in a fixed order, and group g adds
+// n_g * sum w[y] l / sum w[y] (the groups in order).  A null class_weight runs exactly the unweighted code.
 __global__ void __launch_bounds__(256) eval_accumulate_kernel(const float* __restrict__ logits, const int64_t* __restrict__ labels,
                                                               int B, int nc, int64_t* __restrict__ preds, int64_t* conf,
-                                                              double* loss_sum) {
+                                                              double* loss_sum, const float* __restrict__ class_weight, int group) {
     __shared__ double s_part[8];
+    __shared__ double s_wpart[8];
     __shared__ unsigned int s_conf[MAX_NC * MAX_NC];
     for (int i = threadIdx.x; i < nc * nc; i += blockDim.x) s_conf[i] = 0u;
     __syncthreads();
     double local = 0.0;
     for (int b = threadIdx.x; b < B; b += blockDim.x) {
-        float v[MAX_NC];
-        for (int c = 0; c < nc; ++c) v[c] = logits[(size_t)b * nc + c];
-        float mx = v[0];
-        int am = 0;
-        for (int c = 1; c < nc; ++c)              // first maximum; a NaN counts as the maximum, like torch.argmax
-            if (!(mx != mx) && (v[c] > mx || v[c] != v[c])) { mx = v[c]; am = c; }
-        float m2 = -INFINITY;
-        for (int c = 0; c < nc; ++c) m2 = fmaxf(m2, v[c]);
-        float se = 0.f;
-        for (int c = 0; c < nc; ++c) se += expf(v[c] - m2);
-        const float lse = m2 + logf(se);
-        int y = (int)labels[b];
-        y = y < 0 ? 0 : (y >= nc ? nc - 1 : y);
-        local += (double)(lse - v[y]);
+        int am, y;
+        const float l = eval_row(logits, labels, b, nc, &am, &y);
+        local += (double)l;
         if (preds) preds[b] = am;
         atomicAdd(&s_conf[y * nc + am], 1u);
     }
-    local = warp_sum(local);
-    if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = local;
-    __syncthreads();
-    if (threadIdx.x == 0 && loss_sum) {
-        double s = 0.0;
-        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += s_part[w];
-        *loss_sum += s;
+    if (class_weight) {
+        double total = 0.0;                                  // meaningful in thread 0 only
+        for (int g0 = 0; g0 < B; g0 += group) {
+            const int n = B - g0 < group ? B - g0 : group;
+            double num = 0.0, den = 0.0;
+            for (int b = g0 + threadIdx.x; b < g0 + n; b += blockDim.x) {
+                int am, y;
+                const float l = eval_row(logits, labels, b, nc, &am, &y);
+                const double wy = (double)class_weight[y];
+                num += wy * (double)l;
+                den += wy;
+            }
+            num = warp_sum(num);
+            den = warp_sum(den);
+            if ((threadIdx.x & 31) == 0) { s_part[threadIdx.x >> 5] = num; s_wpart[threadIdx.x >> 5] = den; }
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                double sn = 0.0, sd = 0.0;
+                for (int w = 0; w < (int)(blockDim.x >> 5); ++w) { sn += s_part[w]; sd += s_wpart[w]; }
+                total += (double)n * (sn / sd);
+            }
+            __syncthreads();
+        }
+        if (threadIdx.x == 0 && loss_sum) *loss_sum += total;
+    } else {
+        local = warp_sum(local);
+        if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = local;
+        __syncthreads();
+        if (threadIdx.x == 0 && loss_sum) {
+            double s = 0.0;
+            for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += s_part[w];
+            *loss_sum += s;
+        }
     }
     if (conf)
         for (int i = threadIdx.x; i < nc * nc; i += blockDim.x) conf[i] += (int64_t)s_conf[i];
@@ -114,7 +154,21 @@ extern "C" int mms_eval_accumulate(const float* logits, const int64_t* labels, i
     MMS_REQUIRE(num_classes >= 1 && num_classes <= MAX_NC, "eval_accumulate: num_classes %d outside [1,%d]", num_classes, MAX_NC);
     cudaStream_t st = (cudaStream_t)stream;
     MMS_PROF_BEGIN(st);
-    eval_accumulate_kernel<<<1, 256, 0, st>>>(logits, labels, batch, num_classes, preds_out, confusion, loss_sum);
+    eval_accumulate_kernel<<<1, 256, 0, st>>>(logits, labels, batch, num_classes, preds_out, confusion, loss_sum, nullptr, batch);
+    MMS_LAUNCH_CHECK("eval_accumulate_kernel");
+    return MMS_OK;
+}
+
+extern "C" int mms_eval_accumulate_weighted(const float* logits, const int64_t* labels, int32_t batch, int32_t num_classes,
+                                            const float* class_weight, int32_t group, int64_t* preds_out, int64_t* confusion,
+                                            double* loss_sum, mms_stream_t stream) {
+    MMS_REQUIRE(logits && labels && batch > 0, "eval_accumulate_weighted: bad arguments");
+    MMS_REQUIRE(num_classes >= 1 && num_classes <= MAX_NC, "eval_accumulate_weighted: num_classes %d outside [1,%d]", num_classes,
+                MAX_NC);
+    cudaStream_t st = (cudaStream_t)stream;
+    MMS_PROF_BEGIN(st);
+    eval_accumulate_kernel<<<1, 256, 0, st>>>(logits, labels, batch, num_classes, preds_out, confusion, loss_sum, class_weight,
+                                              group > 0 ? group : batch);
     MMS_LAUNCH_CHECK("eval_accumulate_kernel");
     return MMS_OK;
 }

@@ -1,4 +1,4 @@
-// Classifier head (reference models.py:66-71,79-80), CrossEntropyLoss (trainer.py:69,147) and the
+// Classifier head (reference models.py:66-71,79-80), CrossEntropyLoss (trainer.py:69,147; optionally class-weighted, trainer.py:94) and the
 // fused flat Adam (trainer.py:68,149).  All tiny, latency-bound kernels: the point of fusing them is
 // launch count, not bandwidth.
 #include "mms_common.cuh"
@@ -76,6 +76,13 @@ __global__ void __launch_bounds__(4 * HEAD_HID) head_fwd_kernel(const float* __r
 // LAST CTA to finish (counter zeroed with the forward's memset) from the per-row terms in a fixed order, so the loss is
 // bit-reproducible run to run.  Labels outside [0, nc) poison the loss with NaN (torch raises; a silent clamp would train on
 // garbage) and contribute no gradient.
+// class_weight (optional, [nc]): CrossEntropyLoss(weight=w).  Every CTA needs the normaliser W = sum_b w[y_b] before it can
+// write dlogits; rather than wait on the other CTAs, each one reduces the B labels itself (warp 1, while the other warps load
+// the classifier input), in the same fixed order, so all CTAs hold the same bit pattern.  The row term becomes w[y]*(lse - logit[y]),
+// dlogits (softmax - onehot) * w[y] / W and the loss sum_b w*l / W.  The host picks the instance by the pointer: with the
+// weighted code compiled out, a null pointer runs exactly the unweighted kernel (an in-kernel branch on the pointer measured
+// ~1 us slower per training step on a B200 with weights off: a larger kernel scheduled differently).
+template <bool WEIGHTED>
 __global__ void __launch_bounds__(4 * HEAD_HID) head_ce_fused_kernel(const float* __restrict__ src_a, int64_t lda,
                                                                      const float* __restrict__ src_b, int64_t ldb, int Hh,
                                                                      const float* __restrict__ w0, const float* __restrict__ b0,
@@ -86,12 +93,24 @@ __global__ void __launch_bounds__(4 * HEAD_HID) head_ce_fused_kernel(const float
                                                                      float* __restrict__ hid_out, float* __restrict__ logits,
                                                                      float* __restrict__ dlogits, float* __restrict__ dhid,
                                                                      float* __restrict__ rowloss, int32_t* __restrict__ counter,
-                                                                     float* __restrict__ loss_out, double* __restrict__ loss_sum_accum) {
+                                                                     float* __restrict__ loss_out, double* __restrict__ loss_sum_accum,
+                                                                     const float* __restrict__ class_weight) {
     MMS_PDL_PROLOGUE();
     extern __shared__ __align__(16) float s_last[];        // [H2]
     __shared__ float s_hid[HEAD_HID], s_mask[HEAD_HID], s_logit[MAX_NC], s_dl[MAX_NC];
     __shared__ int s_last_cta;
+    __shared__ float s_wsum;
     const int b = blockIdx.x, B = gridDim.x, tid = threadIdx.x, i = tid >> 2, q = tid & 3;
+    if (WEIGHTED && (tid >> 5) == 1) {
+        const int lane = tid & 31;
+        double ws = 0.0;
+        for (int r = lane; r < B; r += 32) {
+            const int64_t yr = labels[r];
+            if (yr >= 0 && yr < nc) ws += (double)__ldg(class_weight + yr);
+        }
+        ws = warp_sum(ws);
+        if (lane == 0) s_wsum = (float)ws;
+    }
     for (int k = tid; k < H2; k += 4 * HEAD_HID) {
         const float v = k < Hh ? src_a[(size_t)b * lda + k] : src_b[(size_t)b * ldb + (k - Hh)];
         s_last[k] = v;
@@ -144,13 +163,20 @@ __global__ void __launch_bounds__(4 * HEAD_HID) head_ce_fused_kernel(const float
         const float lse = mx + logf(se);
         const int64_t y = labels[b];
         const bool ok = y >= 0 && y < nc;
-        const float invB = 1.f / (float)div_batch;
+        float invB, wy = 1.f;
+        if (WEIGHTED) {
+            wy = ok ? __ldg(class_weight + y) : 0.f;
+            invB = wy / s_wsum;
+        } else {
+            invB = 1.f / (float)div_batch;
+        }
         for (int c = 0; c < nc; ++c) {
             const float dl = ok ? (expf(s_logit[c] - lse) - (c == (int)y ? 1.f : 0.f)) * invB : 0.f;
             s_dl[c] = dl;
             dlogits[(size_t)b * nc + c] = dl;
         }
-        rowloss[b] = ok ? lse - s_logit[(int)y] : __int_as_float(0x7fc00000);
+        const float term = ok ? lse - s_logit[(int)y] : __int_as_float(0x7fc00000);
+        rowloss[b] = WEIGHTED ? wy * term : term;
         __threadfence();
         s_last_cta = atomicAdd(counter, 1) == B - 1;
     }
@@ -166,7 +192,7 @@ __global__ void __launch_bounds__(4 * HEAD_HID) head_ce_fused_kernel(const float
         for (int r = tid; r < B; r += 32) s += __ldcg(rowloss + r);       // fixed order: lane-strided sums, then the shuffle tree
         s = warp_sum(s);
         if (tid == 0) {
-            const float mean = s / (float)div_batch;
+            const float mean = s / (WEIGHTED ? s_wsum : (float)div_batch);
             loss_out[0] = mean;
             if (loss_sum_accum) *loss_sum_accum += (double)mean * (double)div_batch;
         }
@@ -233,14 +259,37 @@ __global__ void __launch_bounds__(128) head_bwd_kernel(const float* __restrict__
 }
 
 // Single CTA.  loss_out[0] = mean_b(lse_b - logit[b, y_b]); dlogits = (softmax - onehot) / B.
+// With class_weight [nc] (CrossEntropyLoss(weight=w)): loss_out[0] = sum_b w[y_b] l_b / W, dlogits = w[y_b] (softmax - onehot) / W,
+// where W is *norm (float64, e.g. the global sum under data parallelism) or, with norm == NULL, sum_b w[y_b] over this batch,
+// reduced first in a fixed order.  A null class_weight runs exactly the unweighted arithmetic.
 __global__ void __launch_bounds__(256) cross_entropy_kernel(const float* __restrict__ logits, const int64_t* __restrict__ labels,
                                                             int B, int nc, float* __restrict__ loss_out,
                                                             float* __restrict__ dlogits, double* __restrict__ loss_sum_accum,
-                                                            int div_batch) {
+                                                            int div_batch, const float* __restrict__ class_weight,
+                                                            const double* __restrict__ norm) {
     MMS_PDL_PROLOGUE();
     __shared__ float s_part[8];
+    __shared__ double s_wpart[8];
     float local = 0.f;
-    const float invB = 1.f / (float)div_batch;     // global batch under data parallelism: the per-rank losses add up
+    float invB = 1.f / (float)div_batch;           // global batch under data parallelism: the per-rank losses add up
+    if (class_weight) {
+        double W;
+        if (norm) {
+            W = *norm;
+        } else {
+            double ws = 0.0;
+            for (int b = threadIdx.x; b < B; b += blockDim.x) {
+                const int64_t yl = labels[b];
+                if (yl >= 0 && yl < nc) ws += (double)class_weight[yl];
+            }
+            ws = warp_sum(ws);
+            if ((threadIdx.x & 31) == 0) s_wpart[threadIdx.x >> 5] = ws;
+            __syncthreads();
+            W = 0.0;
+            for (int w = 0; w < (int)(blockDim.x >> 5); ++w) W += s_wpart[w];
+        }
+        invB = 1.f / (float)W;
+    }
     for (int b = threadIdx.x; b < B; b += blockDim.x) {
         float v[MAX_NC];
         float mx = -INFINITY;
@@ -251,6 +300,14 @@ __global__ void __launch_bounds__(256) cross_entropy_kernel(const float* __restr
         const int64_t yl = labels[b];
         const bool ok = yl >= 0 && yl < nc;      // torch raises on such a label; here the loss turns NaN and the row adds no gradient
         const int y = ok ? (int)yl : 0;
+        if (class_weight) {
+            const float wy = ok ? class_weight[y] : 0.f;
+            local += ok ? wy * (lse - v[y]) : __int_as_float(0x7fc00000);
+            const float scale = wy * invB;
+            if (dlogits)
+                for (int c = 0; c < nc; ++c) dlogits[(size_t)b * nc + c] = ok ? (expf(v[c] - lse) - (c == y ? 1.f : 0.f)) * scale : 0.f;
+            continue;
+        }
         local += ok ? lse - v[y] : __int_as_float(0x7fc00000);
         if (dlogits)
             for (int c = 0; c < nc; ++c) dlogits[(size_t)b * nc + c] = ok ? (expf(v[c] - lse) - (c == y ? 1.f : 0.f)) * invB : 0.f;
@@ -317,12 +374,17 @@ int launch_head_ce_fused(const float* src_a, int64_t lda, const float* src_b, in
                          const float* w3, const float* b3, const int64_t* labels, int B, int H2, int nc, float p, uint64_t seed,
                          uint64_t offset, const int64_t* offset_dev, int div_batch, float* last_out, float* hid_out, float* logits,
                          float* dlogits, float* dhid, float* rowloss, int32_t* counter, float* loss_out, double* loss_sum_accum,
-                         cudaStream_t st) {
+                         cudaStream_t st, const float* class_weight) {
     MMS_REQUIRE(nc >= 1 && nc <= MAX_NC, "head: num_classes %d outside [1,%d]", nc, MAX_NC);
     MMS_PROF_BEGIN(st);
-    MMS_LAUNCH(head_ce_fused_kernel, dim3(B), dim3(4 * HEAD_HID), H2 * sizeof(float), st, src_a, lda, src_b, ldb, Hh, w0, b0, w3, b3, labels,
-               H2, nc, p, seed, offset, offset_dev, div_batch > 0 ? div_batch : B, last_out, hid_out, logits, dlogits, dhid, rowloss,
-               counter, loss_out, loss_sum_accum);
+    if (class_weight)
+        MMS_LAUNCH(head_ce_fused_kernel<true>, dim3(B), dim3(4 * HEAD_HID), H2 * sizeof(float), st, src_a, lda, src_b, ldb, Hh, w0, b0, w3,
+                   b3, labels, H2, nc, p, seed, offset, offset_dev, div_batch > 0 ? div_batch : B, last_out, hid_out, logits, dlogits,
+                   dhid, rowloss, counter, loss_out, loss_sum_accum, class_weight);
+    else
+        MMS_LAUNCH(head_ce_fused_kernel<false>, dim3(B), dim3(4 * HEAD_HID), H2 * sizeof(float), st, src_a, lda, src_b, ldb, Hh, w0, b0, w3,
+                   b3, labels, H2, nc, p, seed, offset, offset_dev, div_batch > 0 ? div_batch : B, last_out, hid_out, logits, dlogits,
+                   dhid, rowloss, counter, loss_out, loss_sum_accum, nullptr);
     MMS_LAUNCH_CHECK("head_ce_fused_kernel");
     return MMS_OK;
 }
@@ -347,12 +409,37 @@ int launch_head_bwd(const float* last, const float* hid, const float* dlogits, c
 }
 
 int launch_cross_entropy(const float* logits, const int64_t* labels, int B, int nc, float* loss_out, float* dlogits,
-                         double* loss_sum_accum, cudaStream_t st, int div_batch = 0) {
+                         double* loss_sum_accum, cudaStream_t st, int div_batch = 0, const float* class_weight = nullptr,
+                         const double* norm = nullptr) {
     if (div_batch <= 0) div_batch = B;
     MMS_REQUIRE(nc >= 1 && nc <= MAX_NC, "cross_entropy: num_classes %d outside [1,%d]", nc, MAX_NC);
+    MMS_REQUIRE(class_weight || !norm, "cross_entropy: a normaliser needs class weights");
     MMS_PROF_BEGIN(st);
-    MMS_LAUNCH(cross_entropy_kernel, dim3(1), dim3(256), 0, st, logits, labels, B, nc, loss_out, dlogits, loss_sum_accum, div_batch);
+    MMS_LAUNCH(cross_entropy_kernel, dim3(1), dim3(256), 0, st, logits, labels, B, nc, loss_out, dlogits, loss_sum_accum, div_batch,
+               class_weight, norm);
     MMS_LAUNCH_CHECK("cross_entropy_kernel");
+    return MMS_OK;
+}
+
+// out[0] = sum_b w[y_b] over the labels in [0, nc), float64, one warp in a fixed order: the local normaliser of the weighted
+// cross entropy, written into a slot the data-parallel exchange sums over the ranks.
+__global__ void __launch_bounds__(32) class_weight_sum_kernel(const int64_t* __restrict__ labels, int B, int nc,
+                                                              const float* __restrict__ class_weight, double* __restrict__ out) {
+    MMS_PDL_PROLOGUE();
+    double ws = 0.0;
+    for (int b = threadIdx.x; b < B; b += 32) {
+        const int64_t y = labels[b];
+        if (y >= 0 && y < nc) ws += (double)class_weight[y];
+    }
+    ws = warp_sum(ws);
+    if (threadIdx.x == 0) out[0] = ws;
+}
+
+int launch_class_weight_sum(const int64_t* labels, int B, int nc, const float* class_weight, double* out, cudaStream_t st) {
+    MMS_REQUIRE(nc >= 1 && nc <= MAX_NC, "class_weight_sum: num_classes %d outside [1,%d]", nc, MAX_NC);
+    MMS_PROF_BEGIN(st);
+    MMS_LAUNCH(class_weight_sum_kernel, dim3(1), dim3(32), 0, st, labels, B, nc, class_weight, out);
+    MMS_LAUNCH_CHECK("class_weight_sum_kernel");
     return MMS_OK;
 }
 
@@ -393,6 +480,18 @@ extern "C" int mms_cross_entropy_partial(const float* logits, const int64_t* lab
                                          mms_stream_t stream) {
     MMS_REQUIRE(logits && labels && loss_out && batch > 0 && global_batch >= batch, "cross_entropy_partial: bad arguments");
     return launch_cross_entropy(logits, labels, batch, num_classes, loss_out, dlogits, loss_sum_accum, (cudaStream_t)stream, global_batch);
+}
+extern "C" int mms_cross_entropy_weighted(const float* logits, const int64_t* labels, int32_t batch, int32_t num_classes,
+                                          const float* class_weight, const double* norm_dev, float* loss_out, float* dlogits,
+                                          double* loss_sum_accum, mms_stream_t stream) {
+    MMS_REQUIRE(logits && labels && loss_out && batch > 0, "cross_entropy_weighted: bad arguments");
+    return launch_cross_entropy(logits, labels, batch, num_classes, loss_out, dlogits, loss_sum_accum, (cudaStream_t)stream, batch,
+                                class_weight, norm_dev);
+}
+extern "C" int mms_class_weight_sum(const int64_t* labels, int32_t batch, int32_t num_classes, const float* class_weight,
+                                    double* out, mms_stream_t stream) {
+    MMS_REQUIRE(labels && class_weight && out && batch > 0, "class_weight_sum: bad arguments");
+    return launch_class_weight_sum(labels, batch, num_classes, class_weight, out, (cudaStream_t)stream);
 }
 extern "C" int mms_adam_flat_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n,
                                   const float* lr_dev, float beta1, float beta2, float eps, float weight_decay, int64_t* step_dev,

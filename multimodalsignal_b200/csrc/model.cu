@@ -35,10 +35,11 @@ int launch_head_fwd2(const float*, int64_t, const float*, int64_t, int, const fl
                      int, int, float, uint64_t, uint64_t, const int64_t*, float*, float*, float*, cudaStream_t);
 int launch_head_bwd(const float*, const float*, const float*, const float*, int, int, int, float, uint64_t, uint64_t,
                     const int64_t*, float*, float*, float*, float*, float*, cudaStream_t);
-int launch_cross_entropy(const float*, const int64_t*, int, int, float*, float*, double*, cudaStream_t, int div_batch);
+int launch_cross_entropy(const float*, const int64_t*, int, int, float*, float*, double*, cudaStream_t, int div_batch,
+                         const float* class_weight, const double* norm);
 int launch_head_ce_fused(const float*, int64_t, const float*, int64_t, int, const float*, const float*, const float*, const float*,
                          const int64_t*, int, int, int, float, uint64_t, uint64_t, const int64_t*, int, float*, float*, float*, float*,
-                         float*, float*, int32_t*, float*, double*, cudaStream_t);
+                         float*, float*, int32_t*, float*, double*, cudaStream_t, const float* class_weight);
 int launch_adam(float*, const float*, float*, float*, int64_t, const float*, float, float, float, float, int64_t*, int32_t*,
                 cudaStream_t);
 int launch_chan_dx(const float*, const float*, const float*, int, int, int, float*, cudaStream_t);
@@ -271,6 +272,7 @@ struct Dims {
     int B, Bg, C, T, nc, O, H, layers, A;      // Bg: global batch (== B unless data-parallel)
     int L1c, P1, L2c, L;   // conv1 out, pool1 out, conv2 out, pool2 out (= GRU sequence length)
     bool training, attention, need_grad, drop_gru, drop_head;
+    bool weighted;         // desc.class_weight set: one more float64 (the normaliser sum_b w[y_b]) after the BN2 sums
     float p;
 };
 
@@ -302,6 +304,7 @@ static int make_dims(const mms_cnngru_desc* d, Dims* o) {
     MMS_REQUIRE(o->p >= 0.f && o->p < 1.f, "dropout %f outside [0,1)", (double)o->p);
     o->drop_gru = o->training && o->p > 0.f && o->layers > 1;   // nn.GRU applies dropout only between layers
     o->drop_head = o->training && o->p > 0.f;
+    o->weighted = d->class_weight != nullptr;
     return MMS_OK;
 }
 
@@ -370,11 +373,14 @@ static void carve(const Dims& m, char* base, Workspace* w) {
     };
     const int64_t B = m.B, L = m.L, H = m.H, M = B * L;
     const int64_t f = sizeof(float);
-    w->fwd_zero_bytes = sizeof(double) * 2 * (CONV1_CO + m.O) + 16;        // BN batch sums + the fused head's CTA counter
+    // BN batch sums (+ with class weights the weighted loss's normaliser, summed over the ranks with the BN2 sums) + the fused
+    // head's CTA counter
+    const int wslot = m.weighted ? 1 : 0;
+    w->fwd_zero_bytes = sizeof(double) * (2 * (CONV1_CO + m.O) + wslot) + 16;
     w->fwd_zero = take((int64_t)w->fwd_zero_bytes);
     w->stats1 = (double*)w->fwd_zero;
     w->stats2 = w->stats1 ? w->stats1 + 2 * CONV1_CO : nullptr;
-    w->head_counter = w->stats1 ? (int32_t*)(w->stats2 + 2 * m.O) : nullptr;
+    w->head_counter = w->stats1 ? (int32_t*)(w->stats2 + 2 * m.O + wslot) : nullptr;
     const int64_t bz = (int64_t)sizeof(double) * 2 * (CONV1_CO + m.O) + align_up(B * m.C, 4) * f + align_up(B, 4) * (int64_t)sizeof(int);
     w->bwd_zero = take(bz);
     w->red1 = (double*)w->bwd_zero;
@@ -629,7 +635,7 @@ static int model_forward(const mms_cnngru_desc* d, const float* x, const float* 
         return launch_head_ce_fused(w.hs_tf + (int64_t)(L - 1) * H, (int64_t)L * H, w.h_tr, H, H, P + po.fc0_w, P + po.fc0_b,
                                     P + po.fc3_w, P + po.fc3_b, fl->labels, B, 2 * H, m.nc, m.drop_head ? m.p : 0.f, d->rng_seed,
                                     d->rng_offset, d->rng_offset_dev, m.Bg, w.last, w.hid, logits, w.dlogits, w.dhid, w.rowloss,
-                                    w.head_counter, fl->loss_out, fl->loss_sum_accum, st);
+                                    w.head_counter, fl->loss_out, fl->loss_sum_accum, st, d->class_weight);
     return launch_head_fwd2(w.hs_tf + (int64_t)(L - 1) * H, (int64_t)L * H, w.h_tr, H, H, P + po.fc0_w, P + po.fc0_b, P + po.fc3_w,
                             P + po.fc3_b, B, 2 * H, m.nc, m.drop_head ? m.p : 0.f, d->rng_seed, d->rng_offset, d->rng_offset_dev,
                             w.last, w.hid, logits, st);
@@ -1004,7 +1010,7 @@ extern "C" int mms_cnngru_sync_offsets(const mms_cnngru_desc* d, int64_t* byte_o
     char* base = reinterpret_cast<char*>(4096);          // any non-null base: only differences are used
     carve(m, base, &w);
     byte_offsets_host[0] = (char*)w.stats1 - base; counts_host[0] = 2 * CONV1_CO;
-    byte_offsets_host[1] = (char*)w.stats2 - base; counts_host[1] = 2 * m.O;
+    byte_offsets_host[1] = (char*)w.stats2 - base; counts_host[1] = 2 * m.O + (m.weighted ? 1 : 0);   // + sum_b w[y_b]
     byte_offsets_host[2] = (char*)w.red1 - base;   counts_host[2] = 2 * CONV1_CO;
     byte_offsets_host[3] = (char*)w.red2 - base;   counts_host[3] = 2 * m.O;
     return MMS_OK;
@@ -1021,6 +1027,9 @@ extern "C" int mms_cnngru_train_step(const mms_cnngru_desc* d, const float* x, c
     if (rc) return rc;
     MMS_REQUIRE(m.training && m.need_grad, "train_step: descriptor must have training = need_grad = 1");
     MMS_REQUIRE(labels && grads && exp_avg && exp_avg_sq && loss_out && lr_dev && step_dev && scratch_dev, "train_step: null pointer");
+    // the weighted loss is normalised by sum_b w[y_b] of THIS batch; a rank's share of a larger batch needs the global sum
+    // (mms_cnngru_sync_offsets + mms_cross_entropy_weighted)
+    MMS_REQUIRE(!m.weighted || m.Bg == m.B, "train_step: class weights with global_batch %d > batch %d", m.Bg, m.B);
     ParamOff po;
     make_params(m, &po);
     Workspace w;
@@ -1034,7 +1043,8 @@ extern "C" int mms_cnngru_train_step(const mms_cnngru_desc* d, const float* x, c
     rc = model_forward(d, x, params, bn_buffers, num_batches_tracked, workspace, logits, st, 7, fuse_head ? &fl : nullptr);  // trainer.py:146-147
     if (rc) return rc;
     if (!fuse_head) {
-        rc = launch_cross_entropy(logits, labels, m.B, m.nc, loss_out, w.dlogits, loss_sum_accum, st, m.Bg);  // trainer.py:147
+        rc = launch_cross_entropy(logits, labels, m.B, m.nc, loss_out, w.dlogits, loss_sum_accum, st, m.Bg, d->class_weight,
+                                  nullptr);                                                                // trainer.py:147
         if (rc) return rc;
     }
     rc = model_backward(d, x, params, bn_buffers, workspace, w.dlogits, grads, nullptr, st, 7, fuse_head, zero_bwd);        // trainer.py:148

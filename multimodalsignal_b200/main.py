@@ -44,6 +44,7 @@ BATCH_SIZE = 64
 LEARNING_RATE = 0.001
 PATIENCE = 20
 WEIGHTS_DECAY = 1e-4
+USE_CLASS_WEIGHTS = False                     # class-weighted CrossEntropyLoss, 'balanced' weights (never enabled upstream, SURVEY D9)
 ALL_SUBJECTS = [f"S{i}" for i in range(2, 18) if i != 12]
 CONCURRENT_FOLDS = int(os.environ.get("MMS_CONCURRENT_FOLDS", "1"))     # folds interleaved per GPU (new; 1 = the reference's loop)
 
@@ -65,7 +66,7 @@ def folds_for_rank(n_folds: int, rank: int, world: int):
 def trainer_config():
     return {'trainer': {'epochs': EPOCHS, 'learning_rate': LEARNING_RATE,
                         'early_stopping': {'enabled': True, 'patience': PATIENCE, 'delta': 0},
-                        'weight_decay': WEIGHTS_DECAY}}
+                        'weight_decay': WEIGHTS_DECAY, 'use_class_weights': USE_CLASS_WEIGHTS}}
 
 
 def run_fold_async(fold_index, subject_to_test, run_output_dir, all_channel_names, subject_streams=None, stream=None,

@@ -32,15 +32,21 @@ class DataParallelTrainStep:
     """One rank's share of a data-parallel training step.  ``local_batch`` rows of a ``global_batch`` batch."""
 
     def __init__(self, model, optimizer: FlatAdam, local_batch: int, global_batch: int, seq_len: int, rank: int = 0, group=None,
-                 peer=None, use_graph: bool = True):
+                 peer=None, use_graph: bool = True, class_weight=None):
         """``peer``: None = ``torch.distributed`` all-reduces (NCCL); ``"symm"`` = symmetric memory + the peer kernels
         (one process per GPU, needs an initialised process group); a ``LocalPeers`` registry = several ranks emulated
-        inside one process on one GPU (tests)."""
+        inside one process on one GPU (tests).
+
+        ``class_weight`` (``num_classes`` values, the same on every rank): ``CrossEntropyLoss(weight=...)`` over the
+        GLOBAL batch.  Its normaliser sum_b w[y_b] needs every rank's labels; it travels as one more double at the end
+        of the BN2 sum vector (``mms_cnngru_sync_offsets``), so the existing exchange sums it and no message is added."""
+        from .trainer import class_weight_tensor
         self.lib = _ext.lib()
         self.model, self.opt, self.group = model, optimizer, group
         self.peer, self.rank = peer, rank
         self.flat = model.flat_parameters()
         dev = self.flat.device
+        self.class_weight = None if class_weight is None else class_weight_tensor(class_weight, model.num_classes, dev)
         d = CnnGruDesc()
         d.batch, d.in_channels, d.seq_len, d.num_classes = local_batch, model.in_channels, seq_len, model.num_classes
         d.cnn_out, d.hidden, d.layers = model.cnn_out_channels, model.gru_hidden_size, model.gru_num_layers
@@ -49,6 +55,7 @@ class DataParallelTrainStep:
         d.rng_seed, d.rng_offset = (model._rng_seed ^ (0x9E3779B9 * (rank + 1))) & 0xFFFFFFFFFFFFFFFF, 0
         d.rng_offset_dev = optimizer.step_dev.data_ptr()
         d.global_batch = global_batch
+        d.class_weight = None if self.class_weight is None else self.class_weight.data_ptr()
         self.desc = d
         self.local_batch, self.global_batch = local_batch, global_batch
         nbytes = self.lib.mms_cnngru_workspace_bytes(C.byref(d))
@@ -60,6 +67,7 @@ class DataParallelTrainStep:
         check(self.lib.mms_cnngru_sync_offsets(C.byref(d), offs, cnts))
         view = lambda i: self.workspace[offs[i]:offs[i] + 8 * cnts[i]].view(torch.float64)
         self.stats1, self.stats2, self.red1, self.red2 = view(0), view(1), view(2), view(3)
+        self.weight_sum = self.stats2[-1:] if self.class_weight is not None else None     # sum_b w[y_b], summed over the ranks
         self.logits = torch.zeros(local_batch, model.num_classes, dtype=torch.float32, device=dev)
         self.dlogits = torch.zeros_like(self.logits)
         self.loss = torch.zeros(1, dtype=torch.float32, device=dev)        # this rank's share of the global mean
@@ -121,14 +129,14 @@ class DataParallelTrainStep:
         x, y, o, g = self.x, self.y, self.opt, self.opt.param_groups[0]
         o.grads.zero_()                                          # trainer.py:144
         self._fwd(1, x)
+        self._weight_sum(y)
         self._peer_sum(0)                                        # SyncBN stage 1
         yield
         self._fwd(2, x)
-        self._peer_sum(1)
+        self._peer_sum(1)                                        # (+ the weighted loss's normaliser)
         yield
         self._fwd(4, x)                                          # trainer.py:146
-        check(self.lib.mms_cross_entropy_partial(ptr(self.logits), ptr(y), self.local_batch, self.model.num_classes,
-                                                 self.global_batch, ptr(self.loss), ptr(self.dlogits), None, stream()))   # :147
+        self._loss(y)                                            # :147
         self._bwd(1, x)                                          # trainer.py:148
         self._peer_sum(3)                                        # SyncBN backward, stage 2
         yield
@@ -157,6 +165,22 @@ class DataParallelTrainStep:
             self.graph = capture_graph(self._enqueue_peer)
         self.graph.replay()
 
+    def _weight_sum(self, y):
+        """Local sum_b w[y_b] into the extra slot of the BN2 sum vector (after forward phase 1 cleared it)."""
+        if self.class_weight is not None:
+            check(self.lib.mms_class_weight_sum(ptr(y), self.local_batch, self.model.num_classes, ptr(self.class_weight),
+                                                ptr(self.weight_sum), stream()))
+
+    def _loss(self, y):
+        """This rank's share of the global mean loss and its dlogits (trainer.py:147)."""
+        if self.class_weight is None:
+            check(self.lib.mms_cross_entropy_partial(ptr(self.logits), ptr(y), self.local_batch, self.model.num_classes,
+                                                     self.global_batch, ptr(self.loss), ptr(self.dlogits), None, stream()))
+        else:
+            check(self.lib.mms_cross_entropy_weighted(ptr(self.logits), ptr(y), self.local_batch, self.model.num_classes,
+                                                      ptr(self.class_weight), ptr(self.weight_sum), ptr(self.loss),
+                                                      ptr(self.dlogits), None, stream()))
+
     def _fwd(self, phases, x):
         m = self.model
         check(self.lib.mms_cnngru_forward_phase(C.byref(self.desc), phases, ptr(x), ptr(self.flat), ptr(m._bn_flat), ptr(m._nbt_flat),
@@ -173,12 +197,12 @@ class DataParallelTrainStep:
         y = y.contiguous()
         self.opt.grads.zero_()                                   # trainer.py:144
         self._fwd(1, x)
+        self._weight_sum(y)
         yield self.stats1                                        # SyncBN, stage 1: (sum, sum of squares) per channel
         self._fwd(2, x)
-        yield self.stats2
+        yield self.stats2                                        # (+ sum_b w[y_b] with class weights)
         self._fwd(4, x)                                          # trainer.py:146
-        check(self.lib.mms_cross_entropy_partial(ptr(self.logits), ptr(y), self.local_batch, self.model.num_classes,
-                                                 self.global_batch, ptr(self.loss), ptr(self.dlogits), None, stream()))   # :147
+        self._loss(y)                                            # :147
         self._bwd(1, x)                                          # trainer.py:148
         yield self.red2                                          # SyncBN backward, stage 2: (sum dy, sum dy*xhat)
         self._bwd(2, x)

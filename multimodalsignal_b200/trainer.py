@@ -235,17 +235,30 @@ class FlatAdam(torch.optim.Optimizer):
                                      ptr(self.step_dev), ptr(self.scratch), stream()))
 
 
+def class_weight_tensor(weight, num_classes, device):
+    """``weight`` (a sequence or tensor of ``num_classes`` values) as a contiguous float32 tensor on ``device``."""
+    w = torch.as_tensor(weight, dtype=torch.float32).detach().reshape(-1)
+    if w.numel() != num_classes:
+        raise ValueError(f"class weights: expected {num_classes} values, got {w.numel()}")
+    return w.to(device).contiguous()
+
+
 class FusedTrainStep:
     """One training step = one ``mms_cnngru_train_step`` call, captured once per batch shape into
     a CUDA graph and replayed.  ``__call__(x, y)`` accepts device tensors or pinned host tensors
-    (copied into the static graph inputs on the current stream)."""
+    (copied into the static graph inputs on the current stream).
 
-    def __init__(self, model, optimizer: FlatAdam, batch: int, seq_len: int, use_graph: bool = True, source=None, loss_sum=None):
+    ``class_weight`` (``num_classes`` values) makes the loss ``CrossEntropyLoss(weight=class_weight)``.  The values
+    live in a device tensor whose address the graph holds: ``set_class_weight`` changes them with a copy, no re-capture."""
+
+    def __init__(self, model, optimizer: FlatAdam, batch: int, seq_len: int, use_graph: bool = True, source=None, loss_sum=None,
+                 class_weight=None):
         self.lib = _ext.lib()
         self.model, self.opt = model, optimizer
         self.source = source            # DeviceBatchSource: the batch is gathered on the device inside the graph
         self.flat = model.flat_parameters()
         dev = self.flat.device
+        self.class_weight = None if class_weight is None else class_weight_tensor(class_weight, model.num_classes, dev)
         self.x = torch.zeros(batch, model.in_channels, seq_len, dtype=torch.float32, device=dev)
         self.y = torch.zeros(batch, dtype=torch.int64, device=dev)
         self.logits = torch.zeros(batch, model.num_classes, dtype=torch.float32, device=dev)
@@ -258,6 +271,7 @@ class FusedTrainStep:
         d.dropout_p = float(model.dropout_p)
         d.rng_seed, d.rng_offset = model._rng_seed ^ 0x5DEECE66D, 0
         d.rng_offset_dev = optimizer.step_dev.data_ptr()      # dropout stream advances with the step count
+        d.class_weight = None if self.class_weight is None else self.class_weight.data_ptr()
         self.desc = d
         nbytes = self.lib.mms_cnngru_workspace_bytes(C.byref(d))
         if nbytes < 0:
@@ -267,6 +281,12 @@ class FusedTrainStep:
         self.graph = None
         self.calls = 0
         self.kernels_per_step = None
+
+    def set_class_weight(self, weight):
+        """New class weights for the following steps (a stream-ordered copy into the tensor the graph reads)."""
+        if self.class_weight is None:
+            raise _ext.MmsError("FusedTrainStep was built without class weights")
+        self.class_weight.copy_(class_weight_tensor(weight, self.model.num_classes, self.class_weight.device), non_blocking=True)
 
     def _enqueue(self):
         m, o, g = self.model, self.opt, self.opt.param_groups[0]
@@ -388,13 +408,19 @@ class DeviceBatchSource:
 
 class EvalStep:
     """One evaluation batch (reference trainer.py:213-228) = eval-mode forward + ``mms_eval_accumulate``
-    (summed loss, arg-max predictions, confusion counts) on static buffers, replayed as a CUDA graph."""
+    (summed loss, arg-max predictions, confusion counts) on static buffers, replayed as a CUDA graph.
 
-    def __init__(self, model, batch, seq_len, confusion, loss_sum, use_graph=True):
+    With ``class_weight`` the loss is ``CrossEntropyLoss(weight=class_weight)`` accumulated per group of ``group``
+    consecutive rows (the evaluation loader's batch size; None: the whole batch is one group), each group adding
+    ``n * weighted_mean`` as the reference adds ``loss.item() * batch`` per loader batch."""
+
+    def __init__(self, model, batch, seq_len, confusion, loss_sum, use_graph=True, class_weight=None, group=None):
         self.lib = _ext.lib()
         self.model = model
         self.flat = model.flat_parameters()
         dev = self.flat.device
+        self.class_weight = None if class_weight is None else class_weight_tensor(class_weight, model.num_classes, dev)
+        self.group = int(group) if group else batch
         self.x = torch.zeros(batch, model.in_channels, seq_len, dtype=torch.float32, device=dev)
         self.y = torch.zeros(batch, dtype=torch.int64, device=dev)
         self.logits = torch.zeros(batch, model.num_classes, dtype=torch.float32, device=dev)
@@ -407,8 +433,13 @@ class EvalStep:
         m, e = self.model, self.engine
         check(self.lib.mms_cnngru_forward(C.byref(e.desc), ptr(self.x), ptr(self.flat), ptr(m._bn_flat), ptr(m._nbt_flat),
                                           ptr(e.workspace), ptr(self.logits), stream()))
-        check(self.lib.mms_eval_accumulate(ptr(self.logits), ptr(self.y), self.x.shape[0], m.num_classes, ptr(self.pred),
-                                           ptr(self.confusion), ptr(self.loss_sum), stream()))
+        if self.class_weight is None:
+            check(self.lib.mms_eval_accumulate(ptr(self.logits), ptr(self.y), self.x.shape[0], m.num_classes, ptr(self.pred),
+                                               ptr(self.confusion), ptr(self.loss_sum), stream()))
+        else:
+            check(self.lib.mms_eval_accumulate_weighted(ptr(self.logits), ptr(self.y), self.x.shape[0], m.num_classes,
+                                                        ptr(self.class_weight), self.group, ptr(self.pred), ptr(self.confusion),
+                                                        ptr(self.loss_sum), stream()))
 
     def run(self):
         if self.model._flat is not self.flat:
@@ -437,29 +468,74 @@ def metrics_from_confusion(conf):
     return float(tp.sum() / total), float((f1 * support).sum() / total)
 
 
+def balanced_class_weights(labels, num_classes):
+    """The class weights ``Trainer`` uses with ``use_class_weights``: sklearn's
+    ``compute_class_weight('balanced', classes=range(num_classes), y=labels)``, w_c = N / (num_classes * count_c).
+    The reference computes its weights at trainer.py:81-94 in a branch that never runs; its formula is not
+    available, so this project defines the option as ``'balanced'``.  ``labels``: numpy array or (CUDA) tensor.
+    A class without training windows or a label outside [0, num_classes) raises."""
+    if isinstance(labels, torch.Tensor):
+        labels = labels.detach().to("cpu").numpy()
+    y = np.asarray(labels).reshape(-1).astype(np.int64)
+    if y.size == 0:
+        raise ValueError("class weights: the training set is empty")
+    if y.min() < 0 or y.max() >= num_classes:
+        raise ValueError(f"class weights: labels outside [0, {num_classes})")
+    counts = np.bincount(y, minlength=num_classes)
+    missing = [c for c in range(num_classes) if counts[c] == 0]
+    if missing:
+        raise ValueError(f"class weights: class {missing[0]} has no training windows"
+                         + (f" (nor do classes {missing[1:]})" if len(missing) > 1 else ""))
+    return y.size / (num_classes * counts.astype(np.float64))
+
+
 class _CrossEntropy(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, logits, labels):
+    def forward(ctx, logits, labels, weight=None):
         lib = _ext.lib()
         logits = logits.contiguous().float()
         loss = torch.empty(1, dtype=torch.float32, device=logits.device)
         dlogits = torch.empty_like(logits)
-        check(lib.mms_cross_entropy(ptr(logits), ptr(labels.contiguous()), logits.shape[0], logits.shape[1], ptr(loss),
-                                    ptr(dlogits), None, stream()))
+        if weight is None:
+            check(lib.mms_cross_entropy(ptr(logits), ptr(labels.contiguous()), logits.shape[0], logits.shape[1], ptr(loss),
+                                        ptr(dlogits), None, stream()))
+        else:
+            check(lib.mms_cross_entropy_weighted(ptr(logits), ptr(labels.contiguous()), logits.shape[0], logits.shape[1],
+                                                 ptr(weight), None, ptr(loss), ptr(dlogits), None, stream()))
         ctx.save_for_backward(dlogits)
         return loss[0]
 
     @staticmethod
     def backward(ctx, g):
         (dlogits,) = ctx.saved_tensors
-        return dlogits * g, None
+        return dlogits * g, None, None
 
 
 class CrossEntropyLoss(torch.nn.Module):
-    """``torch.nn.CrossEntropyLoss()`` (mean reduction, reference trainer.py:69) on the CUDA kernel."""
+    """``torch.nn.CrossEntropyLoss()`` (mean reduction, reference trainer.py:69) on the CUDA kernel.
+
+    ``weight`` (``num_classes`` values, a sequence or tensor) is ``CrossEntropyLoss(weight=...)``:
+    ``sum_b w[y_b] l_b / sum_b w[y_b]``.  The other options of torch's loss (``ignore_index``, ``label_smoothing``,
+    a reduction other than ``'mean'``) are not implemented and raise."""
+
+    def __init__(self, weight=None, size_average=None, ignore_index=-100, reduce=None, reduction='mean', label_smoothing=0.0):
+        super().__init__()
+        if size_average is not None or reduce is not None or reduction != 'mean':
+            raise NotImplementedError("CrossEntropyLoss: only reduction='mean' is implemented")
+        if ignore_index != -100:
+            raise NotImplementedError("CrossEntropyLoss: ignore_index is not implemented")
+        if label_smoothing != 0.0:
+            raise NotImplementedError("CrossEntropyLoss: label_smoothing is not implemented")
+        self.weight = None if weight is None else torch.as_tensor(weight, dtype=torch.float32).detach().reshape(-1)
 
     def forward(self, logits, labels):
-        return _CrossEntropy.apply(logits, labels)
+        if self.weight is None:
+            return _CrossEntropy.apply(logits, labels)
+        if self.weight.numel() != logits.shape[1]:
+            raise ValueError(f"CrossEntropyLoss: {self.weight.numel()} class weights for {logits.shape[1]} classes")
+        if self.weight.device != logits.device:
+            self.weight = self.weight.to(logits.device).contiguous()
+        return _CrossEntropy.apply(logits, labels, self.weight)
 
 
 _WRITER = None
@@ -506,7 +582,11 @@ class Trainer:
         t = config['trainer']
         self.epochs, self.learning_rate = t['epochs'], t['learning_rate']
         self.patience, self.weight_decay = t['early_stopping']['patience'], t['weight_decay']
-        self.use_class_weights = t.get('use_class_weights', False)     # never enabled upstream (SURVEY D9)
+        # never enabled upstream (SURVEY D9); here an opt-in with the intended behaviour: balanced_class_weights of the
+        # training labels, fixed by the first train(), used by every later step and evaluation
+        self.use_class_weights = t.get('use_class_weights', False)
+        self.class_weights = None                                      # list of num_classes floats once fixed
+        self._class_weight = None                                      # the same on the device
         self.use_graph = t.get('cuda_graph', True)
         self.quiet = t.get('quiet', False)                             # log to the file only
 
@@ -554,16 +634,31 @@ class Trainer:
         key = (batch, seq_len, id(source))
         if key not in self._steps:
             self._steps[key] = FusedTrainStep(self.model, self.optimizer, batch, seq_len, use_graph=self.use_graph, source=source,
-                                              loss_sum=self._train_loss)
+                                              loss_sum=self._train_loss, class_weight=self._class_weight)
         return self._steps[key]
 
-    def _eval_step(self, batch, seq_len):
-        key = (batch, seq_len)
+    def _eval_step(self, batch, seq_len, group=None):
+        key = (batch, seq_len, group)
         st = self._eval_steps.get(key)
         if st is None or st.flat is not self.model._flat:
-            st = EvalStep(self.model, batch, seq_len, self._eval_conf, self._eval_loss, use_graph=self.use_graph)
+            st = EvalStep(self.model, batch, seq_len, self._eval_conf, self._eval_loss, use_graph=self.use_graph,
+                          class_weight=self._class_weight, group=group)
             self._eval_steps[key] = st
         return st
+
+    def _fix_class_weights(self, train_loader):
+        """``use_class_weights``: the first ``train()`` fixes sklearn's ``'balanced'`` weights of the training labels."""
+        if not self.use_class_weights or self._class_weight is not None:
+            return
+        labels = getattr(train_loader.dataset, 'labels', None)
+        if labels is None:
+            raise ValueError("use_class_weights: the training dataset has no .labels to compute class weights from")
+        w = balanced_class_weights(labels, self.model.num_classes)
+        self.class_weights = [float(v) for v in w]
+        with self._on_stream():
+            self._class_weight = torch.tensor(self.class_weights, dtype=torch.float32, device=self.device)
+        self.criterion = CrossEntropyLoss(weight=self._class_weight)
+        self._log("Class weights ('balanced'): " + ", ".join(f"{v:.4f}" for v in self.class_weights))
 
     @staticmethod
     def _check_batch(batch):
@@ -623,6 +718,7 @@ class Trainer:
         return drive(self.train_async(train_loader, val_loader))
 
     def train_async(self, train_loader, val_loader):
+        self._fix_class_weights(train_loader)
         best_val_acc = 0
         for epoch in range(self.epochs):
             t0 = time.time()
@@ -679,9 +775,14 @@ class Trainer:
             ds = data_loader.dataset
             n, T = len(ds), int(ds.data.shape[2])
             n_eval = n if not data_loader.drop_last else (n // data_loader.batch_size) * data_loader.batch_size
-            for i in range(0, n_eval, self.EVAL_CHUNK):
-                b = min(self.EVAL_CHUNK, n_eval - i)
-                st = self._eval_step(b, T)
+            chunk, group = self.EVAL_CHUNK, None
+            if self._class_weight is not None:
+                # the weighted loss is a per-loader-batch mean: slices hold whole loader batches, each one group
+                group = data_loader.batch_size
+                chunk = group if group > self.EVAL_CHUNK else (self.EVAL_CHUNK // group) * group
+            for i in range(0, n_eval, chunk):
+                b = min(chunk, n_eval - i)
+                st = self._eval_step(b, T, group)
                 st.x.copy_(ds.data[i:i + b])
                 st.y.copy_(ds.labels[i:i + b])
                 st.run()
@@ -716,6 +817,8 @@ class Trainer:
     def evaluate_async(self, data_loader, want_lists=False):
         """Generator form of ``evaluate``: yields the CUDA event that marks the read-back, then returns
         ``(loss, acc, f1)`` (plus the prediction / label arrays with ``want_lists``)."""
+        if self.use_class_weights and self._class_weight is None:
+            raise ValueError("use_class_weights: the class weights are fixed by the first train(); evaluate() cannot run before it")
         t0 = time.time()
         with self._on_stream():
             done, n_seen, lists = self._enqueue_evaluate(data_loader, want_lists)
