@@ -135,6 +135,28 @@ int mms_cnngru_backward(const mms_cnngru_desc* d, const float* x, const float* p
                         const float* bn_buffers, void* workspace, const float* dlogits,
                         float* grads, float* dx, mms_stream_t stream);
 
+/* Input gradient only (attribution): after mms_cnngru_forward with training = 0 and need_grad = 1 on the same workspace,
+ * dx [B,C,T] = d(sum_b,c dlogits[b,c] logits[b,c]) / dx.  No parameter gradient is formed: no weight-gradient product,
+ * conv or head weight gradient or side-stream work is launched, and everything runs on `stream`.  In eval mode BatchNorm
+ * uses the running statistics, so the rows of the batch are independent.  Any other training / need_grad combination
+ * is MMS_E_INVALID. */
+int mms_cnngru_input_gradient(const mms_cnngru_desc* d, const float* x, const float* params,
+                              const float* bn_buffers, void* workspace, const float* dlogits,
+                              float* dx, mms_stream_t stream);
+
+/* Integrated gradients over B windows of n = C*T samples with `steps` midpoint-rule steps, alpha_k = (k + 1/2) / steps.
+ * Interpolation row r = b * steps + k.  x0 is the baseline: [B,C,T] with x0_per_window = 1, or one [C,T] shared by every
+ * window with x0_per_window = 0.  A chunk is the rows [row0, row0 + nrows).
+ * mms_ig_interpolate: z [nrows,C,T] = x0 + alpha_k (x - x0) and dlogits [nrows,num_classes] = one_hot(target[b]).
+ * mms_ig_accumulate : A [B,C,T] += (x - x0) * dx / steps and S [B,C] (float64) += its sum over t, for dx [nrows,C,T] the
+ *                     input gradient of the chunk.  Each element sums over k in increasing order, so A does not depend on
+ *                     how the rows are chunked (chunks must be accumulated in row order; S to float64 rounding). */
+int mms_ig_interpolate(const float* x, const float* x0, int32_t x0_per_window, const int64_t* target, int32_t B,
+                       int32_t C, int32_t T, int32_t num_classes, int32_t steps, int64_t row0, int32_t nrows, float* z,
+                       float* dlogits, mms_stream_t stream);
+int mms_ig_accumulate(const float* x, const float* x0, int32_t x0_per_window, const float* dx, int32_t B, int32_t C,
+                      int32_t T, int32_t steps, int64_t row0, int32_t nrows, float* A, double* S, mms_stream_t stream);
+
 /* Data-parallel form of the two calls above (SURVEY §8e: intra-fold DP).  `phases` is a bit mask:
  *   forward : 1 = gate + conv1 (+BN1 sums) | 2 = BN1/pool1 + conv2 (+BN2 sums) | 4 = the rest
  *   backward: 1 = head..GRU..stage-2 pool/ReLU backward (+BN2 reductions) | 2 = stage-2 BN apply, conv2

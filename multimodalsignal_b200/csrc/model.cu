@@ -944,6 +944,115 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
     return fk.join();       // every gradient is complete before the caller's next kernel (Adam)
 }
 
+int launch_encoder_eval_bwd(const float*, const float*, const float*, const float*, const float*, const float*, const float*,
+                            const float*, const float*, int, int, int, float*, cudaStream_t);
+int launch_attn_input_grad(const float*, const float*, const float*, const float*, const float*, int, int, int, float*, cudaStream_t);
+int launch_head_input_grad(const float*, const float*, const float*, int, int, float*, cudaStream_t);
+
+// dx only, after an eval-mode forward with need_grad = 1 (attribution): the head, GRU and encoder input gradients of
+// model_backward without a single parameter gradient, all on the caller's stream.  The GRU recurrences and the NT input-gradient
+// products are model_backward's; the head and the encoder use the eval-mode kernels of conv_eval_bwd.cu, where BatchNorm is an
+// affine map and the pool / ReLU / BN backward of both stages folds into one launch with conv2's input gradient.
+static int model_input_gradient(const mms_cnngru_desc* d, const float* x, const float* P, const float* bn, void* ws,
+                                const float* dlogits, float* dx, cudaStream_t st) {
+    Dims m;
+    int rc = make_dims(d, &m);
+    if (rc) return rc;
+    MMS_REQUIRE(!m.training && m.need_grad, "cnngru_input_gradient: needs an eval-mode forward (training = 0, need_grad = 1)");
+    MMS_REQUIRE(x && P && bn && ws && dlogits && dx, "cnngru_input_gradient: null pointer");
+    ParamOff po;
+    make_params(m, &po);
+    Workspace w;
+    carve(m, (char*)ws, &w);
+    const int B = m.B, H = m.H, L = m.L;
+    const int M = B * L;
+    const bool tc_bwd = use_tc() && M >= TC_MIN_ROWS;      // W_ih^T for the tensor-core products: made by the forward pass
+
+    rc = launch_head_input_grad(w.hid, dlogits, P + po.fc3_w, B, m.nc, w.dhid, st);
+    if (rc) return rc;
+    const int top = m.layers - 1;
+    const int I_top = top == 0 ? m.O : 2 * H;
+    float* dxcur = w.dxa;
+    float* dxnext = w.dxb;
+    {
+        mms_gru_dir_bwd dirs[2];
+        memset(dirs, 0, sizeof(dirs));
+        dirs[0].w_hh = P + po.w_hh[top];
+        dirs[0].stash = w.stash_tf; dirs[0].st_bs = (int64_t)L * 4 * H; dirs[0].st_ts = 4 * H;
+        dirs[0].hs = w.hs_tf; dirs[0].hs_bs = (int64_t)L * H; dirs[0].hs_ts = H;
+        dirs[0].dh_head = w.dhid; dirs[0].w0 = P + po.fc0_w; dirs[0].w0_ld = 2 * H; dirs[0].w0_col = 0;
+        dirs[0].D = w.D_tf; dirs[0].d_bs = (int64_t)L * 4 * H; dirs[0].d_ts = 4 * H;
+        dirs[0].t0 = 0; dirs[0].dt = 1; dirs[0].nsteps = L;
+        dirs[1].w_hh = P + po.w_hh[top] + (int64_t)3 * H * H;
+        dirs[1].stash = w.stash_tr; dirs[1].st_bs = 4 * H; dirs[1].st_ts = 0;
+        dirs[1].hs = w.h_tr; dirs[1].hs_bs = H; dirs[1].hs_ts = 0;
+        dirs[1].dh_head = w.dhid; dirs[1].w0 = P + po.fc0_w; dirs[1].w0_ld = 2 * H; dirs[1].w0_col = H;
+        dirs[1].D = w.D_tr; dirs[1].d_bs = 4 * H; dirs[1].d_ts = 0;
+        dirs[1].t0 = L - 1; dirs[1].dt = -1; dirs[1].nsteps = 1;
+        rc = launch_gru_bwd(dirs, 2, B, H, 0.f, d->rng_seed, d->rng_offset, d->rng_offset_dev, st);
+        if (rc) return rc;
+        const float* w_rev = P + po.w_ih[top] + (int64_t)3 * H * I_top;
+        if (top >= 1) {      // the single reverse step's B rows, added by the layer underneath at t = L-1
+            if (gemm_skinny_supported(w.D_tr, 4 * H, w_rev, I_top, 0, B, I_top, 3 * H))
+                rc = launch_gemm_skinny(w.D_tr, 4 * H, w_rev, I_top, 0, nullptr, w.dx_extra, I_top, B, I_top, 3 * H, 0, 0,
+                                        (int64_t)L * I_top, 0.f, d->rng_seed, d->rng_offset, d->rng_offset_dev, st);
+            else
+                rc = launch_gemm_nn(w.D_tr, 4 * H, w_rev, I_top, w.dx_extra, I_top, B, I_top, 3 * H, 0, st);
+            if (rc) return rc;
+        }
+        if (tc_bwd && tc_gemm_supported(w.D_tf, 4 * H, w.wT_top, 3 * H, M, I_top, 3 * H))
+            rc = launch_tc_gemm_nt(w.D_tf, 4 * H, w.wT_top, 3 * H, nullptr, dxcur, I_top, M, I_top, 3 * H, 0, st);
+        else
+            rc = launch_gemm_nn(w.D_tf, 4 * H, P + po.w_ih[top], I_top, dxcur, I_top, M, I_top, 3 * H, 0, st);
+        if (rc) return rc;
+        if (top == 0) {
+            rc = launch_gemm_nn(w.D_tr, 4 * H, w_rev, I_top, dxcur + (int64_t)(L - 1) * I_top, (int64_t)L * I_top, B, I_top, 3 * H,
+                                1, st);
+            if (rc) return rc;
+        }
+    }
+    for (int l = top - 1; l >= 0; --l) {
+        const int I_l = l == 0 ? m.O : 2 * H;
+        mms_gru_dir_bwd dirs[2];
+        memset(dirs, 0, sizeof(dirs));
+        for (int dd = 0; dd < 2; ++dd) {
+            mms_gru_dir_bwd& g = dirs[dd];
+            g.w_hh = P + po.w_hh[l] + (int64_t)dd * 3 * H * H;
+            g.stash = w.stash[l] + (int64_t)dd * M * 4 * H; g.st_bs = (int64_t)L * 4 * H; g.st_ts = 4 * H;
+            g.hs = w.hs[l] + dd * H; g.hs_bs = (int64_t)L * 2 * H; g.hs_ts = 2 * H;
+            g.dout = dxcur + dd * H; g.do_bs = (int64_t)L * 2 * H; g.do_ts = 2 * H;
+            if (l == top - 1) { g.dout_last = w.dx_extra + dd * H; g.dl_ld = 2 * H; g.dl_at_first = dd; }
+            g.D = w.D[l] + dd * 4 * H; g.d_bs = (int64_t)L * 8 * H; g.d_ts = 8 * H;
+            g.t0 = dd ? L - 1 : 0; g.dt = dd ? -1 : 1; g.nsteps = L;
+        }
+        rc = launch_gru_bwd(dirs, 2, B, H, 0.f, d->rng_seed, d->rng_offset, d->rng_offset_dev, st);
+        if (rc) return rc;
+        if (tc_bwd && tc_gemm_supported(w.D[l], 8 * H, w.wT[l], 8 * H, M, I_l, 8 * H)) {
+            rc = launch_tc_gemm_nt(w.D[l], 8 * H, w.wT[l], 8 * H, nullptr, dxnext, I_l, M, I_l, 8 * H, 0, st);
+            if (rc) return rc;
+        } else {
+            for (int dd = 0; dd < 2; ++dd) {
+                rc = launch_gemm_nn(w.D[l] + dd * 4 * H, 8 * H, P + po.w_ih[l] + (int64_t)dd * 3 * H * I_l, I_l, dxnext, I_l, M, I_l,
+                                    3 * H, dd, st);
+                if (rc) return rc;
+            }
+        }
+        float* t = dxcur; dxcur = dxnext; dxnext = t;
+    }
+    // dxcur = d(seq) [B, L, O] time-major -> dy1 [B, 16, L1c]
+    rc = launch_encoder_eval_bwd(dxcur, w.y2, w.y1, P + po.conv2_w, P + po.bn1_g, P + po.bn1_b, P + po.bn2_g, P + po.bn2_b, bn, B,
+                                 m.O, m.L1c, w.dy1, st);
+    if (rc) return rc;
+    // conv1's input gradient; with the attention gate it is the gradient of x * gate, reduced against x for dgate
+    const bool gate_mlp = m.attention && m.A > 0;
+    if (gate_mlp) MMS_CUDA(cudaMemsetAsync(w.dgate, 0, (size_t)B * m.C * sizeof(float), st));
+    rc = launch_conv_dgrad(1, w.dy1, P + po.conv1_w, B, m.C, CONV1_CO, m.T, dx, gate_mlp ? x : nullptr, gate_mlp ? w.dgate : nullptr,
+                           st);
+    if (rc) return rc;
+    if (m.attention) return launch_attn_input_grad(w.dgate, w.mean, w.gate, P + po.ca_w1, P + po.ca_w2, B, m.C, m.T, dx, st);
+    return MMS_OK;
+}
+
 }  // namespace mms
 
 using namespace mms;
@@ -985,6 +1094,11 @@ extern "C" int mms_cnngru_forward(const mms_cnngru_desc* d, const float* x, cons
 extern "C" int mms_cnngru_backward(const mms_cnngru_desc* d, const float* x, const float* params, const float* bn_buffers,
                                    void* workspace, const float* dlogits, float* grads, float* dx, mms_stream_t stream) {
     return model_backward(d, x, params, bn_buffers, workspace, dlogits, grads, dx, (cudaStream_t)stream);
+}
+
+extern "C" int mms_cnngru_input_gradient(const mms_cnngru_desc* d, const float* x, const float* params, const float* bn_buffers,
+                                         void* workspace, const float* dlogits, float* dx, mms_stream_t stream) {
+    return model_input_gradient(d, x, params, bn_buffers, workspace, dlogits, dx, (cudaStream_t)stream);
 }
 
 extern "C" int mms_cnngru_forward_phase(const mms_cnngru_desc* d, int32_t phases, const float* x, const float* params,

@@ -45,6 +45,7 @@ LEARNING_RATE = 0.001
 PATIENCE = 20
 WEIGHTS_DECAY = 1e-4
 USE_CLASS_WEIGHTS = False                     # class-weighted CrossEntropyLoss, 'balanced' weights (never enabled upstream, SURVEY D9)
+ATTRIBUTION_STEPS = 0                         # > 0: integrated-gradients channel attribution of each fold's test set, this many steps
 ALL_SUBJECTS = [f"S{i}" for i in range(2, 18) if i != 12]
 CONCURRENT_FOLDS = int(os.environ.get("MMS_CONCURRENT_FOLDS", "1"))     # folds interleaved per GPU (new; 1 = the reference's loop)
 
@@ -112,8 +113,12 @@ def run_fold_async(fold_index, subject_to_test, run_output_dir, all_channel_name
     yield from trainer.train_async(train_loader, val_loader)
     out = yield from trainer.evaluate_async(test_loader, want_lists=True)
     _, test_acc, test_f1 = trainer.finish_test(*out)
-    return {'subject': subject_to_test, 'accuracy': float(test_acc), 'f1_score': float(test_f1),
-            'windows_trained': int(trainer.windows_trained), 'timing': dict(trainer.timing)}
+    result = {'subject': subject_to_test, 'accuracy': float(test_acc), 'f1_score': float(test_f1),
+              'windows_trained': int(trainer.windows_trained), 'timing': dict(trainer.timing)}
+    if ATTRIBUTION_STEPS > 0:
+        att = trainer.channel_attribution(test_loader, steps=ATTRIBUTION_STEPS, channel_names=CHANNELS_TO_USE)
+        result['channel_attribution'] = att.tolist()
+    return result
 
 
 def run_fold(fold_index, subject_to_test, run_output_dir, all_channel_names, subject_streams=None):
@@ -184,6 +189,21 @@ def write_summary(run_output_dir, results):
     return summary_file
 
 
+def write_attribution_summary(run_output_dir, results):
+    """Mean +- std over the folds of each fold's ``Trainer.channel_attribution`` (channels x classes)."""
+    att = np.array([r['channel_attribution'] for r in results], dtype=np.float64)       # [folds, nc, C]
+    mean, std = att.mean(axis=0), att.std(axis=0)
+    path = Path(run_output_dir) / 'attribution_summary.txt'
+    with open(path, 'w', encoding='utf-8') as f:
+        f.write(f"# integrated gradients, {ATTRIBUTION_STEPS} steps, zero baseline, target = predicted class; "
+                f"{len(results)} folds\n")
+        f.write("# per fold: mean over the test windows of each true class of |S_c| / sum_c' |S_c'|; here mean +- std over folds\n")
+        f.write("channel" + "".join(f"\tclass_{k}" for k in range(att.shape[1])) + "\n")
+        for c, name in enumerate(CHANNELS_TO_USE[:att.shape[2]]):
+            f.write(name + "".join(f"\t{mean[k, c]:.4f} ± {std[k, c]:.4f}" for k in range(att.shape[1])) + "\n")
+    return path
+
+
 def gather_results(local_results, world):
     """Collect the per-fold results of every rank on all ranks, ordered by subject (ALL_SUBJECTS)."""
     if world > 1:
@@ -226,6 +246,8 @@ def run_simple_experiment(run_output_dir, device, all_channel_names, subject_str
     if rank == 0:
         print("\n\n====== 留一法交叉验证全部完成 ======")
         write_summary(run_output_dir, results)
+        if ATTRIBUTION_STEPS > 0:
+            write_attribution_summary(run_output_dir, results)
     return results
 
 

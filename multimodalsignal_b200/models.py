@@ -123,6 +123,15 @@ class _Engine:
                                            ptr(dlogits), ptr(grads), ptr(dx), stream()))
         return grads, dx
 
+    def input_gradient(self, x, dlogits, dx=None):
+        """dx only (mms_cnngru_input_gradient) after an eval-mode forward with need_grad on this engine."""
+        m = self.model
+        if dx is None:
+            dx = torch.empty_like(x)
+        check(self.lib.mms_cnngru_input_gradient(C.byref(self.desc), ptr(x), ptr(m._flat), ptr(m._bn_flat),
+                                                 ptr(self.workspace), ptr(dlogits), ptr(dx), stream()))
+        return dx
+
 
 class _CnnGruFn(torch.autograd.Function):
     @staticmethod
@@ -139,8 +148,13 @@ class _CnnGruFn(torch.autograd.Function):
             raise _ext.MmsError("backward() after a newer forward() of the same shape: the activation workspace "
                                 "holds one step (the reference trainer does forward->backward per batch, trainer.py:146-148)")
         (x,) = ctx.saved_tensors
-        grads, dx = eng.backward(x, dlogits.contiguous().float(), ctx.needs_input_grad[0])
         model = ctx.model
+        if not eng.desc.training and ctx.needs_input_grad[0] and not any(ctx.needs_input_grad[4:]):
+            # eval mode with frozen parameters (model.eval().requires_grad_(False)): the input gradient alone, no
+            # parameter-gradient work at all
+            dx = eng.input_gradient(x, dlogits.contiguous().float())
+            return (dx, None, None, None, *([None] * len(model._param_views)))
+        grads, dx = eng.backward(x, dlogits.contiguous().float(), ctx.needs_input_grad[0])
         out = [grads[o:o + n].view(shape) if n else torch.zeros(shape, device=grads.device)
                for (o, n, shape) in model._param_views]
         return (dx, None, None, None, *out)

@@ -848,6 +848,42 @@ class Trainer:
             return loss, acc, f1, list(all_preds), list(all_labels)
         return out
 
+    def channel_attribution(self, data_loader, steps=32, channel_names=None, max_rows=2048):
+        """Which input channels the model's predictions rest on: integrated gradients (``attribution.py``, eval mode,
+        zero baseline, target = the predicted class) over every window of ``data_loader``.  Returns float64
+        ``[num_classes, C]``: row k is the mean, over the windows whose TRUE class is k, of |S_b,c| / sum_c' |S_b,c'|
+        (zeros for a class without windows).  Also writes ``channel_attribution.txt`` (channels x classes) in the fold
+        directory."""
+        from .attribution import channel_shares, integrated_gradients
+        m = self.model
+        nc, Cc = m.num_classes, m.in_channels
+        names = list(channel_names) if channel_names is not None else [f"channel_{c}" for c in range(Cc)]
+        if len(names) != Cc:
+            raise ValueError(f"channel_attribution: {len(names)} channel names for {Cc} channels")
+        was_training = m.training
+        m.eval()
+        sums = torch.zeros(nc, Cc, dtype=torch.float64, device=self.device)
+        counts = torch.zeros(nc, dtype=torch.float64, device=self.device)
+        try:
+            with self._on_stream():
+                for batch in data_loader:
+                    x, y = batch[0], batch[1]
+                    x = x.to(self.device, non_blocking=True).float()
+                    y = y.to(self.device, non_blocking=True).long()
+                    _, S, _ = integrated_gradients(m, x, steps=steps, max_rows=max_rows)
+                    sums.index_add_(0, y, channel_shares(S))
+                    counts.index_add_(0, y, torch.ones_like(y, dtype=torch.float64))
+                out = (sums / counts.clamp_min(1.0)[:, None]).cpu()
+        finally:
+            m.train(was_training)
+        with open(self.fold_dir / 'channel_attribution.txt', 'w', encoding='utf-8') as f:
+            f.write(f"# integrated gradients, {steps} steps, zero baseline, target = predicted class\n")
+            f.write("# mean over the windows of each true class of |S_c| / sum_c' |S_c'|\n")
+            f.write("channel" + "".join(f"\tclass_{k}" for k in range(nc)) + "\n")
+            for c, name in enumerate(names):
+                f.write(name + "".join(f"\t{out[k, c].item():.6f}" for k in range(nc)) + "\n")
+        return out
+
     def finish_test(self, loss, acc, f1, all_preds, all_labels):
         """The is_test tail of reference trainer.py:231-240: confusion-matrix plot + the two log lines."""
         self.plot_confusion_matrix(all_labels, all_preds, filename="test_confusion_matrix.png")
