@@ -155,8 +155,10 @@ __device__ __forceinline__ double warp_sum(double v) {
 }
 
 // Counter-based dropout stream: murmur3 finaliser over (seed, offset, element index).
-// Not bit-compatible with torch's Philox stream (nothing outside torch can be); parity
-// tests run with p = 0 or in eval mode, exactly as SURVEY.md §7 hard part 4 prescribes.
+// Not bit-compatible with torch's Philox stream (nothing outside torch can be).  oracle/dropout_stream.py
+// ports it to the host and states the element ids of every dropout site; tests/test_gpu_dropout.py pins
+// the port to these kernels bit for bit and checks training steps with dropout against the float64
+// oracle, with the masks the kernels drew rebuilt from (seed, offset, id).
 __device__ __forceinline__ uint32_t fmix32(uint32_t h) {
     h ^= h >> 16; h *= 0x85ebca6bu; h ^= h >> 13; h *= 0xc2b2ae35u; h ^= h >> 16;
     return h;
