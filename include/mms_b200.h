@@ -98,6 +98,14 @@ typedef struct {
                                   loss = sum_b w[y_b] l_b / sum_b w[y_b], dlogits = w[y_b] (softmax - onehot) / sum_b w[y_b].
                                   The train step needs global_batch == batch; under data parallelism the BN2 sum
                                   vector of mms_cnngru_sync_offsets gets one more double for sum_b w[y_b] */
+    uint64_t frozen_segments; /* fine-tuning (requires_grad=False): bit s = segment s of mms_cnngru_param_layout needs
+                                 no gradient.  0 = every parameter trains.  See "Frozen segments" below.             */
+    const int64_t* adam_ranges_host; /* HOST int64 [adam_nranges][3] = (offset, count, step slot): the flat ranges
+                                        mms_cnngru_train_step's Adam updates, one per trainable tensor (see
+                                        mms_adam_ranges_step)                                                        */
+    int64_t* adam_steps;      /* device int64 step counters indexed by the ranges' step slots.  NULL (with no
+                                 table): Adam over the whole buffer with step_dev as the count of every element    */
+    int32_t adam_nranges;     /* rows of adam_ranges_host, 0..MMS_MAX_ADAM_RANGES (0: no tensor trains)          */
 } mms_cnngru_desc;
 
 /* Flat parameter buffer.  The model's parameters live in ONE float32 buffer so that Adam and
@@ -115,6 +123,23 @@ typedef struct {
 #define MMS_MAX_SEGMENTS 64
 int mms_cnngru_param_layout(const mms_cnngru_desc* d, int64_t* offsets_host, int64_t* sizes_host,
                             int32_t max_segments, int64_t* total_floats_host);
+
+/* Frozen segments (desc.frozen_segments, the torch idiom module.requires_grad_(False)).  A segment whose bit is set is
+ * never written by mms_cnngru_backward, mms_cnngru_backward_phase or mms_cnngru_train_step (its gradient slots keep
+ * whatever they held; the train step's zero_grad clears only the other segments), and the backward stops as early as
+ * the mask allows:
+ *   - head weight gradients run only if a head segment trains;
+ *   - GRU layer l's weight-gradient products run only if one of its four segments trains; its recurrence backward and
+ *     the input-gradient product that feeds it only if a segment at or below layer l trains (or dx is requested);
+ *   - the encoder's stage 2 (BN2/pool backward, conv2) runs only if one of segments 0-7 trains, stage 1 only if one of
+ *     segments 0-4 does, the ChannelAttention gradients only if segment 0 or 1 does.
+ * Empty segments (the attention weights at C < 4) and the attention segments of an attention = 0 model never keep the
+ * chain alive.  Under data parallelism a phase with nothing left to do launches nothing; the SyncBN backward vectors of
+ * mms_cnngru_sync_offsets are then meaningless: [3] (BN2 reductions) when segments 0-7 are all frozen, [2] (BN1
+ * reductions) when segments 0-4 are.  With every bit clear nothing changes, launch for launch.
+ * mms_cnngru_train_step with frozen segments needs the Adam range table (desc.adam_steps, adam_ranges_host), and no
+ * range may touch a frozen segment. */
+#define MMS_MAX_ADAM_RANGES 96
 
 /* BatchNorm buffers: bn_buffers = [running_mean1[16] | running_var1[16] | running_mean2[O] |
  * running_var2[O]] float32, num_batches_tracked = int64[2] (state_dict entries
@@ -205,6 +230,13 @@ int mms_peer_allreduce_adam(float* params, const void* const* grads_host, void* 
                             int32_t rank, int32_t signal_base, float* exp_avg, float* exp_avg_sq, int64_t n,
                             const float* lr_dev, float beta1, float beta2, float eps, float weight_decay,
                             int64_t* step_dev, uint32_t* epoch_dev, uint32_t* scratch2_dev, mms_stream_t stream);
+/* The same with the update of mms_adam_ranges_step: only the elements inside the ranges are summed over the ranks and
+ * updated; the others are neither read nor written. */
+int mms_peer_allreduce_adam_ranges(float* params, const void* const* grads_host, void* const* signals_host, int32_t world,
+                                   int32_t rank, int32_t signal_base, float* exp_avg, float* exp_avg_sq,
+                                   const int64_t* ranges_host, int32_t nranges, int64_t* steps_dev, const float* lr_dev,
+                                   float beta1, float beta2, float eps, float weight_decay, int64_t* step_dev,
+                                   uint32_t* epoch_dev, uint32_t* scratch2_dev, mms_stream_t stream);
 
 /* trainer.py:69,147 CrossEntropyLoss() (mean): loss_out[0] = mean_b(lse - logit[y]),
  * dlogits = (softmax - onehot)/B (NULL to skip).  If loss_sum_accum != NULL it receives
@@ -233,6 +265,15 @@ int mms_class_weight_sum(const int64_t* labels, int32_t batch, int32_t num_class
 int mms_adam_flat_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq,
                        int64_t n, const float* lr_dev, float beta1, float beta2, float eps,
                        float weight_decay, int64_t* step_dev, int32_t* scratch_dev, mms_stream_t stream);
+/* torch.optim.Adam over some tensors of the flat buffer, each with its own step count (torch's state['step'] is per
+ * parameter; a tensor without a gradient is skipped and keeps its moments and count).  ranges_host: HOST int64
+ * [nranges][3] = (offset, count, slot) in floats, disjoint, nranges in [0, MMS_MAX_ADAM_RANGES]; range k uses
+ * steps_dev[slot] + 1 for its bias corrections and increments it.  Elements outside every range are neither read nor
+ * written.  step_dev still advances by one per call (the fused step's dropout stream offset reads it).  The arithmetic
+ * of every element is mms_adam_flat_step's. */
+int mms_adam_ranges_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, const int64_t* ranges_host,
+                         int32_t nranges, int64_t* steps_dev, const float* lr_dev, float beta1, float beta2, float eps,
+                         float weight_decay, int64_t* step_dev, int32_t* scratch_dev, mms_stream_t stream);
 
 /* trainer.py:130,140-142 -- one batch of DataLoader(dataset, batch_size, shuffle=True) (main.py:111) assembled on
  * the device: out_x[b, :] = data[perm[cursor + b], :], out_y[b] = labels[perm[cursor + b]] for b < batch.

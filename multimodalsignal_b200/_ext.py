@@ -21,6 +21,7 @@ c_u64 = C.c_uint64
 c_f32 = C.c_float
 
 MAX_SEGMENTS = 64
+MAX_ADAM_RANGES = 96
 
 
 class MmsError(RuntimeError):
@@ -34,6 +35,7 @@ class CnnGruDesc(C.Structure):
         ("attention", c_i32), ("need_grad", c_i32), ("dropout_p", c_f32),
         ("rng_seed", c_u64), ("rng_offset", c_u64), ("rng_offset_dev", C.c_void_p),
         ("global_batch", c_i32), ("class_weight", C.c_void_p),
+        ("frozen_segments", c_u64), ("adam_ranges_host", C.c_void_p), ("adam_steps", C.c_void_p), ("adam_nranges", c_i32),
     ]
 
 
@@ -102,7 +104,10 @@ _SIGNATURES = {
     "mms_peer_allreduce_f64": (c_i32, [P, P, c_i32, c_i32, c_i32, c_i32, P, P]),
     "mms_peer_status": (c_i32, [P]),
     "mms_peer_allreduce_adam": (c_i32, [P, P, P, c_i32, c_i32, c_i32, P, P, c_i64, P, c_f32, c_f32, c_f32, c_f32, P, P, P, P]),
+    "mms_peer_allreduce_adam_ranges": (c_i32, [P, P, P, c_i32, c_i32, c_i32, P, P, P, c_i32, P, P, c_f32, c_f32, c_f32, c_f32, P, P,
+                                               P, P]),
     "mms_adam_flat_step": (c_i32, [P, P, P, P, c_i64, P, c_f32, c_f32, c_f32, c_f32, P, P, P]),
+    "mms_adam_ranges_step": (c_i32, [P, P, P, P, P, c_i32, P, P, c_f32, c_f32, c_f32, c_f32, P, P, P]),
     "mms_cnngru_train_step": (c_i32, [C.POINTER(CnnGruDesc), P, P, P, P, P, P, P, P, P, P, P, P, P,
                                       c_f32, c_f32, c_f32, c_f32, P, P, P]),
     "mms_batch_gather": (c_i32, [P, P, P, P, c_i64, c_i64, c_i32, P, P, c_i32, P, P]),

@@ -202,9 +202,11 @@ __global__ void __launch_bounds__(256) pool_bwd_ncl_kernel(const float* __restri
 constexpr int C2B_TM = 128, C2B_RW = 136, C2B_PW = 140, C2B_DS = 132, C2B_CO = 32, C2B_TS = C2B_CO + 4, C2B_NW = C2B_CO * 80;
 constexpr int C2B_SMEM_FLOATS = 2 * C2B_CO * C2B_RW + 2 * 16 * C2B_PW + C2B_NW + C2B_CO * C2B_DS + 130 * C2B_TS;
 
-__global__ void __launch_bounds__(128) conv2_bwd_kernel(const float* __restrict__ dyn, const float* __restrict__ wdg,
-                                                        const float* __restrict__ p1, float* __restrict__ dp1,
-                                                        float* __restrict__ dw_part, int Lin, int Lout, const BnBwd bn) {
+// DGRAD = false: the weight gradient alone (stage 1 needs no gradient, frozen segments): warps 0-1 stop after the staging.
+template <bool DGRAD>
+__device__ __forceinline__ void conv2_bwd_body(const float* __restrict__ dyn, const float* __restrict__ wdg,
+                                               const float* __restrict__ p1, float* __restrict__ dp1,
+                                               float* __restrict__ dw_part, int Lin, int Lout, const BnBwd bn) {
     MMS_PDL_TRIGGER();
     constexpr int CO2 = C2B_CO;
     extern __shared__ __align__(128) float c2b_smem[];
@@ -274,6 +276,7 @@ __global__ void __launch_bounds__(128) conv2_bwd_kernel(const float* __restrict_
     __syncthreads();
 
     if (warp < 2) {
+        if (!DGRAD) return;
         // ===== input gradient: pairs u = m0 + 64 warp + 8 pg + e (positions 2u, 2u + 1), input channels 4 cg .. 4 cg + 3 =====
         //   even j = 2u   : taps k = 0, 2, 4 with m = u + 1, u, u - 1;    odd j = 2u + 1 : taps k = 1, 3 with m = u + 1, u
         const int pg = (lane & 3) | ((lane >> 2) & 4), cg = (lane >> 2) & 3;     // a quarter-warp = 4 pair groups x 2 channel groups
@@ -403,6 +406,18 @@ __global__ void __launch_bounds__(128) conv2_bwd_kernel(const float* __restrict_
         const float4* srcp = reinterpret_cast<const float4*>(ex);
         for (int i = tid - 64; i < C2B_NW / 4; i += 64) dstp[i] = srcp[i];
     }
+}
+
+__global__ void __launch_bounds__(128) conv2_bwd_kernel(const float* __restrict__ dyn, const float* __restrict__ wdg,
+                                                        const float* __restrict__ p1, float* __restrict__ dp1,
+                                                        float* __restrict__ dw_part, int Lin, int Lout, const BnBwd bn) {
+    conv2_bwd_body<true>(dyn, wdg, p1, dp1, dw_part, Lin, Lout, bn);
+}
+
+__global__ void __launch_bounds__(128) conv2_wgrad_bwd_kernel(const float* __restrict__ dyn, const float* __restrict__ wdg,
+                                                              const float* __restrict__ p1, float* __restrict__ dw_part, int Lin,
+                                                              int Lout, const BnBwd bn) {
+    conv2_bwd_body<false>(dyn, wdg, p1, nullptr, dw_part, Lin, Lout, bn);
 }
 
 // wd[(o*5 + k)*16 + ci] = w[o][ci][k]: the order conv2_bwd_kernel's input-gradient warps read (one bulk copy per CTA instead of a
@@ -675,7 +690,7 @@ int launch_pool_bwd_ncl(const float* y, const double* stats, const float* gamma,
 
 static const BnBwd kNoBn = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, 1.f};
 
-// Both gradients of conv2 (C_out = 32).  dp1 [B,16,P1] is written; dw (+=) receives the weight gradient through `scratch`
+// Both gradients of conv2 (C_out = 32).  dp1 [B,16,P1] is written (dp1 == nullptr: the weight gradient alone); dw (+=) receives the weight gradient through `scratch`
 // (conv2_bwd_scratch_floats) and launch_wgrad_reduce.  w: the weights in conv2_w_relayout_kernel's order.
 int launch_conv2_w_relayout(const float* w, float* wd, cudaStream_t st) {
     MMS_PROF_BEGIN(st);
@@ -694,11 +709,19 @@ int launch_conv2_bwd(const float* dyn, const float* w, const float* p1, int B, i
                   reinterpret_cast<uintptr_t>(scratch) | reinterpret_cast<uintptr_t>(bn.y) | reinterpret_cast<uintptr_t>(w)) & 15) == 0, "conv2_bwd: operands must be 16-byte aligned");
     const size_t smem = (size_t)C2B_SMEM_FLOATS * sizeof(float);
     static PerDeviceOnce attr_once;
-    if (attr_once.need()) MMS_CUDA(cudaFuncSetAttribute(conv2_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (attr_once.need()) {
+        MMS_CUDA(cudaFuncSetAttribute(conv2_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        MMS_CUDA(cudaFuncSetAttribute(conv2_wgrad_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    }
     dim3 grid(cdiv(Lout, C2B_TM), B);
     MMS_PROF_BEGIN(st);
-    MMS_LAUNCH(conv2_bwd_kernel, grid, dim3(128), smem, st, dyn, w, p1, dp1, scratch, P1, Lout, bn);
-    MMS_LAUNCH_CHECK("conv2_bwd_kernel");
+    if (dp1) {
+        MMS_LAUNCH(conv2_bwd_kernel, grid, dim3(128), smem, st, dyn, w, p1, dp1, scratch, P1, Lout, bn);
+        MMS_LAUNCH_CHECK("conv2_bwd_kernel");
+    } else {        // stage 1 frozen: the weight gradient alone
+        MMS_LAUNCH(conv2_wgrad_bwd_kernel, grid, dim3(128), smem, st, dyn, w, p1, scratch, P1, Lout, bn);
+        MMS_LAUNCH_CHECK("conv2_wgrad_bwd_kernel");
+    }
     return MMS_OK;
 }
 

@@ -324,39 +324,77 @@ __global__ void __launch_bounds__(256) cross_entropy_kernel(const float* __restr
     }
 }
 
-// torch.optim.Adam single-tensor rule over the flat buffer (coupled L2 weight decay):
-//   g += wd*p; m = b1*m + (1-b1)*g; v = b2*v + (1-b2)*g*g;
-//   p -= (lr / (1-b1^t)) * m / (sqrt(v)/sqrt(1-b2^t) + eps),   t = *step_dev + 1
+// torch.optim.Adam (adam_update, mms_common.cuh) over the flat buffer, t = *step_dev + 1.
 // The last CTA to finish increments *step_dev (every CTA has read it by then).
 __global__ void __launch_bounds__(256) adam_flat_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                                                         float* __restrict__ v, int64_t n, const float* __restrict__ lr_dev,
                                                         float beta1, float beta2, float eps, float wd, int64_t* step_dev,
                                                         int32_t* scratch) {
     MMS_PDL_PROLOGUE();
-    const double t = (double)(*step_dev + 1);
+    const int64_t done = *step_dev;
     const float lr = *lr_dev;
-    const float bc1 = (float)(1.0 - pow((double)beta1, t));
-    const float bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, t));
-    const float step_size = lr / bc1;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        const float pi = p[i];
-        const float gi = g[i] + wd * pi;
-        const float mi = beta1 * m[i] + (1.f - beta1) * gi;
-        const float vi = beta2 * v[i] + (1.f - beta2) * gi * gi;
-        m[i] = mi;
-        v[i] = vi;
-        const float denom = sqrtf(vi) / bc2_sqrt + eps;
-        p[i] = pi - step_size * (mi / denom);
+    const AdamCoef c = adam_coef(done, lr, beta1, beta2);
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+        adam_update(p, g, m, v, i, c, beta1, beta2, eps, wd);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        const int last = atomicAdd(scratch, 1);
+        if (last == (int)gridDim.x - 1) {
+            *step_dev += 1;
+            *scratch = 0;
+        }
+    }
+}
+
+// The same update over the ranges of `r` only, range k with its own count steps[r.slot[k]].  The ranges are laid end to end
+// into one virtual index space that the grid strides over, so small tensors do not all land on the first threads.  The last
+// CTA to finish advances every range's count and *step_dev.
+__global__ void __launch_bounds__(256) adam_ranges_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
+                                                          float* __restrict__ v, const __grid_constant__ AdamRanges r,
+                                                          int64_t* steps, const float* __restrict__ lr_dev, float beta1, float beta2,
+                                                          float eps, float wd, int64_t* step_dev, int32_t* scratch) {
+    MMS_PDL_PROLOGUE();
+    __shared__ AdamCoef s_c[MMS_MAX_ADAM_RANGES];
+    const float lr = *lr_dev;
+    for (int k = threadIdx.x; k < r.n; k += blockDim.x) s_c[k] = adam_coef(steps[r.slot[k]], lr, beta1, beta2);
+    __syncthreads();
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x, gt = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    int64_t base = 0;                       // virtual index of the range's first element
+    for (int k = 0; k < r.n; ++k) {
+        const AdamCoef c = s_c[k];
+        int64_t j = (gt - base) % stride;
+        if (j < 0) j += stride;
+        for (; j < r.cnt[k]; j += stride) {
+            adam_update(p, g, m, v, r.off[k] + j, c, beta1, beta2, eps, wd);
+        }
+        base += r.cnt[k];
     }
     __syncthreads();
     if (threadIdx.x == 0) {
         __threadfence();
         const int done = atomicAdd(scratch, 1);
         if (done == (int)gridDim.x - 1) {
+            for (int k = 0; k < r.n; ++k) steps[r.slot[k]] += 1;
             *step_dev += 1;
             *scratch = 0;
         }
     }
+}
+
+int adam_ranges_from_host(const int64_t* table, int n, int64_t total, AdamRanges* r) {
+    MMS_REQUIRE((table || n == 0) && n >= 0 && n <= MMS_MAX_ADAM_RANGES, "adam ranges: %d ranges, need 0..%d", n, MMS_MAX_ADAM_RANGES);
+    r->n = n;
+    for (int k = 0; k < n; ++k) {
+        const int64_t off = table[3 * k], cnt = table[3 * k + 1], slot = table[3 * k + 2];
+        MMS_REQUIRE(off >= 0 && cnt >= 1 && off + cnt <= total && slot >= 0 && slot <= INT32_MAX,
+                    "adam ranges: range %d = (%lld, %lld, %lld) outside a buffer of %lld floats", k, (long long)off, (long long)cnt,
+                    (long long)slot, (long long)total);
+        for (int q = 0; q < k; ++q)
+            MMS_REQUIRE(off + cnt <= r->off[q] || r->off[q] + r->cnt[q] <= off, "adam ranges: ranges %d and %d overlap", q, k);
+        r->off[k] = off; r->cnt[k] = cnt; r->slot[k] = (int32_t)slot;
+    }
+    return MMS_OK;
 }
 
 int launch_head_fwd2(const float* src_a, int64_t lda, const float* src_b, int64_t ldb, int Hh, const float* w0, const float* b0,
@@ -452,6 +490,18 @@ int launch_adam(float* p, const float* g, float* m, float* v, int64_t n, const f
     return MMS_OK;
 }
 
+int launch_adam_ranges(float* p, const float* g, float* m, float* v, const AdamRanges& r, int64_t* steps, const float* lr_dev,
+                       float beta1, float beta2, float eps, float wd, int64_t* step_dev, int32_t* scratch, cudaStream_t st) {
+    int64_t n = 0;
+    for (int k = 0; k < r.n; ++k) n += r.cnt[k];
+    const int blocks = (int)((n + 255) / 256 < 592 ? (n + 255) / 256 : 592);
+    MMS_PROF_BEGIN(st);
+    MMS_LAUNCH(adam_ranges_kernel, dim3(blocks > 0 ? blocks : 1), dim3(256), 0, st, p, g, m, v, r, steps, lr_dev, beta1, beta2, eps, wd,
+               step_dev, scratch);
+    MMS_LAUNCH_CHECK("adam_ranges_kernel");
+    return MMS_OK;
+}
+
 }  // namespace mms
 
 using namespace mms;
@@ -499,4 +549,14 @@ extern "C" int mms_adam_flat_step(float* params, const float* grads, float* exp_
     MMS_REQUIRE(params && grads && exp_avg && exp_avg_sq && lr_dev && step_dev && scratch_dev && n > 0, "adam_flat_step: bad arguments");
     return launch_adam(params, grads, exp_avg, exp_avg_sq, n, lr_dev, beta1, beta2, eps, weight_decay, step_dev, scratch_dev,
                        (cudaStream_t)stream);
+}
+extern "C" int mms_adam_ranges_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, const int64_t* ranges_host,
+                                    int32_t nranges, int64_t* steps_dev, const float* lr_dev, float beta1, float beta2, float eps,
+                                    float weight_decay, int64_t* step_dev, int32_t* scratch_dev, mms_stream_t stream) {
+    MMS_REQUIRE(params && grads && exp_avg && exp_avg_sq && steps_dev && lr_dev && step_dev && scratch_dev, "adam_ranges_step: bad arguments");
+    AdamRanges r;
+    const int rc = adam_ranges_from_host(ranges_host, nranges, INT64_MAX / 2, &r);
+    if (rc) return rc;
+    return launch_adam_ranges(params, grads, exp_avg, exp_avg_sq, r, steps_dev, lr_dev, beta1, beta2, eps, weight_decay, step_dev,
+                              scratch_dev, (cudaStream_t)stream);
 }

@@ -99,6 +99,16 @@ struct BnBwd {
     float grad_scale;
 };
 
+// Flat ranges of the Adam update (mms_adam_ranges_step), passed by value: range k is [off[k], off[k] + cnt[k]) with step
+// counter steps[slot[k]].
+struct AdamRanges {
+    int n;
+    int64_t off[MMS_MAX_ADAM_RANGES], cnt[MMS_MAX_ADAM_RANGES];
+    int32_t slot[MMS_MAX_ADAM_RANGES];
+};
+// Reads a HOST (offset, count, slot) table; every range must lie inside [0, total) and be disjoint from the others.
+int adam_ranges_from_host(const int64_t* table, int n, int64_t total, AdamRanges* r);
+
 // ---- programmatic dependent launch (build variant, -DMMS_PDL; default build: every macro below is a no-op) ---------
 // 25 dependent launches make up the critical path of a step, and each edge costs the drain of the producer plus the launch,
 // CTA scheduling and prologue of the consumer.  With MMS_PDL the kernels of the main chain are launched with
@@ -186,6 +196,40 @@ __device__ __forceinline__ uint64_t resolve_offset(uint64_t host_off, const int6
 }
 
 __device__ __forceinline__ float sigmoid_f(float x) { return 1.f / (1.f + expf(-x)); }
+
+// torch.optim.Adam single-tensor rule (coupled L2 weight decay), shared by every Adam kernel of the library:
+//   g += wd*p; m = b1*m + (1-b1)*g; v = b2*v + (1-b2)*g*g;
+//   p -= (lr / (1-b1^t)) * m / (sqrt(v)/sqrt(1-b2^t) + eps),   t = steps_done + 1
+struct AdamCoef {
+    float step_size, bc2_sqrt;
+};
+__device__ __forceinline__ AdamCoef adam_coef(int64_t steps_done, float lr, float beta1, float beta2) {
+    const double t = (double)(steps_done + 1);
+    const float bc1 = (float)(1.0 - pow((double)beta1, t));
+    const float bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, t));
+    return {lr / bc1, bc2_sqrt};
+}
+// element i, the gradient read from g[i]
+__device__ __forceinline__ void adam_update(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
+                                            float* __restrict__ v, int64_t i, const AdamCoef c, float beta1, float beta2, float eps,
+                                            float wd) {
+    const float pi = p[i];
+    const float gi = g[i] + wd * pi;
+    const float mi = beta1 * m[i] + (1.f - beta1) * gi;
+    const float vi = beta2 * v[i] + (1.f - beta2) * gi * gi;
+    m[i] = mi;
+    v[i] = vi;
+    const float denom = sqrtf(vi) / c.bc2_sqrt + eps;
+    p[i] = pi - c.step_size * (mi / denom);
+}
+// the same for one element of registers whose gradient has already been summed (the peer kernels)
+__device__ __forceinline__ float adam_update(float pi, float gsum, float& mi, float& vi, const AdamCoef c, float beta1, float beta2,
+                                             float eps, float wd) {
+    const float gi = gsum + wd * pi;
+    mi = beta1 * mi + (1.f - beta1) * gi;
+    vi = beta2 * vi + (1.f - beta2) * gi * gi;
+    return pi - c.step_size * (mi / (sqrtf(vi) / c.bc2_sqrt + eps));
+}
 
 #endif  // __CUDACC__
 

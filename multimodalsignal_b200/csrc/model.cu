@@ -42,6 +42,8 @@ int launch_head_ce_fused(const float*, int64_t, const float*, int64_t, int, cons
                          float*, float*, int32_t*, float*, double*, cudaStream_t, const float* class_weight);
 int launch_adam(float*, const float*, float*, float*, int64_t, const float*, float, float, float, float, int64_t*, int32_t*,
                 cudaStream_t);
+int launch_adam_ranges(float*, const float*, float*, float*, const AdamRanges&, int64_t*, const float*, float, float, float, float,
+                       int64_t*, int32_t*, cudaStream_t);
 int launch_chan_dx(const float*, const float*, const float*, int, int, int, float*, cudaStream_t);
 bool conv_fused_supported(const float*, int, int, int);
 bool conv_bwd_supported(const float*, int, int, int);
@@ -348,6 +350,49 @@ static void make_params(const Dims& m, ParamOff* p) {
     p->nseg = n;
 }
 
+// Which parts of the backward pass run, from desc.frozen_segments (include/mms_b200.h, "Frozen segments").  A segment
+// trains when its bit is clear and it has elements; the attention segments of an attention = 0 model never train.
+struct Live {
+    bool seg[MMS_MAX_SEGMENTS];      // the segment's gradient is written
+    bool head_w;                     // a head segment trains
+    bool layer_w[MAX_LAYERS];        // one of GRU layer l's four segments trains
+    bool recur[MAX_LAYERS];          // layer l's recurrence backward runs: a segment at or below it trains, or dx is wanted
+    bool enc2, enc1, attn;           // encoder stage 2 (segments 0-7), stage 1 (0-4), ChannelAttention (0-1)
+};
+
+static Live liveness(const Dims& m, const ParamOff& po, uint64_t frozen, bool want_dx) {
+    Live v;
+    for (int s = 0; s < MMS_MAX_SEGMENTS; ++s)
+        v.seg[s] = s < po.nseg && po.size[s] > 0 && !((frozen >> s) & 1ull) && (s >= 2 || m.attention);
+    auto any = [&](int lo, int hi) { bool a = false; for (int s = lo; s <= hi; ++s) a = a || v.seg[s]; return a; };
+    v.attn = any(0, 1);
+    v.enc1 = any(0, 4) || want_dx;
+    v.enc2 = v.enc1 || any(5, 7);
+    v.head_w = any(8 + 4 * m.layers, 11 + 4 * m.layers);
+    bool below = v.enc2;
+    for (int l = 0; l < m.layers; ++l) {
+        v.layer_w[l] = any(8 + 4 * l, 11 + 4 * l);
+        below = below || v.layer_w[l];
+        v.recur[l] = below;
+    }
+    return v;
+}
+
+// zero_grad of the trainable segments: one memset per run of segments without a frozen bit (the whole buffer when nothing is
+// frozen), so that frozen gradient slots keep their contents
+static int zero_trainable(float* G, const ParamOff& po, uint64_t frozen, cudaStream_t st) {
+    int s = 0;
+    while (s < po.nseg) {
+        if ((frozen >> s) & 1ull) { ++s; continue; }
+        int e = s;
+        while (e + 1 < po.nseg && !((frozen >> (e + 1)) & 1ull)) ++e;
+        const int64_t lo = po.off[s], hi = e + 1 < po.nseg ? po.off[e + 1] : po.total;
+        MMS_CUDA(cudaMemsetAsync(G + lo, 0, (size_t)(hi - lo) * sizeof(float), st));
+        s = e + 1;
+    }
+    return MMS_OK;
+}
+
 struct Workspace {
     // zeroed at the start of every forward
     double* stats1; double* stats2;
@@ -361,6 +406,7 @@ struct Workspace {
     float *wT_top, *wT[MAX_LAYERS], *dx_extra;
     int32_t* head_counter; float* rowloss;
     float *dhid, *dlogits, *D_tf, *D_tr, *D[MAX_LAYERS], *dxa, *dxb, *dy2, *dp1, *dy1, *ca_scratch, *c2_part, *c1_part, *c2_wd;
+    float* gsink;          // where kernels that write several segments put the gradients of frozen ones
     int64_t total;
 };
 
@@ -429,6 +475,10 @@ static void carve(const Dims& m, char* base, Workspace* w) {
         w->c2_part = (float*)take(conv2_bwd_scratch_floats(m.B, m.P1) * f);      // partial conv2 weight gradients, one per CTA
         w->c1_part = (float*)take(conv1_bwd_scratch_floats(m.B, m.C) * f);       // partial conv1 G per (row, chunk)
         w->c2_wd = (float*)take(conv2_w_relayout_floats() * f);                  // conv2 weights as [o][k][ci]
+        int64_t sink = (int64_t)HEAD_HID * 2 * H;                                  // the largest segment such a kernel writes
+        if ((int64_t)m.O * CONV2_CI * CONV2_K > sink) sink = (int64_t)m.O * CONV2_CI * CONV2_K;
+        if ((int64_t)CONV1_CO * 16 * CONV1_K > sink) sink = (int64_t)CONV1_CO * 16 * CONV1_K;
+        w->gsink = (float*)take(sink * f);
     }
     w->total = cur;
 }
@@ -443,7 +493,8 @@ struct FusedLoss {
     float* loss_out;
     double* loss_sum_accum;
     float* grads;            // zero_grad of the fused step: cleared on a side stream of the forward (nullptr: the caller did it)
-    size_t grads_bytes;
+    const ParamOff* po;      // ... segment by segment: frozen segments (desc.frozen_segments) keep their slots
+    uint64_t frozen;
     bool zero_bwd;           // the backward follows in the same call chain: clear its reductions with the forward's
 };
 
@@ -515,7 +566,10 @@ static int model_forward(const mms_cnngru_desc* d, const float* x, const float* 
         const bool tc_bwd = m.need_grad && use_tc() && M >= TC_MIN_ROWS;
         if ((fl && fl->grads) || tc_bwd) {
             cudaStream_t s1 = fka.fork(1);
-            if (fl && fl->grads) MMS_CUDA(cudaMemsetAsync(fl->grads, 0, fl->grads_bytes, s1));
+            if (fl && fl->grads) {
+                rc = zero_trainable(fl->grads, *fl->po, fl->frozen, s1);
+                if (rc) return rc;
+            }
             if (tc_bwd) {
                 // W_ih^T of every layer, up to four matrices per launch; the bottom layers' copies carry zero columns where the
                 // D rows hold dq
@@ -641,6 +695,15 @@ static int model_forward(const mms_cnngru_desc* d, const float* x, const float* 
                             w.last, w.hid, logits, st);
 }
 
+// Appends TN product `c` to list[n] with the frozen outputs removed: no weight gradient (C == nullptr) leaves the bias gradient
+// alone (N2 = 0), neither leaves nothing.  Returns the new count.
+static int tn_keep(TnCall* list, int n, TnCall c) {
+    if (!c.C) { c.N2 = 0; c.Bm = nullptr; c.ldb = 0; c.ldc = 0; }
+    if (!c.C && !c.bias_grad) return n;
+    list[n] = c;
+    return n + 1;
+}
+
 // phases: bit 0 = head ... GRU ... pool/ReLU backward of stage 2 (+ its BN reductions), bit 1 = BN apply of stage 2,
 // conv2 gradients, pool/ReLU backward of stage 1 (+ reductions), bit 2 = the rest.  A data-parallel caller
 // all-reduces the float64 reductions between the phases; 7 = everything.
@@ -664,13 +727,20 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
     const float gscale = (float)m.B / (float)m.Bg;       // share of the global BN affine gradient this rank adds
     // conv_bwd.cu (the default when the shapes allow it): T % 32 == 0, C_out == 32, BatchNorm backward folded, no input gradient
     const bool bwd2 = bn_fold() && !dx && option_get("CONV_BWD", 1) == 1 && conv_bwd_supported(x, m.C, m.T, m.O);
+    // frozen segments: what runs (Live), and the gradient slot of segment s -- nullptr where it must stay untouched (the TN
+    // products and BnBwd skip null outputs), or a scratch sink for kernels that write several segments in one launch
+    const Live lv = liveness(m, po, d->frozen_segments, dx != nullptr);
+    auto gs = [&](int s) -> float* { return lv.seg[s] ? G + po.off[s] : nullptr; };
+    auto gk = [&](int s) -> float* { return lv.seg[s] ? G + po.off[s] : w.gsink; };
+    const int top = m.layers - 1;
+    const int hs0 = 8 + 4 * m.layers;                    // first head segment
     Forker fk(st);
-    if (phases & 1) {
-    if (!bwd_zeroed) MMS_CUDA(cudaMemsetAsync(w.bwd_zero, 0, w.bwd_zero_bytes, st));
+    if ((phases & 1) && (lv.head_w || lv.recur[top])) {
+    if (!bwd_zeroed && lv.enc2) MMS_CUDA(cudaMemsetAsync(w.bwd_zero, 0, w.bwd_zero_bytes, st));
     const bool tc_bwd = use_tc() && M >= TC_MIN_ROWS;      // W_ih^T for the tensor-core dx products: made by the forward pass
     // conv2's weights in conv2_bwd_kernel's order: left in the workspace by the fused forward (attn_conv1_fwd_kernel); after a
     // per-layer forward they are made here, on a side stream, long before they are needed
-    if (bwd2 && phases == 7 && !fwd_is_fused(m, x)) {
+    if (bwd2 && phases == 7 && lv.enc2 && !fwd_is_fused(m, x)) {
         rc = launch_conv2_w_relayout(P + po.conv2_w, w.c2_wd, fk.fork(1));
         if (rc) return rc;
         rc = fk.mark(1);
@@ -678,12 +748,15 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
     }
     // head: dhid feeds the top recurrence; with the fused forward it already exists and only the weight gradients remain,
     // which nothing on the chain needs -> side stream
-    rc = launch_head_bwd(w.last, w.hid, dlogits, P + po.fc3_w, B, 2 * H, m.nc, m.drop_head ? p : 0.f, d->rng_seed, d->rng_offset,
-                         d->rng_offset_dev, head_done ? nullptr : w.dhid, G + po.fc0_w, G + po.fc0_b, G + po.fc3_w, G + po.fc3_b,
-                         head_done ? fk.fork(2) : st);
-    if (rc) return rc;
+    const bool need_dhid = !head_done && lv.recur[top];
+    if (lv.head_w || need_dhid) {
+        rc = launch_head_bwd(w.last, w.hid, dlogits, P + po.fc3_w, B, 2 * H, m.nc, m.drop_head ? p : 0.f, d->rng_seed, d->rng_offset,
+                             d->rng_offset_dev, need_dhid ? w.dhid : nullptr, gk(hs0), gk(hs0 + 1), gk(hs0 + 2), gk(hs0 + 3),
+                             head_done ? fk.fork(2) : st);
+        if (rc) return rc;
+    }
+    if (!lv.recur[top]) return fk.join();      // head only: nothing below it trains
 
-    const int top = m.layers - 1;
     const float* in_top = top == 0 ? w.seq : w.outd[top - 1];
     const int I_top = top == 0 ? m.O : 2 * H;
     float* dxcur = w.dxa;
@@ -693,23 +766,34 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
     // forks them after the NEXT layer's recurrence has been enqueued instead of right after the top one, so that they overlap
     // the conv backward chain rather than the layer-0 recurrence (whose CTAs lose issue slots to co-resident GEMM CTAs).
     auto top_wgrad = [&]() -> int {
-        cudaStream_t sw = fk.fork(0);
-        const TnCall big[2] = {
-            {w.D_tf, 4 * H, 3 * H, 0, in_top, I_top, 0, L, G + po.w_ih[top], I_top, G + po.b_ih[top], M, 3 * H, I_top},
-            {w.D_tf, 4 * H, 2 * H, H, w.hs_tf, H, -1, L, G + po.w_hh[top], H, G + po.b_hh[top], M, 3 * H, H}};
-        int r = gemm_tn_many(big, 2, sw);
-        if (r) return r;
+        if (!lv.layer_w[top]) return MMS_OK;
+        const int sg = 8 + 4 * top;
+        float *g_wih = gs(sg), *g_whh = gs(sg + 1), *g_bih = gs(sg + 2), *g_bhh = gs(sg + 3);
+        TnCall big[2];
+        const int nb = tn_keep(big, 0, {w.D_tf, 4 * H, 3 * H, 0, in_top, I_top, 0, L, g_wih, I_top, g_bih, M, 3 * H, I_top});
+        const int nbig = tn_keep(big, nb, {w.D_tf, 4 * H, 2 * H, H, w.hs_tf, H, -1, L, g_whh, H, g_bhh, M, 3 * H, H});
+        if (nbig) {
+            const int r = gemm_tn_many(big, nbig, fk.fork(0));
+            if (r) return r;
+        }
         // the B-row products of the single reverse step: their own side stream, beside the big products instead of behind them
-        cudaStream_t ss = fk.fork(2);
-        r = gemm_tn(w.D_tr, 4 * H, 3 * H, 0, in_top + (int64_t)(L - 1) * I_top, (int64_t)L * I_top, 0, 1,
-                    G + po.w_ih[top] + (int64_t)3 * H * I_top, I_top, G + po.b_ih[top] + 3 * H, B, 3 * H, I_top, ss);
-        if (r) return r;
+        TnCall rev[2];
+        int nrev = tn_keep(rev, 0, {w.D_tr, 4 * H, 3 * H, 0, in_top + (int64_t)(L - 1) * I_top, (int64_t)L * I_top, 0, 1,
+                                    g_wih ? g_wih + (int64_t)3 * H * I_top : nullptr, I_top, g_bih ? g_bih + 3 * H : nullptr, B, 3 * H, I_top});
         // h_prev = 0 for the single reverse step: dW_hh(reverse) = 0, only the bias gradient remains
-        return gemm_tn(w.D_tr, 4 * H, 2 * H, H, nullptr, 0, 0, 1, nullptr, 0, G + po.b_hh[top] + 3 * H, B, 3 * H, 0, ss);
+        nrev = tn_keep(rev, nrev, {w.D_tr, 4 * H, 2 * H, H, nullptr, 0, 0, 1, nullptr, 0, g_bhh ? g_bhh + 3 * H : nullptr, B, 3 * H, 0});
+        cudaStream_t ss = nrev ? fk.fork(2) : st;
+        for (int j = 0; j < nrev; ++j) {
+            const TnCall& c = rev[j];
+            const int r = gemm_tn(c.A, c.lda, c.a_split, c.a_skip, c.Bm, c.ldb, c.shift, c.seq, c.C, c.ldc, c.bias_grad, c.M, c.N1, c.N2, ss);
+            if (r) return r;
+        }
+        return MMS_OK;
     };
     // MMS_WGRAD_DEFER: 0 = right behind the top recurrence (beside the dx product), 1 (default) = behind the next recurrence,
     // 2 (experiment) = behind the dx product, i.e. beside the next recurrence only
-    const int defer_mode = top >= 1 ? option_get("WGRAD_DEFER", 1) : 0;
+    const int defer_mode = top >= 1 && lv.recur[top - 1] ? option_get("WGRAD_DEFER", 1) : 0;
+    const bool dx_top = top >= 1 ? lv.recur[top - 1] : lv.enc2;     // the top layer's input gradient is consumed
     const bool defer_top_wgrad = defer_mode >= 1;
     {
         mms_gru_dir_bwd dirs[2];
@@ -733,7 +817,7 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
             rc = top_wgrad();
             if (rc) return rc;
         }
-        if (top >= 1) {
+        if (top >= 1 && dx_top) {
             // the single reverse step only touches the rows t = L-1: its B-row product goes to dx_extra on a side
             // stream, beside the big product below; the layer underneath adds it at t = L-1
             cudaStream_t sx = fk.fork(2);
@@ -755,7 +839,8 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
             }
         }
         // gradient w.r.t. the top layer's input
-        if (tc_bwd && tc_gemm_supported(w.D_tf, 4 * H, w.wT_top, 3 * H, M, I_top, 3 * H)) {
+        if (!dx_top) {
+        } else if (tc_bwd && tc_gemm_supported(w.D_tf, 4 * H, w.wT_top, 3 * H, M, I_top, 3 * H)) {
             // tensor-core path: dx = D @ W_ih as an NT product against the transposed weights
             // the gradient through the dropout between layer top-1 and top (same multipliers as the forward) rides on this
             // product's epilogue instead of a separate pass over dxcur
@@ -772,13 +857,13 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
             if (rc) return rc;
         }
         // the single reverse step only touches the rows t = L-1 (B rows, SIMT)
-        if (top == 0) {
+        if (top == 0 && dx_top) {
             rc = launch_gemm_nn(w.D_tr, 4 * H, P + po.w_ih[top] + (int64_t)3 * H * I_top, I_top, dxcur + (int64_t)(L - 1) * I_top,
                                 (int64_t)L * I_top, B, I_top, 3 * H, 1, st);
             if (rc) return rc;
         }
     }
-    for (int l = top - 1; l >= 0; --l) {
+    for (int l = top - 1; l >= 0 && lv.recur[l]; --l) {
         const float* in_l = l == 0 ? w.seq : w.outd[l - 1];
         const int I_l = l == 0 ? m.O : 2 * H;
         if (m.drop_gru && drop_done_for != l) {      // gradient through the dropout between layer l and l + 1 (same multipliers)
@@ -821,22 +906,27 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
         // stretched the (critical-path) input-gradient product 2.4x (round-2 timeline); started behind it they overlap the
         // encoder's backward kernels instead.
         auto layer_wgrad = [&]() -> int {
-            cudaStream_t sw = fk.fork(1 - (l & 1));
+            if (!lv.layer_w[l]) return MMS_OK;
+            const int sg = 8 + 4 * l;
+            float *g_wih = gs(sg), *g_whh = gs(sg + 1), *g_bih = gs(sg + 2), *g_bhh = gs(sg + 3);
             TnCall four[4];
+            int n4 = 0;
             for (int dd = 0; dd < 2; ++dd) {
                 const float* Dd = w.D[l] + dd * 4 * H;
-                four[2 * dd] = {Dd, 8 * H, 3 * H, 0, in_l, I_l, 0, L, G + po.w_ih[l] + (int64_t)dd * 3 * H * I_l, I_l,
-                                G + po.b_ih[l] + dd * 3 * H, M, 3 * H, I_l};
-                four[2 * dd + 1] = {Dd, 8 * H, 2 * H, H, w.hs[l] + dd * H, 2 * H, dd ? 1 : -1, L,
-                                    G + po.w_hh[l] + (int64_t)dd * 3 * H * H, H, G + po.b_hh[l] + dd * 3 * H, M, 3 * H, H};
+                n4 = tn_keep(four, n4, {Dd, 8 * H, 3 * H, 0, in_l, I_l, 0, L, g_wih ? g_wih + (int64_t)dd * 3 * H * I_l : nullptr, I_l,
+                                        g_bih ? g_bih + dd * 3 * H : nullptr, M, 3 * H, I_l});
+                n4 = tn_keep(four, n4, {Dd, 8 * H, 2 * H, H, w.hs[l] + dd * H, 2 * H, dd ? 1 : -1, L,
+                                        g_whh ? g_whh + (int64_t)dd * 3 * H * H : nullptr, H, g_bhh ? g_bhh + dd * 3 * H : nullptr, M, 3 * H, H});
             }
-            return gemm_tn_many(four, 4, sw);
+            return gemm_tn_many(four, n4, fk.fork(1 - (l & 1)));
         };
         if (!tn_after) {
             rc = layer_wgrad();
             if (rc) return rc;
         }
-        if (tc_bwd && tc_gemm_supported(w.D[l], 8 * H, w.wT[l], 8 * H, M, I_l, 8 * H)) {
+        if (!(l >= 1 ? lv.recur[l - 1] : lv.enc2)) {
+            // nothing underneath needs this layer's input gradient
+        } else if (tc_bwd && tc_gemm_supported(w.D[l], 8 * H, w.wT[l], 8 * H, M, I_l, 8 * H)) {
             // both directions in one NT product: K = [fwd 3H | (dq) | rev 3H | (dq)], zero weights on the dq columns
             rc = launch_tc_gemm_nt(w.D[l], 8 * H, w.wT[l], 8 * H, nullptr, dxnext, I_l, M, I_l, 8 * H, 0, st);
             if (rc) return rc;
@@ -857,15 +947,17 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
         }
         float* t = dxcur; dxcur = dxnext; dxnext = t;
     }
+    if (!lv.enc2) return fk.join();           // the encoder is frozen: the chain ends at the bottom GRU layer
     // dxcur = d(seq) [B, L, O] time-major
     if (bwd2)
         rc = launch_pool_bwd_tm(w.y2, w.stats2, P + po.bn2_g, P + po.bn2_b, rm2, rv2, dxcur, B, m.O, m.L2c, m.training, w.dy2, w.red2, st,
                                 m.Bg);
     else
         rc = launch_bn_relu_pool_bwd(w.y2, w.stats2, P + po.bn2_g, P + po.bn2_b, rm2, rv2, dxcur, B, m.O, m.L2c, m.training, 1, w.dy2,
-                                     G + po.bn2_g, G + po.bn2_b, w.red2, st, 1, m.Bg, gscale);
+                                     gk(6), gk(7), w.red2, st, 1, m.Bg, gscale);
     if (rc) return rc;
     }   // phase bit 0
+    if (!lv.enc2) return fk.join();
     // The BatchNorm-backward apply pass is folded into the consumers of dy (BnBwd, mms_common.cuh): w.dy2 / w.dy1 hold the
     // un-normalised gradients written by pool_relu_bwd, and conv dgrad / wgrad form dy while staging their tiles (after the
     // reductions in w.red2 / w.red1 are complete -- all-reduced by the caller under data parallelism).
@@ -873,10 +965,10 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
     if (phases & 2) {
         if (!fold) {
             rc = launch_bn_relu_pool_bwd(w.y2, w.stats2, P + po.bn2_g, P + po.bn2_b, rm2, rv2, nullptr, B, m.O, m.L2c, m.training, 1, w.dy2,
-                                         G + po.bn2_g, G + po.bn2_b, w.red2, st, 2, m.Bg, gscale);
+                                         gk(6), gk(7), w.red2, st, 2, m.Bg, gscale);
             if (rc) return rc;
         }
-        const BnBwd bn2w = {fold ? w.y2 : nullptr, w.stats2, P + po.bn2_g, P + po.bn2_b, rm2, rv2, w.red2, G + po.bn2_g, G + po.bn2_b, m.Bg, m.training, gscale};
+        const BnBwd bn2w = {fold ? w.y2 : nullptr, w.stats2, P + po.bn2_g, P + po.bn2_b, rm2, rv2, w.red2, gs(6), gs(7), m.Bg, m.training, gscale};
         BnBwd bn2d = bn2w;
         bn2d.dgamma = nullptr; bn2d.dbeta = nullptr;
         if (bwd2) {
@@ -887,50 +979,62 @@ static int model_backward(const mms_cnngru_desc* d, const float* x, const float*
             }
             rc = fk.wait_mark();
             if (rc) return rc;
-            rc = launch_conv2_bwd(w.dy2, w.c2_wd, w.p1, B, m.P1, w.dp1, w.c2_part, st, &bn2w);
+            // with stage 1 frozen the kernel forms the weight gradient alone (no dp1)
+            rc = launch_conv2_bwd(w.dy2, w.c2_wd, w.p1, B, m.P1, lv.enc1 ? w.dp1 : nullptr, w.c2_part, st, &bn2w);
             if (rc) return rc;
-            rc = launch_wgrad_reduce(w.c2_part, conv2_bwd_parts(B, m.P1), m.O * CONV2_CI * CONV2_K, G + po.conv2_w, fk.fork(0));
-            if (rc) return rc;
-            rc = launch_pool_bwd_ncl(w.y1, w.stats1, P + po.bn1_g, P + po.bn1_b, rm1, rv1, w.dp1, B, CONV1_CO, m.L1c, m.training, w.dy1,
-                                     w.red1, st, m.Bg);
-            if (rc) return rc;
+            if (lv.seg[5]) {
+                rc = launch_wgrad_reduce(w.c2_part, conv2_bwd_parts(B, m.P1), m.O * CONV2_CI * CONV2_K, gs(5), fk.fork(0));
+                if (rc) return rc;
+            }
+            if (lv.enc1) {
+                rc = launch_pool_bwd_ncl(w.y1, w.stats1, P + po.bn1_g, P + po.bn1_b, rm1, rv1, w.dp1, B, CONV1_CO, m.L1c, m.training, w.dy1,
+                                         w.red1, st, m.Bg);
+                if (rc) return rc;
+            }
         } else {
-        rc = launch_conv_wgrad(2, w.p1, w.dy2, nullptr, B, CONV2_CI, m.O, m.P1, G + po.conv2_w, fk.fork(0), &bn2w);
-        if (rc) return rc;
-        rc = launch_conv_dgrad(2, w.dy2, P + po.conv2_w, B, CONV2_CI, m.O, m.P1, w.dp1, nullptr, nullptr, st, &bn2d);
-        if (rc) return rc;
-        rc = launch_bn_relu_pool_bwd(w.y1, w.stats1, P + po.bn1_g, P + po.bn1_b, rm1, rv1, w.dp1, B, CONV1_CO, m.L1c, m.training, 0,
-                                     w.dy1, G + po.bn1_g, G + po.bn1_b, w.red1, st, 1, m.Bg, gscale);
-        if (rc) return rc;
+        // the weight-gradient kernel also adds the BN2 affine gradients (BnBwd)
+        if (lv.seg[5] || lv.seg[6] || lv.seg[7]) {
+            rc = launch_conv_wgrad(2, w.p1, w.dy2, nullptr, B, CONV2_CI, m.O, m.P1, gk(5), fk.fork(0), &bn2w);
+            if (rc) return rc;
+        }
+        if (lv.enc1) {
+            rc = launch_conv_dgrad(2, w.dy2, P + po.conv2_w, B, CONV2_CI, m.O, m.P1, w.dp1, nullptr, nullptr, st, &bn2d);
+            if (rc) return rc;
+            rc = launch_bn_relu_pool_bwd(w.y1, w.stats1, P + po.bn1_g, P + po.bn1_b, rm1, rv1, w.dp1, B, CONV1_CO, m.L1c, m.training, 0,
+                                         w.dy1, gk(3), gk(4), w.red1, st, 1, m.Bg, gscale);
+            if (rc) return rc;
+        }
         }
     }
-    if (!(phases & 4)) return fk.join();
+    if (!(phases & 4) || !lv.enc1) return fk.join();
     if (bwd2) {
         // conv1 weight gradient, attention-gate gradient and the ChannelAttention parameter gradients in one launch
-        const BnBwd bn1f = {w.y1, w.stats1, P + po.bn1_g, P + po.bn1_b, rm1, rv1, w.red1, G + po.bn1_g, G + po.bn1_b, m.Bg, m.training, gscale};
+        const BnBwd bn1f = {w.y1, w.stats1, P + po.bn1_g, P + po.bn1_b, rm1, rv1, w.red1, gs(3), gs(4), m.Bg, m.training, gscale};
         rc = launch_conv1_bwd(x, w.dy1, P + po.conv1_w, m.attention ? w.gate : nullptr, w.mean, P + po.ca_w1, P + po.ca_w2, B, m.C, m.T,
-                              w.c1_part, w.row_counter, G + po.conv1_w, G + po.ca_w1, G + po.ca_w2, st, &bn1f);
+                              w.c1_part, w.row_counter, gk(2), gk(0), gk(1), st, &bn1f);
         if (rc) return rc;
         return fk.join();
     }
     if (!fold) {
         rc = launch_bn_relu_pool_bwd(w.y1, w.stats1, P + po.bn1_g, P + po.bn1_b, rm1, rv1, nullptr, B, CONV1_CO, m.L1c, m.training, 0,
-                                     w.dy1, G + po.bn1_g, G + po.bn1_b, w.red1, st, 2, m.Bg, gscale);
+                                     w.dy1, gk(3), gk(4), w.red1, st, 2, m.Bg, gscale);
         if (rc) return rc;
     }
-    const BnBwd bn1w = {fold ? w.y1 : nullptr, w.stats1, P + po.bn1_g, P + po.bn1_b, rm1, rv1, w.red1, G + po.bn1_g, G + po.bn1_b, m.Bg, m.training, gscale};
+    const BnBwd bn1w = {fold ? w.y1 : nullptr, w.stats1, P + po.bn1_g, P + po.bn1_b, rm1, rv1, w.red1, gs(3), gs(4), m.Bg, m.training, gscale};
     BnBwd bn1d = bn1w;
     bn1d.dgamma = nullptr; bn1d.dbeta = nullptr;
-    rc = launch_conv_wgrad(1, x, w.dy1, m.attention ? w.gate : nullptr, B, m.C, CONV1_CO, m.T, G + po.conv1_w, fk.fork(1), &bn1w);
-    if (rc) return rc;
+    if (lv.seg[2] || lv.seg[3] || lv.seg[4]) {     // the weight-gradient kernel also adds the BN1 affine gradients
+        rc = launch_conv_wgrad(1, x, w.dy1, m.attention ? w.gate : nullptr, B, m.C, CONV1_CO, m.T, gk(2), fk.fork(1), &bn1w);
+        if (rc) return rc;
+    }
     if (m.attention) {
-        if (m.A > 0 || dx) {
+        if ((m.A > 0 && lv.attn) || dx) {
             // dx (if requested) first receives d(x*gate); dgate[b,c] = sum_t d(x*gate) * x
             rc = launch_conv_dgrad(1, w.dy1, P + po.conv1_w, B, m.C, CONV1_CO, m.T, dx, x, w.dgate, st, &bn1d);
             if (rc) return rc;
             float* ds = dx && m.A > 0 ? w.ca_scratch : nullptr;
             rc = launch_chan_param_bwd(w.dgate, w.mean, w.gate, P + po.ca_w1, P + po.ca_w2, B, m.C, w.ca_scratch + (int64_t)B * m.C, ds,
-                                       G + po.ca_w1, G + po.ca_w2, st);
+                                       gk(0), gk(1), st);
             if (rc) return rc;
             if (dx) {
                 rc = launch_chan_dx(dx, w.gate, ds, B, m.C, m.T, dx, st);
@@ -1148,12 +1252,30 @@ extern "C" int mms_cnngru_train_step(const mms_cnngru_desc* d, const float* x, c
     make_params(m, &po);
     Workspace w;
     carve(m, (char*)workspace, &w);
+    // fine-tuning: Adam over the trainable tensors' ranges, which must leave the frozen segments' (untouched) gradient slots alone
+    const uint64_t frozen = d->frozen_segments;
+    AdamRanges ranges;
+    const bool by_range = d->adam_steps != nullptr;
+    MMS_REQUIRE(by_range || (d->adam_nranges == 0 && !d->adam_ranges_host), "train_step: an Adam range table without adam_steps");
+    MMS_REQUIRE(by_range || !frozen, "train_step: frozen segments need the Adam range table (adam_steps, adam_ranges_host)");
+    if (by_range) {
+        rc = adam_ranges_from_host(d->adam_ranges_host, d->adam_nranges, po.total, &ranges);
+        if (rc) return rc;
+        for (int k = 0; k < ranges.n; ++k)
+            for (int sg = 0; sg < po.nseg; ++sg)
+                MMS_REQUIRE(!((frozen >> sg) & 1ull) || ranges.off[k] + ranges.cnt[k] <= po.off[sg] ||
+                                po.off[sg] + po.size[sg] <= ranges.off[k],
+                            "train_step: Adam range %d overlaps frozen segment %d", k, sg);
+    }
     const bool fuse_head = option_get("HEAD_FUSED", 1) == 1;
     // zero_grad (trainer.py:144): nothing writes a gradient before the backward pass, so with the fused head the memset runs on
     // a side stream of the forward instead of in front of its first kernel
-    if (!fuse_head) MMS_CUDA(cudaMemsetAsync(grads, 0, po.total * sizeof(float), st));
+    if (!fuse_head) {
+        rc = zero_trainable(grads, po, frozen, st);
+        if (rc) return rc;
+    }
     const bool zero_bwd = fuse_head && fwd_is_fused(m, x);
-    const FusedLoss fl = {labels, loss_out, loss_sum_accum, grads, po.total * sizeof(float), zero_bwd};
+    const FusedLoss fl = {labels, loss_out, loss_sum_accum, grads, &po, frozen, zero_bwd};
     rc = model_forward(d, x, params, bn_buffers, num_batches_tracked, workspace, logits, st, 7, fuse_head ? &fl : nullptr);  // trainer.py:146-147
     if (rc) return rc;
     if (!fuse_head) {
@@ -1163,6 +1285,9 @@ extern "C" int mms_cnngru_train_step(const mms_cnngru_desc* d, const float* x, c
     }
     rc = model_backward(d, x, params, bn_buffers, workspace, w.dlogits, grads, nullptr, st, 7, fuse_head, zero_bwd);        // trainer.py:148
     if (rc) return rc;
+    if (by_range)
+        return launch_adam_ranges(params, grads, exp_avg, exp_avg_sq, ranges, d->adam_steps, lr_dev, beta1, beta2, eps, weight_decay,
+                                  step_dev, scratch_dev, st);
     return launch_adam(params, grads, exp_avg, exp_avg_sq, po.total, lr_dev, beta1, beta2, eps, weight_decay, step_dev,
                        scratch_dev, st);                                                          // trainer.py:149
 }

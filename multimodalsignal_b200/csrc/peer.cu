@@ -113,52 +113,66 @@ __global__ void __launch_bounds__(256) peer_allreduce_f64_kernel(const PeerPtrs 
     if (tid == 0) *epoch_dev = e;
 }
 
-// Fused gradient all-reduce + Adam (same update rule as adam_flat_kernel in head_opt.cu).  CTA 0 tells the peers that this
+// Fused gradient all-reduce + Adam (adam_update, the rule of adam_flat_kernel in head_opt.cu).  CTA 0 tells the peers that this
 // rank's gradient is complete; EVERY CTA waits for the peers' signals on the rank's own pad (no CTA waits for another CTA of
 // the same launch, so nothing depends on co-residency); the last CTA to finish runs the closing barrier.
-__global__ void __launch_bounds__(256) peer_allreduce_adam_kernel(float* __restrict__ p, const PeerPtrs pp, float* __restrict__ m,
-                                                                  float* __restrict__ v, int64_t n, const float* __restrict__ lr_dev,
-                                                                  float beta1, float beta2, float eps, float wd, int64_t* step_dev,
-                                                                  int world, int rank, int base, uint32_t* epoch_dev,
-                                                                  uint32_t* done_dev, uint64_t timeout_ns) {
+// RANGES: only the elements of `r` are summed and updated, range k with its own step count steps[r.slot[k]] (see
+// adam_ranges_kernel); otherwise the whole buffer with *step_dev.
+template <bool RANGES>
+__device__ __forceinline__ void peer_adam_body(float* __restrict__ p, const PeerPtrs& pp, float* __restrict__ m, float* __restrict__ v,
+                                               int64_t n, const AdamRanges* r, int64_t* steps, const float* __restrict__ lr_dev,
+                                               float beta1, float beta2, float eps, float wd, int64_t* step_dev, int world, int rank,
+                                               int base, uint32_t* epoch_dev, uint32_t* done_dev, uint64_t timeout_ns) {
     const int tid = threadIdx.x;
     const uint32_t e = *epoch_dev + 1;
-    const double t = (double)(*step_dev + 1);
     const float lr = *lr_dev;
+    __shared__ AdamCoef s_c[RANGES ? MMS_MAX_ADAM_RANGES : 1];
+    if (RANGES)
+        for (int k = tid; k < r->n; k += blockDim.x) s_c[k] = adam_coef(steps[r->slot[k]], lr, beta1, beta2);
+    const AdamCoef c = RANGES ? AdamCoef{0.f, 0.f} : adam_coef(*step_dev, lr, beta1, beta2);
     if (blockIdx.x == 0) peer_signal(pp, world, rank, base, e, tid);      // this rank's gradient buffer is complete (stream order)
     peer_wait(pp, world, rank, base, e, tid, timeout_ns);                   // ... and so is every peer's
     __syncthreads();
-    const float bc1 = (float)(1.0 - pow((double)beta1, t));
-    const float bc2_sqrt = (float)sqrt(1.0 - pow((double)beta2, t));
-    const float step_size = lr / bc1;
-    const int64_t n4 = n >> 2;
-    for (int64_t i4 = (int64_t)blockIdx.x * blockDim.x + tid; i4 < n4; i4 += (int64_t)gridDim.x * blockDim.x) {
-        float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (int q = 0; q < world; ++q) {
-            const float4 x = ld_relaxed_sys_f4(reinterpret_cast<const float*>(pp.buf[q]) + 4 * i4);
-            g.x += x.x; g.y += x.y; g.z += x.z; g.w += x.w;
+    if (RANGES) {
+        const int64_t stride = (int64_t)gridDim.x * blockDim.x, gt = (int64_t)blockIdx.x * blockDim.x + tid;
+        int64_t vbase = 0;
+        for (int k = 0; k < r->n; ++k) {
+            const AdamCoef ck = s_c[k];
+            int64_t j = (gt - vbase) % stride;
+            if (j < 0) j += stride;
+            for (; j < r->cnt[k]; j += stride) {
+                const int64_t i = r->off[k] + j;
+                float g = 0.f;
+                for (int q = 0; q < world; ++q) g += ld_relaxed_sys_f(reinterpret_cast<const float*>(pp.buf[q]) + i);
+                float mi = m[i], vi = v[i];
+                p[i] = adam_update(p[i], g, mi, vi, ck, beta1, beta2, eps, wd);
+                m[i] = mi;
+                v[i] = vi;
+            }
+            vbase += r->cnt[k];
         }
-        float4 pv = reinterpret_cast<float4*>(p)[i4], mv = reinterpret_cast<float4*>(m)[i4], vv = reinterpret_cast<float4*>(v)[i4];
-        float* gp = &g.x; float* pq = &pv.x; float* mq = &mv.x; float* vq = &vv.x;
+    } else {
+        const int64_t n4 = n >> 2;
+        for (int64_t i4 = (int64_t)blockIdx.x * blockDim.x + tid; i4 < n4; i4 += (int64_t)gridDim.x * blockDim.x) {
+            float4 g = make_float4(0.f, 0.f, 0.f, 0.f);
+            for (int q = 0; q < world; ++q) {
+                const float4 x = ld_relaxed_sys_f4(reinterpret_cast<const float*>(pp.buf[q]) + 4 * i4);
+                g.x += x.x; g.y += x.y; g.z += x.z; g.w += x.w;
+            }
+            float4 pv = reinterpret_cast<float4*>(p)[i4], mv = reinterpret_cast<float4*>(m)[i4], vv = reinterpret_cast<float4*>(v)[i4];
+            float* gp = &g.x; float* pq = &pv.x; float* mq = &mv.x; float* vq = &vv.x;
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const float gi = gp[j] + wd * pq[j];
-            mq[j] = beta1 * mq[j] + (1.f - beta1) * gi;
-            vq[j] = beta2 * vq[j] + (1.f - beta2) * gi * gi;
-            pq[j] = pq[j] - step_size * (mq[j] / (sqrtf(vq[j]) / bc2_sqrt + eps));
+            for (int j = 0; j < 4; ++j) pq[j] = adam_update(pq[j], gp[j], mq[j], vq[j], c, beta1, beta2, eps, wd);
+            reinterpret_cast<float4*>(p)[i4] = pv;
+            reinterpret_cast<float4*>(m)[i4] = mv;
+            reinterpret_cast<float4*>(v)[i4] = vv;
         }
-        reinterpret_cast<float4*>(p)[i4] = pv;
-        reinterpret_cast<float4*>(m)[i4] = mv;
-        reinterpret_cast<float4*>(v)[i4] = vv;
-    }
-    if (blockIdx.x == 0) {                                     // tail (n is a multiple of 4 for every supported layout; kept for safety)
-        for (int64_t i = (n4 << 2) + tid; i < n; i += blockDim.x) {
-            float g = 0.f;
-            for (int q = 0; q < world; ++q) g += ld_relaxed_sys_f(reinterpret_cast<const float*>(pp.buf[q]) + i);
-            const float gi = g + wd * p[i];
-            m[i] = beta1 * m[i] + (1.f - beta1) * gi;
-            v[i] = beta2 * v[i] + (1.f - beta2) * gi * gi;
-            p[i] = p[i] - step_size * (m[i] / (sqrtf(v[i]) / bc2_sqrt + eps));
+        if (blockIdx.x == 0) {                                 // tail (n is a multiple of 4 for every supported layout; kept for safety)
+            for (int64_t i = (n4 << 2) + tid; i < n; i += blockDim.x) {
+                float g = 0.f;
+                for (int q = 0; q < world; ++q) g += ld_relaxed_sys_f(reinterpret_cast<const float*>(pp.buf[q]) + i);
+                p[i] = adam_update(p[i], g, m[i], v[i], c, beta1, beta2, eps, wd);
+            }
         }
     }
     __syncthreads();
@@ -177,8 +191,29 @@ __global__ void __launch_bounds__(256) peer_allreduce_adam_kernel(float* __restr
             *done_dev = 0u;
             *epoch_dev = e;
             *step_dev += 1;
+            if (RANGES)
+                for (int k = 0; k < r->n; ++k) steps[r->slot[k]] += 1;
         }
     }
+}
+
+__global__ void __launch_bounds__(256) peer_allreduce_adam_kernel(float* __restrict__ p, const PeerPtrs pp, float* __restrict__ m,
+                                                                  float* __restrict__ v, int64_t n, const float* __restrict__ lr_dev,
+                                                                  float beta1, float beta2, float eps, float wd, int64_t* step_dev,
+                                                                  int world, int rank, int base, uint32_t* epoch_dev,
+                                                                  uint32_t* done_dev, uint64_t timeout_ns) {
+    peer_adam_body<false>(p, pp, m, v, n, nullptr, nullptr, lr_dev, beta1, beta2, eps, wd, step_dev, world, rank, base, epoch_dev,
+                          done_dev, timeout_ns);
+}
+
+__global__ void __launch_bounds__(256) peer_allreduce_adam_ranges_kernel(float* __restrict__ p, const PeerPtrs pp, float* __restrict__ m,
+                                                                         float* __restrict__ v, const __grid_constant__ AdamRanges r,
+                                                                         int64_t* steps, const float* __restrict__ lr_dev, float beta1,
+                                                                         float beta2, float eps, float wd, int64_t* step_dev, int world,
+                                                                         int rank, int base, uint32_t* epoch_dev, uint32_t* done_dev,
+                                                                         uint64_t timeout_ns) {
+    peer_adam_body<true>(p, pp, m, v, 0, &r, steps, lr_dev, beta1, beta2, eps, wd, step_dev, world, rank, base, epoch_dev, done_dev,
+                         timeout_ns);
 }
 
 static int fill_peer(PeerPtrs* pp, const void* const* bufs_host, void* const* signals_host, int world) {
@@ -246,5 +281,33 @@ extern "C" int mms_peer_allreduce_adam(float* params, const void* const* grads_h
     peer_allreduce_adam_kernel<<<blocks, 256, 0, st>>>(params, pp, exp_avg, exp_avg_sq, n, lr_dev, beta1, beta2, eps, weight_decay,
                                                        step_dev, world, rank, signal_base, epoch_dev, scratch2_dev + 1, peer_timeout_ns());
     MMS_LAUNCH_CHECK("peer_allreduce_adam_kernel");
+    return MMS_OK;
+}
+
+extern "C" int mms_peer_allreduce_adam_ranges(float* params, const void* const* grads_host, void* const* signals_host, int32_t world,
+                                              int32_t rank, int32_t signal_base, float* exp_avg, float* exp_avg_sq,
+                                              const int64_t* ranges_host, int32_t nranges, int64_t* steps_dev, const float* lr_dev,
+                                              float beta1, float beta2, float eps, float weight_decay, int64_t* step_dev,
+                                              uint32_t* epoch_dev, uint32_t* scratch2_dev, mms_stream_t stream) {
+    MMS_REQUIRE(params && grads_host && signals_host && exp_avg && exp_avg_sq && steps_dev && lr_dev && step_dev && epoch_dev &&
+                    scratch2_dev && rank >= 0 && rank < world && signal_base >= 0,
+                "peer_allreduce_adam_ranges: bad arguments");
+    AdamRanges r;
+    int rc = adam_ranges_from_host(ranges_host, nranges, INT64_MAX / 2, &r);
+    if (rc) return rc;
+    PeerPtrs pp;
+    rc = fill_peer(&pp, grads_host, signals_host, world);
+    if (rc) return rc;
+    int64_t n = 0;
+    for (int k = 0; k < r.n; ++k) n += r.cnt[k];
+    int blocks = (int)((n + 255) / 256);
+    if (blocks > 64) blocks = 64;
+    if (blocks < 1) blocks = 1;
+    cudaStream_t st = (cudaStream_t)stream;
+    MMS_PROF_BEGIN(st);
+    peer_allreduce_adam_ranges_kernel<<<blocks, 256, 0, st>>>(params, pp, exp_avg, exp_avg_sq, r, steps_dev, lr_dev, beta1, beta2, eps,
+                                                              weight_decay, step_dev, world, rank, signal_base, epoch_dev,
+                                                              scratch2_dev + 1, peer_timeout_ns());
+    MMS_LAUNCH_CHECK("peer_allreduce_adam_ranges_kernel");
     return MMS_OK;
 }

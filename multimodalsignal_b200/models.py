@@ -115,12 +115,18 @@ class _Engine:
         self.generation += 1
         return logits
 
-    def backward(self, x, dlogits, want_dx):
+    def backward(self, x, dlogits, want_dx, frozen_segments=0):
+        """Parameter gradients (flat, zeros in frozen segments) and optionally dx; the backward stops as early as the
+        mask of frozen segments allows (desc.frozen_segments)."""
         m = self.model
         grads = torch.zeros_like(m._flat)
         dx = torch.empty_like(x) if want_dx else None
-        check(self.lib.mms_cnngru_backward(C.byref(self.desc), ptr(x), ptr(m._flat), ptr(m._bn_flat), ptr(self.workspace),
-                                           ptr(dlogits), ptr(grads), ptr(dx), stream()))
+        self.desc.frozen_segments = frozen_segments
+        try:
+            check(self.lib.mms_cnngru_backward(C.byref(self.desc), ptr(x), ptr(m._flat), ptr(m._bn_flat), ptr(self.workspace),
+                                               ptr(dlogits), ptr(grads), ptr(dx), stream()))
+        finally:
+            self.desc.frozen_segments = 0
         return grads, dx
 
     def input_gradient(self, x, dlogits, dx=None):
@@ -149,14 +155,16 @@ class _CnnGruFn(torch.autograd.Function):
                                 "holds one step (the reference trainer does forward->backward per batch, trainer.py:146-148)")
         (x,) = ctx.saved_tensors
         model = ctx.model
-        if not eng.desc.training and ctx.needs_input_grad[0] and not any(ctx.needs_input_grad[4:]):
-            # eval mode with frozen parameters (model.eval().requires_grad_(False)): the input gradient alone, no
-            # parameter-gradient work at all
+        want = ctx.needs_input_grad[4:]
+        mask, _ = model.freeze_plan(want)
+        if not any(want) and not eng.desc.training:
+            # eval mode with every parameter frozen (model.eval().requires_grad_(False)): the input gradient alone, through
+            # the eval-mode encoder kernels, no parameter-gradient work at all
             dx = eng.input_gradient(x, dlogits.contiguous().float())
-            return (dx, None, None, None, *([None] * len(model._param_views)))
-        grads, dx = eng.backward(x, dlogits.contiguous().float(), ctx.needs_input_grad[0])
-        out = [grads[o:o + n].view(shape) if n else torch.zeros(shape, device=grads.device)
-               for (o, n, shape) in model._param_views]
+            return (dx, None, None, None, *([None] * len(want)))
+        grads, dx = eng.backward(x, dlogits.contiguous().float(), ctx.needs_input_grad[0], mask)
+        out = [(grads[o:o + n].view(shape) if n else torch.zeros(shape, device=grads.device)) if w else None
+               for (o, n, shape), w in zip(model._param_views, want)]
         return (dx, None, None, None, *out)
 
 
@@ -254,6 +262,35 @@ class CnnGruAttentionModel(nn.Module):
                 assert sizes[seg] == 2 * n
             out.append((name, offs[seg] + half * n, n, tuple(p.shape)))
         return out, total
+
+    def freeze_plan(self, trainable=None):
+        """What fine-tuning with frozen parameters (``requires_grad_(False)``) asks of the library:
+        ``(frozen_segments, ranges)``.  ``trainable``: one flag per parameter in ``parameters()`` order (default: the
+        parameters' ``requires_grad``).  Bit s of ``frozen_segments`` is set when segment s of the flat layout holds
+        elements and every one of its non-empty tensors is frozen -- one GRU direction frozen and the other trainable keeps
+        the segment's gradient computed.  ``ranges`` is one ``(offset, count, slot)`` per trainable non-empty tensor, slot =
+        the tensor's index in ``parameters()``: the flat ranges Adam updates, each with its own step count.  Host-only."""
+        flags = tuple(p.requires_grad for p in self.parameters()) if trainable is None else tuple(bool(t) for t in trainable)
+        cache = getattr(self, "_plan_cache", None)
+        if cache is not None and cache[0] == flags:
+            return cache[1]
+        layout, _ = self.flat_layout()
+        if len(flags) != len(layout):
+            raise ValueError(f"freeze_plan: {len(flags)} flags for {len(layout)} parameters")
+        table, nseg = self._segments()
+        frozen_only = [None] * nseg              # per segment: True = every non-empty tensor frozen, None = no elements
+        ranges = []
+        for slot, ((name, off, n, _), t) in enumerate(zip(layout, flags)):
+            if n == 0:
+                continue
+            seg = table[name][0]
+            frozen_only[seg] = (frozen_only[seg] is not False) and not t
+            if t:
+                ranges.append((off, n, slot))
+        mask = sum(1 << s for s, f in enumerate(frozen_only) if f)
+        plan = (mask, tuple(ranges))
+        self._plan_cache = (flags, plan)
+        return plan
 
     def _flatten(self, device):
         layout, total = self.flat_layout()

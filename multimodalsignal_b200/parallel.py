@@ -73,6 +73,7 @@ class DataParallelTrainStep:
         self.loss = torch.zeros(1, dtype=torch.float32, device=dev)        # this rank's share of the global mean
         self._sync_offsets = [(int(offs[i]), int(cnts[i])) for i in range(4)]
         self.use_graph, self.graph, self.calls = use_graph, None, 0
+        self._graphs, self._eager_done, self._table = {}, set(), None     # peer path: one graph per freeze plan
         self.x = torch.zeros(local_batch, model.in_channels, seq_len, dtype=torch.float32, device=dev)
         self.y = torch.zeros(local_batch, dtype=torch.int64, device=dev)
         if peer is not None:
@@ -127,6 +128,7 @@ class DataParallelTrainStep:
         """The whole data-parallel step with the peer kernels at the five exchange points, as a generator that yields
         after every exchange kernel has been enqueued (the single-process emulation interleaves the ranks there)."""
         x, y, o, g = self.x, self.y, self.opt, self.opt.param_groups[0]
+        self._set_plan()
         o.grads.zero_()                                          # trainer.py:144
         self._fwd(1, x)
         self._weight_sum(y)
@@ -145,24 +147,40 @@ class DataParallelTrainStep:
         yield
         self._bwd(4, x)
         _, grads, sig = self._peer_tables()
-        check(self.lib.mms_peer_allreduce_adam(ptr(self.flat), grads, sig, self.world, self.rank, 0, ptr(o.exp_avg), ptr(o.exp_avg_sq),
-                                               self.flat.numel(), ptr(o.lr_dev), g['betas'][0], g['betas'][1], g['eps'],
-                                               g['weight_decay'], ptr(o.step_dev), ptr(self.epoch), ptr(self.scratch2), stream()))   # :149
+        if self._table is None:
+            check(self.lib.mms_peer_allreduce_adam(ptr(self.flat), grads, sig, self.world, self.rank, 0, ptr(o.exp_avg), ptr(o.exp_avg_sq),
+                                                   self.flat.numel(), ptr(o.lr_dev), g['betas'][0], g['betas'][1], g['eps'],
+                                                   g['weight_decay'], ptr(o.step_dev), ptr(self.epoch), ptr(self.scratch2), stream()))   # :149
+        else:                       # frozen parameters: the update (and the sum it reads) over the trainable tensors only
+            check(self.lib.mms_peer_allreduce_adam_ranges(ptr(self.flat), grads, sig, self.world, self.rank, 0, ptr(o.exp_avg),
+                                                          ptr(o.exp_avg_sq), self._table, len(self._table) // 3, ptr(o.tensor_steps),
+                                                          ptr(o.lr_dev), g['betas'][0], g['betas'][1], g['eps'], g['weight_decay'],
+                                                          ptr(o.step_dev), ptr(self.epoch), ptr(self.scratch2), stream()))
 
     def _enqueue_peer(self):
         for _ in self._peer_phases():
             pass
 
+    def _set_plan(self):
+        """Reads the parameters' ``requires_grad`` (FlatAdam.plan) into the descriptor; returns the plan's graph key."""
+        mask, table = self.opt.plan()
+        self.desc.frozen_segments = mask
+        self._table = table
+        return mask, None if table is None else tuple(table)
+
     def run_peer(self):
-        """One step on the static inputs ``self.x`` / ``self.y`` (graph replay after the first call)."""
+        """One step on the static inputs ``self.x`` / ``self.y`` (graph replay after the first call of each freeze plan)."""
         from .trainer import capture_graph
         self.opt.sync_lr()
         self.calls += 1
-        if not self.use_graph or self.calls == 1:
+        key = self._set_plan()
+        if not self.use_graph or key not in self._eager_done:
+            self._eager_done.add(key)
             self._enqueue_peer()
             return
+        self.graph = self._graphs.get(key)
         if self.graph is None:
-            self.graph = capture_graph(self._enqueue_peer)
+            self.graph = self._graphs[key] = capture_graph(self._enqueue_peer)
         self.graph.replay()
 
     def _weight_sum(self, y):
@@ -195,6 +213,7 @@ class DataParallelTrainStep:
         """Generator over the step: yields each tensor that must be sum-reduced over the ranks before it resumes."""
         x = x.contiguous().float()
         y = y.contiguous()
+        self._set_plan()
         self.opt.grads.zero_()                                   # trainer.py:144
         self._fwd(1, x)
         self._weight_sum(y)

@@ -193,7 +193,12 @@ class FlatAdam(torch.optim.Optimizer):
     """``torch.optim.Adam(model.parameters(), lr, weight_decay)`` (reference trainer.py:68) over
     the model's flat parameter buffer: one kernel for all 30 tensors.  It is a real
     ``Optimizer`` (``param_groups[0]['lr']`` is what ``ReduceLROnPlateau`` edits, trainer.py:72-77);
-    the learning rate and the step count live on the device so the step can be graph-replayed."""
+    the learning rate and the step count live on the device so the step can be graph-replayed.
+
+    Frozen parameters follow torch: a tensor that is not updated (``step()``: no ``.grad``; ``flat_step()`` and the fused
+    steps: ``requires_grad`` False) keeps its value, its moments and its step count, and on unfreezing continues from
+    them.  The per-tensor step counts (``tensor_steps``) are used from the first step that leaves a tensor out; until then
+    every tensor's count is ``step_dev`` and the single whole-buffer kernel runs."""
 
     def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0):
         params = [p for p in model.parameters()]
@@ -206,6 +211,9 @@ class FlatAdam(torch.optim.Optimizer):
         self.lr_dev = torch.full((1,), float(lr), dtype=torch.float32, device=flat.device)
         self.step_dev = torch.zeros(1, dtype=torch.int64, device=flat.device)
         self.scratch = torch.zeros(1, dtype=torch.int32, device=flat.device)
+        self.tensor_steps = torch.zeros(len(params), dtype=torch.int64, device=flat.device)
+        self._per_tensor = False            # tensor_steps in use (some step has left a tensor out)
+        self._tables = {}                   # ranges -> HOST int64 [n][3] table (kept alive for the library)
         self._lr_on_device = float(lr)
 
     def sync_lr(self):
@@ -214,25 +222,61 @@ class FlatAdam(torch.optim.Optimizer):
             self.lr_dev.fill_(lr)
             self._lr_on_device = lr
 
+    def plan(self, trainable=None):
+        """``(frozen_segments, table)`` for a step that updates the tensors flagged in ``trainable`` (default: their
+        ``requires_grad``; see ``CnnGruAttentionModel.freeze_plan``).  ``table`` is None while every tensor trains and no
+        earlier step left one out (the whole-buffer kernel, ``step_dev`` as every count); otherwise the HOST ctypes array
+        of the Adam ranges, ``len(table) // 3`` of them, and from then on the per-tensor counts are in use."""
+        mask, ranges = self.model.freeze_plan(trainable)
+        everything = len(ranges) == sum(1 for (_, n, _) in self.model._param_views if n)
+        if everything and not self._per_tensor:
+            return mask, None
+        if not self._per_tensor:            # every tensor's count so far is the global one
+            self.tensor_steps.copy_(self.step_dev.expand_as(self.tensor_steps))
+            self._per_tensor = True
+        table = self._tables.get(ranges)
+        if table is None:
+            table = self._tables[ranges] = (C.c_int64 * max(1, 3 * len(ranges)))(*[v for r in ranges for v in r])
+        return mask, table
+
     @torch.no_grad()
     def step(self, closure=None):
-        """Generic path: gather ``p.grad`` into the flat gradient buffer, then one Adam launch."""
-        lib = _ext.lib()
+        """Generic path: gather ``p.grad`` into the flat gradient buffer, then one Adam launch over the tensors that have a
+        gradient (torch skips the others)."""
         flat = self.model.flat_parameters()
         self.grads.zero_()
-        for (off, n, _), p in zip(self.model._param_views, self.model.parameters()):
+        params = list(self.model.parameters())
+        for (off, n, _), p in zip(self.model._param_views, params):
             if n and p.grad is not None:
                 self.grads[off:off + n].copy_(p.grad.reshape(-1))
-        self.flat_step(flat)
+        self._update(flat, [p.grad is not None for p in params])
 
     def flat_step(self, flat=None):
+        """Adam over the flat gradient buffer for the parameters that currently require a gradient."""
+        self._update(self.model.flat_parameters() if flat is None else flat, None)
+
+    def _update(self, flat, trainable):
         lib = _ext.lib()
-        flat = self.model.flat_parameters() if flat is None else flat
         self.sync_lr()
         g = self.param_groups[0]
-        check(lib.mms_adam_flat_step(ptr(flat), ptr(self.grads), ptr(self.exp_avg), ptr(self.exp_avg_sq), flat.numel(),
-                                     ptr(self.lr_dev), g['betas'][0], g['betas'][1], g['eps'], g['weight_decay'],
-                                     ptr(self.step_dev), ptr(self.scratch), stream()))
+        _, table = self.plan(trainable)
+        if table is None:
+            check(lib.mms_adam_flat_step(ptr(flat), ptr(self.grads), ptr(self.exp_avg), ptr(self.exp_avg_sq), flat.numel(),
+                                         ptr(self.lr_dev), g['betas'][0], g['betas'][1], g['eps'], g['weight_decay'],
+                                         ptr(self.step_dev), ptr(self.scratch), stream()))
+        else:
+            check(lib.mms_adam_ranges_step(ptr(flat), ptr(self.grads), ptr(self.exp_avg), ptr(self.exp_avg_sq), table,
+                                           len(table) // 3, ptr(self.tensor_steps), ptr(self.lr_dev),
+                                           g['betas'][0], g['betas'][1], g['eps'], g['weight_decay'], ptr(self.step_dev),
+                                           ptr(self.scratch), stream()))
+
+    def set_plan(self, desc, plan):
+        """Writes ``plan`` (from ``plan()``) into a train-step descriptor."""
+        mask, table = plan
+        desc.frozen_segments = mask
+        desc.adam_ranges_host = None if table is None else C.addressof(table)
+        desc.adam_steps = None if table is None else self.tensor_steps.data_ptr()
+        desc.adam_nranges = 0 if table is None else len(table) // 3
 
 
 def class_weight_tensor(weight, num_classes, device):
@@ -281,6 +325,8 @@ class FusedTrainStep:
         self.graph = None
         self.calls = 0
         self.kernels_per_step = None
+        # one graph per freeze plan (requires_grad flags, read at every step): progressive unfreezing switches graphs
+        self._graphs, self._eager_done, self._plan = {}, set(), None
 
     def set_class_weight(self, weight):
         """New class weights for the following steps (a stream-ordered copy into the tensor the graph reads)."""
@@ -343,16 +389,21 @@ class FusedTrainStep:
         self.run()
 
     def run(self):
-        """Enqueue one step on the static inputs (graph replay after the first two calls)."""
+        """Enqueue one step on the static inputs (graph replay after the first two calls of each freeze plan)."""
         if self.model._flat is not self.flat:       # .to() / .cuda() drop the flat buffer (models.py: _apply)
             raise _ext.MmsError("the model's parameter storage moved after FusedTrainStep was built")
         self.opt.sync_lr()
         self.calls += 1
-        if not self.use_graph or self.calls == 1:
-            self._enqueue()                       # first call eager: sets kernel attributes, warms caches
+        mask, table = self.opt.plan()
+        key = (mask, None if table is None else tuple(table))
+        self.opt.set_plan(self.desc, (mask, table))
+        if not self.use_graph or key not in self._eager_done:
+            self._eager_done.add(key)
+            self._enqueue()                       # first call of a plan eager: sets kernel attributes, warms caches
             return
+        self.graph = self._graphs.get(key)
         if self.graph is None:
-            self.graph = capture_graph(self._enqueue)
+            self.graph = self._graphs[key] = capture_graph(self._enqueue)
         self.graph.replay()
 
     def post_loss(self):
@@ -717,8 +768,17 @@ class Trainer:
     def train(self, train_loader, val_loader):
         return drive(self.train_async(train_loader, val_loader))
 
+    def _log_frozen(self):
+        """One log line when some parameters are frozen (fine-tuning); nothing otherwise."""
+        params = list(self.model.parameters())
+        if all(p.requires_grad for p in params if p.numel()):
+            return
+        n = sum(p.numel() for p in params if p.requires_grad)
+        self._log(f"Trainable parameters: {n} of {sum(p.numel() for p in params)} (the others are frozen)")
+
     def train_async(self, train_loader, val_loader):
         self._fix_class_weights(train_loader)
+        self._log_frozen()
         best_val_acc = 0
         for epoch in range(self.epochs):
             t0 = time.time()
