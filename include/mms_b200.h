@@ -182,6 +182,30 @@ int mms_ig_interpolate(const float* x, const float* x0, int32_t x0_per_window, c
 int mms_ig_accumulate(const float* x, const float* x0, int32_t x0_per_window, const float* dx, int32_t B, int32_t C,
                       int32_t T, int32_t steps, int64_t row0, int32_t nrows, float* A, double* S, mms_stream_t stream);
 
+/* Monte-Carlo dropout (uncertainty.py): BatchNorm on its running statistics, dropout on, `samples` forward samples per
+ * window.  Sample s of window b, b the window's index within the whole call of the caller, is sample row
+ * r = b * samples + s, and each sample row draws the multipliers a training-mode forward of the expanded batch would draw
+ * at row r: GRU site l (0 <= l < layers - 1) id = l * 2^40 + (r * L + t) * 2H + j, head site id = 2^38 + r * 64 + i, with
+ * one (rng_seed, rng_offset) for every row (oracle/dropout_stream.py).
+ * mms_cnngru_mc_forward: d->batch = the windows x [batch,C,T] of this chunk, d->training = 0, d->need_grad = 0 (other
+ *   descriptor states, global_batch, class_weight and frozen segments are MMS_E_INVALID).  row0 = the chunk's first sample
+ *   row, a multiple of `samples`.  logits [batch*samples, num_classes] in sample-row order.  The encoder and GRU layer 0
+ *   run once per window (no dropout acts before layer 0's output); the layers above and the head run per sample row.  The
+ *   BatchNorm buffers are read, never written.  A call whose site-0 ids would reach the head site,
+ *   (row0 + batch*samples) * L * 2H >= 2^38, is MMS_E_INVALID.
+ * mms_cnngru_mc_workspace_bytes: workspace of such a chunk (-1 for an invalid descriptor).
+ * mms_mc_accumulate: for the rows [row0, row0 + nrows) of B*samples sample rows, logits the chunk's [nrows, num_classes],
+ *   adds in float64 and in increasing s the softmax p_s to psum [B,num_classes] and -sum p_s log p_s to hsum [B] (both
+ *   zeroed by the caller); a window's last sample writes probs = psum/samples, entropy = H(probs) and
+ *   mutual_info = entropy - hsum/samples (float64 [B,num_classes], [B], [B]).  Chunks accumulated in row order give the
+ *   same result however the rows are chunked. */
+int64_t mms_cnngru_mc_workspace_bytes(const mms_cnngru_desc* d, int32_t samples);
+int mms_cnngru_mc_forward(const mms_cnngru_desc* d, const float* x, const float* params, const float* bn_buffers,
+                          void* workspace, int32_t samples, int64_t row0, float* logits, mms_stream_t stream);
+int mms_mc_accumulate(const float* logits, int32_t B, int32_t nc, int32_t samples, int64_t row0, int32_t nrows,
+                      double* psum, double* hsum, double* probs, double* entropy, double* mutual_info,
+                      mms_stream_t stream);
+
 /* Data-parallel form of the two calls above (SURVEY §8e: intra-fold DP).  `phases` is a bit mask:
  *   forward : 1 = gate + conv1 (+BN1 sums) | 2 = BN1/pool1 + conv2 (+BN2 sums) | 4 = the rest
  *   backward: 1 = head..GRU..stage-2 pool/ReLU backward (+BN2 reductions) | 2 = stage-2 BN apply, conv2

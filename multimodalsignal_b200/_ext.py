@@ -92,6 +92,9 @@ _SIGNATURES = {
     "mms_cnngru_forward": (c_i32, [C.POINTER(CnnGruDesc), P, P, P, P, P, P, P]),
     "mms_cnngru_backward": (c_i32, [C.POINTER(CnnGruDesc), P, P, P, P, P, P, P, P]),
     "mms_cnngru_input_gradient": (c_i32, [C.POINTER(CnnGruDesc), P, P, P, P, P, P, P]),
+    "mms_cnngru_mc_workspace_bytes": (c_i64, [C.POINTER(CnnGruDesc), c_i32]),
+    "mms_cnngru_mc_forward": (c_i32, [C.POINTER(CnnGruDesc), P, P, P, P, c_i32, c_i64, P, P]),
+    "mms_mc_accumulate": (c_i32, [P, c_i32, c_i32, c_i32, c_i64, c_i32, P, P, P, P, P, P]),
     "mms_ig_interpolate": (c_i32, [P, P, c_i32, P, c_i32, c_i32, c_i32, c_i32, c_i32, c_i64, c_i32, P, P, P]),
     "mms_ig_accumulate": (c_i32, [P, P, c_i32, P, c_i32, c_i32, c_i32, c_i32, c_i64, c_i32, P, P, P]),
     "mms_cross_entropy": (c_i32, [P, P, c_i32, c_i32, P, P, P, P]),

@@ -11,14 +11,16 @@ constexpr uint64_t HEAD_DROP_BASE = 0x4000000000ull;   // element ids of the hea
 // grid = B, block = 4 * 64: thread (i, q) = (tid >> 2, tid & 3) sums a quarter of hidden unit i's dot product (128-bit
 // weight loads, all in flight at once) and the four quarters meet by shuffles.  hid_out keeps relu(W0 last + b0)
 // (before dropout).  The classifier input is the concatenation [src_a[b, 0:Hh) | src_b[b, 0:H2-Hh)] (forward-direction
-// final state and reverse-direction first-step state, models.py:79); it is also written to last_out.
+// final state and reverse-direction first-step state, models.py:79); it is also written to last_out.  Row b draws its
+// dropout multipliers as row drop_row0 + b of the head site (0 for a whole batch; MC dropout passes its chunk's first
+// sample row).
 __global__ void __launch_bounds__(4 * HEAD_HID) head_fwd_kernel(const float* __restrict__ src_a, int64_t lda,
                                                                 const float* __restrict__ src_b, int64_t ldb, int Hh,
                                                                 const float* __restrict__ w0,
                                                                 const float* __restrict__ b0, const float* __restrict__ w3,
                                                                 const float* __restrict__ b3, int H2, int nc, float p,
                                                                 uint64_t seed, uint64_t offset, const int64_t* offset_dev,
-                                                                float* __restrict__ last_out,
+                                                                int64_t drop_row0, float* __restrict__ last_out,
                                                                 float* __restrict__ hid_out, float* __restrict__ logits) {
     MMS_PDL_PROLOGUE();
     extern __shared__ __align__(16) float s_last[];        // [H2]
@@ -55,7 +57,7 @@ __global__ void __launch_bounds__(4 * HEAD_HID) head_fwd_kernel(const float* __r
         if (p > 0.f) {
             DropRng rng;
             rng.init(seed, resolve_offset(offset, offset_dev), p);
-            m = rng.mult(HEAD_DROP_BASE + (uint64_t)b * HEAD_HID + i);
+            m = rng.mult(HEAD_DROP_BASE + (uint64_t)(drop_row0 + b) * HEAD_HID + i);
         }
         s_hid[i] = h * m;
     }
@@ -399,11 +401,12 @@ int adam_ranges_from_host(const int64_t* table, int n, int64_t total, AdamRanges
 
 int launch_head_fwd2(const float* src_a, int64_t lda, const float* src_b, int64_t ldb, int Hh, const float* w0, const float* b0,
                      const float* w3, const float* b3, int B, int H2, int nc, float p, uint64_t seed, uint64_t offset,
-                     const int64_t* offset_dev, float* last_out, float* hid_out, float* logits, cudaStream_t st) {
+                     const int64_t* offset_dev, float* last_out, float* hid_out, float* logits, cudaStream_t st,
+                     int64_t drop_row0) {
     MMS_REQUIRE(nc >= 1 && nc <= MAX_NC, "head: num_classes %d outside [1,%d]", nc, MAX_NC);
     MMS_PROF_BEGIN(st);
     MMS_LAUNCH(head_fwd_kernel, dim3(B), dim3(4 * HEAD_HID), H2 * sizeof(float), st, src_a, lda, src_b, ldb, Hh, w0, b0, w3, b3, H2, nc, p, seed, offset,
-                                                             offset_dev, last_out, hid_out, logits);
+                                                             offset_dev, drop_row0, last_out, hid_out, logits);
     MMS_LAUNCH_CHECK("head_fwd_kernel");
     return MMS_OK;
 }
@@ -431,7 +434,7 @@ int launch_head_fwd(const float* last, const float* w0, const float* b0, const f
                     int nc, float p, uint64_t seed, uint64_t offset, const int64_t* offset_dev, float* hid_out, float* logits,
                     cudaStream_t st) {
     return launch_head_fwd2(last, H2, last + H2 / 2, H2, H2 / 2, w0, b0, w3, b3, B, H2, nc, p, seed, offset, offset_dev, nullptr,
-                            hid_out, logits, st);
+                            hid_out, logits, st, 0);
 }
 
 int launch_head_bwd(const float* last, const float* hid, const float* dlogits, const float* w3, int B, int H2, int nc, float p,

@@ -32,7 +32,7 @@ int launch_tc_gemm_tn(const float*, int64_t, int, int, const float*, int64_t, in
 int launch_gru_fwd(const mms_gru_dir_fwd*, int, int, int, float, uint64_t, uint64_t, const int64_t*, cudaStream_t);
 int launch_gru_bwd(const mms_gru_dir_bwd*, int, int, int, float, uint64_t, uint64_t, const int64_t*, cudaStream_t);
 int launch_head_fwd2(const float*, int64_t, const float*, int64_t, int, const float*, const float*, const float*, const float*, int,
-                     int, int, float, uint64_t, uint64_t, const int64_t*, float*, float*, float*, cudaStream_t);
+                     int, int, float, uint64_t, uint64_t, const int64_t*, float*, float*, float*, cudaStream_t, int64_t);
 int launch_head_bwd(const float*, const float*, const float*, const float*, int, int, int, float, uint64_t, uint64_t,
                     const int64_t*, float*, float*, float*, float*, float*, cudaStream_t);
 int launch_cross_entropy(const float*, const int64_t*, int, int, float*, float*, double*, cudaStream_t, int div_batch,
@@ -692,7 +692,7 @@ static int model_forward(const mms_cnngru_desc* d, const float* x, const float* 
                                     w.head_counter, fl->loss_out, fl->loss_sum_accum, st, d->class_weight);
     return launch_head_fwd2(w.hs_tf + (int64_t)(L - 1) * H, (int64_t)L * H, w.h_tr, H, H, P + po.fc0_w, P + po.fc0_b, P + po.fc3_w,
                             P + po.fc3_b, B, 2 * H, m.nc, m.drop_head ? m.p : 0.f, d->rng_seed, d->rng_offset, d->rng_offset_dev,
-                            w.last, w.hid, logits, st);
+                            w.last, w.hid, logits, st, 0);
 }
 
 // Appends TN product `c` to list[n] with the frozen outputs removed: no weight gradient (C == nullptr) leaves the bias gradient
@@ -1157,9 +1157,199 @@ static int model_input_gradient(const mms_cnngru_desc* d, const float* x, const 
     return MMS_OK;
 }
 
+int launch_mc_expand(const float*, int64_t, int64_t, int, int64_t, float*, int64_t, float, uint64_t, uint64_t, const int64_t*,
+                     cudaStream_t);
+
+// MC dropout (mms_cnngru_mc_forward): eval-mode BatchNorm, dropout on, `samples` sample rows per window.  No dropout acts
+// before GRU layer 0's output, so the encoder and layer 0 run once on the windows (model_forward's carve and kernels);
+// layer 0's output is then broadcast to the sample rows with the first site's multipliers, and the layers above and the
+// head run on the sample rows.  A 1-layer model shares its whole GRU and only the head's mask varies.
+constexpr int64_t MC_SITE0_LIMIT = 1ll << 38;     // HEAD_DROP_BASE (head_opt.cu): site-0 ids must stay below it
+
+struct McWorkspace {
+    Workspace win;                                  // the windows: encoder, layer 0 (1 layer: the whole GRU)
+    float* in0;                                     // [rows, L, 2H] layer 0's output per sample row, site 0 applied
+    float *gi[MAX_LAYERS], *hs[MAX_LAYERS], *outd[MAX_LAYERS];   // middle layers 1 .. layers-2 on the sample rows
+    float *gi_tf, *gi_tr, *hs_tf, *h_tr;            // top layer on the sample rows
+    float *last_a, *last_b;                         // 1 layer: the windows' classifier input per sample row
+    float *last, *hid;                              // head on the sample rows
+    int64_t total;
+};
+
+static void mc_carve(const Dims& m, int samples, char* base, McWorkspace* w) {
+    carve(m, base, &w->win);
+    int64_t cur = w->win.total;
+    auto take = [&](int64_t bytes) {
+        float* p = base ? (float*)(base + cur) : nullptr;
+        cur = align_up(cur + bytes, 256);
+        return p;
+    };
+    const int64_t R = (int64_t)m.B * samples, L = m.L, H = m.H, M = R * L, f = sizeof(float);
+    memset(w->gi, 0, sizeof(w->gi)); memset(w->hs, 0, sizeof(w->hs)); memset(w->outd, 0, sizeof(w->outd));
+    w->in0 = w->gi_tf = w->gi_tr = w->hs_tf = w->h_tr = w->last_a = w->last_b = nullptr;
+    if (m.layers >= 2) {
+        w->in0 = take(M * 2 * H * f);
+        for (int l = 1; l < m.layers - 1; ++l) {
+            w->gi[l] = take(M * 6 * H * f);
+            w->hs[l] = take(M * 2 * H * f);
+            w->outd[l] = m.p > 0.f ? take(M * 2 * H * f) : w->hs[l];
+        }
+        w->gi_tf = take(M * 3 * H * f);
+        w->gi_tr = take(R * 3 * H * f);
+        w->hs_tf = take(M * H * f);
+        w->h_tr = take(R * H * f);
+    } else {
+        w->last_a = take(R * H * f);
+        w->last_b = take(R * H * f);
+    }
+    w->last = take(R * 2 * H * f);
+    w->hid = take(R * HEAD_HID * f);
+    w->total = cur;
+}
+
+// one bidirectional layer over all L steps of `rows` rows, eval: in [rows, L, I] -> gi [rows*L, 6H] -> hs [rows, L, 2H]
+static int mc_bidir_layer(const Dims& m, const ParamOff& po, const float* P, int l, const float* in, int I, int rows, float* gi,
+                          float* hs, const mms_cnngru_desc* d, cudaStream_t st) {
+    const int H = m.H, L = m.L;
+    const int64_t M = (int64_t)rows * L;
+    int rc = gemm_nt(in, I, P + po.w_ih[l], I, P + po.b_ih[l], gi, 6 * H, (int)M, 6 * H, I, st);
+    if (rc) return rc;
+    mms_gru_dir_fwd dirs[2];
+    memset(dirs, 0, sizeof(dirs));
+    for (int dd = 0; dd < 2; ++dd) {
+        mms_gru_dir_fwd& g = dirs[dd];
+        g.gi = gi + dd * 3 * H; g.gi_bs = (int64_t)L * 6 * H; g.gi_ts = 6 * H;
+        g.w_hh = P + po.w_hh[l] + (int64_t)dd * 3 * H * H;
+        g.b_hh = P + po.b_hh[l] + dd * 3 * H;
+        g.hs = hs + dd * H; g.hs_bs = (int64_t)L * 2 * H; g.hs_ts = 2 * H;
+        g.st_bs = (int64_t)L * 4 * H; g.st_ts = 4 * H;
+        g.t0 = dd ? L - 1 : 0; g.dt = dd ? -1 : 1; g.nsteps = L;
+    }
+    return launch_gru_fwd(dirs, 2, rows, H, 0.f, d->rng_seed, d->rng_offset, d->rng_offset_dev, st);
+}
+
+// the top layer, eval: forward direction over the whole sequence, reverse direction for its first step only (model_forward's
+// top-layer block without dropout, stash or side stream)
+static int mc_top_layer(const Dims& m, const ParamOff& po, const float* P, const float* in, int I, int rows, float* gi_tf, float* gi_tr,
+                        float* hs_tf, float* h_tr, const mms_cnngru_desc* d, cudaStream_t st) {
+    const int H = m.H, L = m.L, l = m.layers - 1;
+    const int64_t M = (int64_t)rows * L;
+    const float* w_rev = P + po.w_ih[l] + (int64_t)3 * H * I;
+    const float* rows_in = in + (int64_t)(L - 1) * I;
+    int rc;
+    if (gemm_skinny_supported(rows_in, (int64_t)L * I, w_rev, I, 1, rows, 3 * H, I))
+        rc = launch_gemm_skinny(rows_in, (int64_t)L * I, w_rev, I, 1, P + po.b_ih[l] + 3 * H, gi_tr, 3 * H, rows, 3 * H, I, 0, 0, 0, 0.f,
+                                d->rng_seed, d->rng_offset, d->rng_offset_dev, st);
+    else
+        rc = gemm_nt(rows_in, (int64_t)L * I, w_rev, I, P + po.b_ih[l] + 3 * H, gi_tr, 3 * H, rows, 3 * H, I, st);
+    if (rc) return rc;
+    rc = gemm_nt(in, I, P + po.w_ih[l], I, P + po.b_ih[l], gi_tf, 3 * H, (int)M, 3 * H, I, st);
+    if (rc) return rc;
+    mms_gru_dir_fwd dirs[2];
+    memset(dirs, 0, sizeof(dirs));
+    dirs[0].gi = gi_tf; dirs[0].gi_bs = (int64_t)L * 3 * H; dirs[0].gi_ts = 3 * H;
+    dirs[0].w_hh = P + po.w_hh[l]; dirs[0].b_hh = P + po.b_hh[l];
+    dirs[0].hs = hs_tf; dirs[0].hs_bs = (int64_t)L * H; dirs[0].hs_ts = H;
+    dirs[0].st_bs = (int64_t)L * 4 * H; dirs[0].st_ts = 4 * H;
+    dirs[0].t0 = 0; dirs[0].dt = 1; dirs[0].nsteps = L;
+    dirs[1].gi = gi_tr; dirs[1].gi_bs = 3 * H; dirs[1].gi_ts = 0;
+    dirs[1].w_hh = P + po.w_hh[l] + (int64_t)3 * H * H; dirs[1].b_hh = P + po.b_hh[l] + 3 * H;
+    dirs[1].hs = h_tr; dirs[1].hs_bs = H; dirs[1].hs_ts = 0;
+    dirs[1].st_bs = 4 * H; dirs[1].st_ts = 0;
+    dirs[1].t0 = L - 1; dirs[1].dt = -1; dirs[1].nsteps = 1;
+    return launch_gru_fwd(dirs, 2, rows, H, 0.f, d->rng_seed, d->rng_offset, d->rng_offset_dev, st);
+}
+
+static int mc_dims(const mms_cnngru_desc* d, int samples, int64_t row0, Dims* m) {
+    int rc = make_dims(d, m);
+    if (rc) return rc;
+    MMS_REQUIRE(!m->training && !m->need_grad, "cnngru_mc_forward: needs training = 0 and need_grad = 0");
+    MMS_REQUIRE(m->Bg == m->B && !m->weighted && d->frozen_segments == 0,
+                "cnngru_mc_forward: global_batch, class_weight and frozen_segments are not used by MC dropout");
+    MMS_REQUIRE(samples >= 1, "cnngru_mc_forward: samples %d < 1", samples);
+    MMS_REQUIRE(row0 >= 0 && row0 % samples == 0, "cnngru_mc_forward: row0 %lld is not a window boundary", (long long)row0);
+    const int64_t rows = (int64_t)m->B * samples;
+    MMS_REQUIRE(rows * m->L < INT32_MAX, "cnngru_mc_forward: %lld sample rows x %d steps is too many for one call", (long long)rows,
+                m->L);
+    // the largest site-0 id, (row0 + rows) * L * 2H - 1, must stay below the head site's base
+    MMS_REQUIRE(row0 < MC_SITE0_LIMIT && (row0 + rows) * ((int64_t)m->L * 2 * m->H) < MC_SITE0_LIMIT,
+                "cnngru_mc_forward: sample rows up to %lld reach the head site's dropout ids (rows * L * 2H >= 2^38)",
+                (long long)(row0 + rows));
+    return MMS_OK;
+}
+
+static int model_mc_forward(const mms_cnngru_desc* d, const float* x, const float* P, const float* bn, void* ws, int samples,
+                            int64_t row0, float* logits, cudaStream_t st) {
+    Dims m;
+    int rc = mc_dims(d, samples, row0, &m);
+    if (rc) return rc;
+    MMS_REQUIRE(x && P && bn && ws && logits, "cnngru_mc_forward: null pointer");
+    ParamOff po;
+    make_params(m, &po);
+    McWorkspace w;
+    mc_carve(m, samples, (char*)ws, &w);
+    const int B = m.B, H = m.H, L = m.L, R = B * samples;
+    const float p = m.p;
+    float* bnw = const_cast<float*>(bn);             // eval mode: the running statistics are read, never written
+    // shared prefix: encoder stages 1 and 2 (model_forward's kernels), BN2/ReLU/pool into the GRU input, layer 0
+    rc = model_forward(d, x, P, bnw, nullptr, ws, logits, st, 3);
+    if (rc) return rc;
+    rc = launch_bn_relu_pool_fwd(w.win.y2, w.win.stats2, P + po.bn2_g, P + po.bn2_b, bnw + 2 * CONV1_CO, bnw + 2 * CONV1_CO + m.O, nullptr,
+                                 B, m.O, m.L2c, 0, 1, w.win.seq, st, B);
+    if (rc) return rc;
+    const float *head_a, *head_b;
+    int64_t lda, ldb;
+    if (m.layers == 1) {
+        rc = mc_top_layer(m, po, P, w.win.seq, m.O, B, w.win.gi_tf, w.win.gi_tr, w.win.hs_tf, w.win.h_tr, d, st);
+        if (rc) return rc;
+        rc = launch_mc_expand(w.win.hs_tf + (int64_t)(L - 1) * H, (int64_t)L * H, H, samples, R, w.last_a, 0, 0.f, 0, 0, nullptr, st);
+        if (rc) return rc;
+        rc = launch_mc_expand(w.win.h_tr, H, H, samples, R, w.last_b, 0, 0.f, 0, 0, nullptr, st);
+        if (rc) return rc;
+        head_a = w.last_a; lda = H; head_b = w.last_b; ldb = H;
+    } else {
+        rc = mc_bidir_layer(m, po, P, 0, w.win.seq, m.O, B, w.win.gi[0], w.win.hs[0], d, st);
+        if (rc) return rc;
+        // per sample row from here: site 0 on layer 0's output, broadcast from the windows
+        const int64_t row_len = (int64_t)L * 2 * H;
+        rc = launch_mc_expand(w.win.hs[0], row_len, row_len, samples, R, w.in0, row0 * row_len, p, d->rng_seed, d->rng_offset,
+                              d->rng_offset_dev, st);
+        if (rc) return rc;
+        const float* in = w.in0;
+        for (int l = 1; l < m.layers - 1; ++l) {
+            rc = mc_bidir_layer(m, po, P, l, in, 2 * H, R, w.gi[l], w.hs[l], d, st);
+            if (rc) return rc;
+            if (p > 0.f) {
+                rc = launch_dropout_apply(w.hs[l], w.outd[l], (int64_t)R * row_len, (int64_t)l * DROP_LAYER_STRIDE + row0 * row_len, p,
+                                          d->rng_seed, d->rng_offset, d->rng_offset_dev, st);
+                if (rc) return rc;
+            }
+            in = w.outd[l];
+        }
+        rc = mc_top_layer(m, po, P, in, 2 * H, R, w.gi_tf, w.gi_tr, w.hs_tf, w.h_tr, d, st);
+        if (rc) return rc;
+        head_a = w.hs_tf + (int64_t)(L - 1) * H; lda = (int64_t)L * H; head_b = w.h_tr; ldb = H;
+    }
+    return launch_head_fwd2(head_a, lda, head_b, ldb, H, P + po.fc0_w, P + po.fc0_b, P + po.fc3_w, P + po.fc3_b, R, 2 * H, m.nc, p,
+                            d->rng_seed, d->rng_offset, d->rng_offset_dev, w.last, w.hid, logits, st, row0);
+}
+
 }  // namespace mms
 
 using namespace mms;
+
+extern "C" int64_t mms_cnngru_mc_workspace_bytes(const mms_cnngru_desc* d, int32_t samples) {
+    Dims m;
+    if (mc_dims(d, samples, 0, &m)) return -1;
+    McWorkspace w;
+    mc_carve(m, samples, nullptr, &w);
+    return w.total;
+}
+
+extern "C" int mms_cnngru_mc_forward(const mms_cnngru_desc* d, const float* x, const float* params, const float* bn_buffers,
+                                     void* workspace, int32_t samples, int64_t row0, float* logits, mms_stream_t stream) {
+    return model_mc_forward(d, x, params, bn_buffers, workspace, samples, row0, logits, (cudaStream_t)stream);
+}
 
 extern "C" int mms_cnngru_param_layout(const mms_cnngru_desc* d, int64_t* offsets_host, int64_t* sizes_host, int32_t max_segments,
                                        int64_t* total_floats_host) {

@@ -46,6 +46,7 @@ PATIENCE = 20
 WEIGHTS_DECAY = 1e-4
 USE_CLASS_WEIGHTS = False                     # class-weighted CrossEntropyLoss, 'balanced' weights (never enabled upstream, SURVEY D9)
 ATTRIBUTION_STEPS = 0                         # > 0: integrated-gradients channel attribution of each fold's test set, this many steps
+MC_DROPOUT_SAMPLES = 0                        # > 0: MC-dropout uncertainty of each fold's test set, this many samples per window
 ALL_SUBJECTS = [f"S{i}" for i in range(2, 18) if i != 12]
 CONCURRENT_FOLDS = int(os.environ.get("MMS_CONCURRENT_FOLDS", "1"))     # folds interleaved per GPU (new; 1 = the reference's loop)
 
@@ -118,6 +119,8 @@ def run_fold_async(fold_index, subject_to_test, run_output_dir, all_channel_name
     if ATTRIBUTION_STEPS > 0:
         att = trainer.channel_attribution(test_loader, steps=ATTRIBUTION_STEPS, channel_names=CHANNELS_TO_USE)
         result['channel_attribution'] = att.tolist()
+    if MC_DROPOUT_SAMPLES > 0:
+        result['uncertainty'] = trainer.mc_dropout_uncertainty(test_loader, samples=MC_DROPOUT_SAMPLES)
     return result
 
 
@@ -204,6 +207,21 @@ def write_attribution_summary(run_output_dir, results):
     return path
 
 
+def write_uncertainty_summary(run_output_dir, results):
+    """Mean +- std over the folds of each number of the folds' ``Trainer.mc_dropout_uncertainty``; a NaN (an AUROC of a
+    fold without errors) is left out of its mean and counted."""
+    keys = [k for k in results[0]['uncertainty'] if k not in ('windows', 'samples')]
+    path = Path(run_output_dir) / 'uncertainty_summary.txt'
+    with open(path, 'w', encoding='utf-8') as f:
+        f.write(f"# MC dropout, {MC_DROPOUT_SAMPLES} samples per window; {len(results)} folds; mean +- std over the folds\n")
+        for k in keys:
+            v = np.array([r['uncertainty'][k] for r in results], dtype=np.float64)
+            ok = v[~np.isnan(v)]
+            line = f"{k}\t{ok.mean():.4f} ± {ok.std():.4f}" if ok.size else f"{k}\tnan"
+            f.write(line + (f"\t({v.size - ok.size} folds NaN)" if ok.size < v.size else "") + "\n")
+    return path
+
+
 def gather_results(local_results, world):
     """Collect the per-fold results of every rank on all ranks, ordered by subject (ALL_SUBJECTS)."""
     if world > 1:
@@ -248,6 +266,8 @@ def run_simple_experiment(run_output_dir, device, all_channel_names, subject_str
         write_summary(run_output_dir, results)
         if ATTRIBUTION_STEPS > 0:
             write_attribution_summary(run_output_dir, results)
+        if MC_DROPOUT_SAMPLES > 0:
+            write_uncertainty_summary(run_output_dir, results)
     return results
 
 

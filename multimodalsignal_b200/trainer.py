@@ -944,6 +944,56 @@ class Trainer:
                 f.write(name + "".join(f"\t{out[k, c].item():.6f}" for k in range(nc)) + "\n")
         return out
 
+    def mc_dropout_uncertainty(self, data_loader, samples=32, max_rows=2048):
+        """How sure the model is, window by window: MC dropout (``uncertainty.mc_dropout``, BatchNorm in eval mode,
+        ``samples`` dropout samples) over every window of ``data_loader``, as one call with the explicit seed
+        ``model._rng_seed``, so the result does not depend on how the loader batches the windows.  Returns a dict: the
+        accuracy and weighted F1 of the MC prediction; the mean entropy and mutual information over all, correctly
+        classified and misclassified windows (NaN for an empty group); the AUROC of each as a detector of misclassified
+        windows (NaN without errors or without correct windows); the ECE of the MC mean and of the plain eval softmax.
+        Also writes ``uncertainty.txt`` in the fold directory."""
+        from .uncertainty import auroc, expected_calibration_error, mc_dropout
+        m = self.model
+        nc = m.num_classes
+        was_training = m.training
+        m.eval()
+        try:
+            with self._on_stream():
+                xs, ys = [], []
+                for batch in data_loader:
+                    xs.append(batch[0].to(self.device, non_blocking=True).float())
+                    ys.append(batch[1].to(self.device, non_blocking=True).long())
+                if not xs:
+                    raise ValueError("mc_dropout_uncertainty: the loader holds no windows")
+                x, y = torch.cat(xs), torch.cat(ys)
+                res = mc_dropout(m, x, samples=samples, seed=m._rng_seed, max_rows=max_rows)
+                with torch.no_grad():
+                    eval_probs = torch.cat([torch.softmax(m(x[i:i + max_rows]).double(), dim=1)
+                                            for i in range(0, x.shape[0], max_rows)])
+                out = [t.cpu().numpy() for t in (res.probs, res.entropy, res.mutual_info, res.prediction, y, eval_probs)]
+        finally:
+            m.train(was_training)
+        probs, ent, mi, pred, labels, eval_probs = out
+        conf = np.zeros((nc, nc), dtype=np.int64)
+        np.add.at(conf, (labels, pred), 1)
+        acc, f1 = metrics_from_confusion(conf)
+        wrong = pred != labels
+        mean = lambda v: float(v.mean()) if v.size else float("nan")
+        result = {
+            'windows': int(labels.size), 'samples': int(samples), 'accuracy': acc, 'f1_score': f1,
+            'mean_entropy': mean(ent), 'mean_entropy_correct': mean(ent[~wrong]), 'mean_entropy_wrong': mean(ent[wrong]),
+            'mean_mutual_info': mean(mi), 'mean_mutual_info_correct': mean(mi[~wrong]),
+            'mean_mutual_info_wrong': mean(mi[wrong]),
+            'auroc_entropy': auroc(ent, wrong), 'auroc_mutual_info': auroc(mi, wrong),
+            'ece_mc': expected_calibration_error(probs, labels), 'ece_eval': expected_calibration_error(eval_probs, labels),
+        }
+        with open(self.fold_dir / 'uncertainty.txt', 'w', encoding='utf-8') as f:
+            f.write(f"# MC dropout, {samples} samples per window, BatchNorm on running statistics, p = {m.dropout_p}\n")
+            f.write("# AUROC: entropy / mutual information as a detector of misclassified windows; ECE: 10 equal-width bins\n")
+            for k, v in result.items():
+                f.write(f"{k}\t{v:.6f}\n" if isinstance(v, float) else f"{k}\t{v}\n")
+        return result
+
     def finish_test(self, loss, acc, f1, all_preds, all_labels):
         """The is_test tail of reference trainer.py:231-240: confusion-matrix plot + the two log lines."""
         self.plot_confusion_matrix(all_labels, all_preds, filename="test_confusion_matrix.png")
