@@ -106,6 +106,11 @@ typedef struct {
     int64_t* adam_steps;      /* device int64 step counters indexed by the ranges' step slots.  NULL (with no
                                  table): Adam over the whole buffer with step_dev as the count of every element    */
     int32_t adam_nranges;     /* rows of adam_ranges_host, 0..MMS_MAX_ADAM_RANGES (0: no tensor trains)          */
+    const float* clip_max_norm; /* device float32 scalar: mms_cnngru_train_step clips the gradient to this total norm
+                                   before Adam (torch.nn.utils.clip_grad_norm_, see "Gradient-norm clipping" below).
+                                   NULL: no clipping, and the next two fields are ignored                             */
+    double* clip_record;      /* device float64 [5] added to by every clipped step (may be NULL), see mms_grad_norm     */
+    void* clip_scratch;       /* device, MMS_GRAD_CLIP_SCRATCH_BYTES, zero-initialised: the step's norm and coefficient */
 } mms_cnngru_desc;
 
 /* Flat parameter buffer.  The model's parameters live in ONE float32 buffer so that Adam and
@@ -262,6 +267,31 @@ int mms_peer_allreduce_adam_ranges(float* params, const void* const* grads_host,
                                    float beta1, float beta2, float eps, float weight_decay, int64_t* step_dev,
                                    uint32_t* epoch_dev, uint32_t* scratch2_dev, mms_stream_t stream);
 
+/* Gradient-norm clipping on the peer path.  mms_peer_grad_norm runs behind this rank's "gradient complete" signal: it
+ * forms the norm of the world's summed gradient, each element summed in rank order with the fp32 additions of
+ * mms_peer_allreduce_adam, so every rank obtains the same norm and coefficient with no further message (record and
+ * clip_scratch as for mms_grad_norm; ranges_host NULL: elements [0, n)).  It uses words [signal_base, signal_base + world)
+ * of every pad and its own epoch counter norm_epoch_dev (local uint32, zero at start): neither may be shared with the Adam
+ * call that follows, which must read the same clip_scratch.  It has no closing barrier: the following Adam call's closing
+ * barrier also tells every rank that the peers have finished this kernel.  Waits are bounded and counted as for the other
+ * peer kernels.
+ * mms_peer_allreduce_adam_clip / _ranges_clip: mms_peer_allreduce_adam / _ranges on coef_dev[0] * the summed gradient
+ * (coef_dev = (float*)clip_scratch + 1). */
+int mms_peer_grad_norm(const void* const* grads_host, void* const* signals_host, int32_t world, int32_t rank,
+                       int32_t signal_base, int64_t n, const int64_t* ranges_host, int32_t nranges, const float* max_norm,
+                       double* record, void* clip_scratch, uint32_t* norm_epoch_dev, mms_stream_t stream);
+int mms_peer_allreduce_adam_clip(float* params, const void* const* grads_host, void* const* signals_host, int32_t world,
+                                 int32_t rank, int32_t signal_base, float* exp_avg, float* exp_avg_sq, int64_t n,
+                                 const float* lr_dev, float beta1, float beta2, float eps, float weight_decay,
+                                 int64_t* step_dev, uint32_t* epoch_dev, uint32_t* scratch2_dev, const float* coef_dev,
+                                 mms_stream_t stream);
+int mms_peer_allreduce_adam_ranges_clip(float* params, const void* const* grads_host, void* const* signals_host,
+                                        int32_t world, int32_t rank, int32_t signal_base, float* exp_avg, float* exp_avg_sq,
+                                        const int64_t* ranges_host, int32_t nranges, int64_t* steps_dev,
+                                        const float* lr_dev, float beta1, float beta2, float eps, float weight_decay,
+                                        int64_t* step_dev, uint32_t* epoch_dev, uint32_t* scratch2_dev,
+                                        const float* coef_dev, mms_stream_t stream);
+
 /* trainer.py:69,147 CrossEntropyLoss() (mean): loss_out[0] = mean_b(lse - logit[y]),
  * dlogits = (softmax - onehot)/B (NULL to skip).  If loss_sum_accum != NULL it receives
  * += loss * B in float64 (trainer.py:152 accumulates loss.item()*batch_size on the host;
@@ -299,6 +329,34 @@ int mms_adam_ranges_step(float* params, const float* grads, float* exp_avg, floa
                          int32_t nranges, int64_t* steps_dev, const float* lr_dev, float beta1, float beta2, float eps,
                          float weight_decay, int64_t* step_dev, int32_t* scratch_dev, mms_stream_t stream);
 
+/* Gradient-norm clipping, torch.nn.utils.clip_grad_norm_(params, max_norm) with norm_type 2 and error_if_nonfinite=False,
+ * between the backward and Adam:
+ *   total_norm = || the gradient of the trainable elements ||_2,  coef = clamp(max_norm / (total_norm + 1e-6), max = 1),
+ *   and Adam (coupled weight decay) runs on coef * g.
+ * The sum of squares is formed in float64 in a fixed order and rounded once to the fp32 total_norm, so the norm is
+ * bit-reproducible (it differs from torch's per-tensor fp32 norms in the last bits).  For a given fp32 total_norm the
+ * coefficient is torch's bit for bit: reciprocal(total_norm + 1e-6f) * max_norm, a NaN kept by the clamp; a non-finite norm
+ * therefore makes the parameters NaN, as in torch.  The gradient buffer keeps the UNCLIPPED gradient.
+ * clip_scratch (MMS_GRAD_CLIP_SCRATCH_BYTES, zero-initialised, one per concurrently running step): float32 [0] = the last
+ * step's total norm, [1] = its coefficient; the rest is the kernels' own.
+ * record (float64 [5], may be NULL; the caller zeroes it, e.g. per epoch) accumulates: [0] the sum of the finite norms,
+ * [1] their maximum, [2] the steps with coef < 1, [3] the steps with a non-finite norm, [4] the steps.
+ * mms_grad_norm: the norm over the ranges of ranges_host ((offset, count, slot) rows as for mms_adam_ranges_step; the slots
+ *   are ignored) or, with ranges_host == NULL, over grads[0, n).  One launch; max_norm is a device float32 scalar.
+ * mms_adam_flat_clip_step / mms_adam_ranges_clip_step: mms_adam_flat_step / mms_adam_ranges_step on coef_dev[0] * g
+ *   (coef_dev = (float*)clip_scratch + 1 after mms_grad_norm).  With coef 1 the result is theirs bit for bit. */
+#define MMS_GRAD_CLIP_SCRATCH_BYTES 1040
+int mms_grad_norm(const float* grads, int64_t n, const int64_t* ranges_host, int32_t nranges, const float* max_norm,
+                  double* record, void* clip_scratch, mms_stream_t stream);
+int mms_adam_flat_clip_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq,
+                            int64_t n, const float* lr_dev, float beta1, float beta2, float eps,
+                            float weight_decay, int64_t* step_dev, int32_t* scratch_dev, const float* coef_dev,
+                            mms_stream_t stream);
+int mms_adam_ranges_clip_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq,
+                              const int64_t* ranges_host, int32_t nranges, int64_t* steps_dev, const float* lr_dev,
+                              float beta1, float beta2, float eps, float weight_decay, int64_t* step_dev,
+                              int32_t* scratch_dev, const float* coef_dev, mms_stream_t stream);
+
 /* trainer.py:130,140-142 -- one batch of DataLoader(dataset, batch_size, shuffle=True) (main.py:111) assembled on
  * the device: out_x[b, :] = data[perm[cursor + b], :], out_y[b] = labels[perm[cursor + b]] for b < batch.
  * data: float32 [n_rows, row_floats] (the normalised [N, C*W] window array), labels int64 [n_rows], perm: int64
@@ -327,7 +385,8 @@ int mms_eval_accumulate_weighted(const float* logits, const int64_t* labels, int
 
 /* One whole training step, trainer.py:144-149: zero_grad, forward, CE, backward, Adam.
  * (With world_size > 1 the host calls forward/backward/adam separately around its NCCL
- * all-reduce instead.) */
+ * all-reduce instead.)  With d->clip_max_norm set, mms_grad_norm over the trainable elements (the Adam range table, or
+ * every non-empty segment) runs after the backward and the clipped Adam replaces Adam: one launch more. */
 int mms_cnngru_train_step(const mms_cnngru_desc* d, const float* x, const int64_t* labels,
                           float* params, float* grads, float* exp_avg, float* exp_avg_sq,
                           float* bn_buffers, int64_t* num_batches_tracked, void* workspace,

@@ -22,6 +22,7 @@ c_f32 = C.c_float
 
 MAX_SEGMENTS = 64
 MAX_ADAM_RANGES = 96
+GRAD_CLIP_SCRATCH_BYTES = 1040
 
 
 class MmsError(RuntimeError):
@@ -36,6 +37,7 @@ class CnnGruDesc(C.Structure):
         ("rng_seed", c_u64), ("rng_offset", c_u64), ("rng_offset_dev", C.c_void_p),
         ("global_batch", c_i32), ("class_weight", C.c_void_p),
         ("frozen_segments", c_u64), ("adam_ranges_host", C.c_void_p), ("adam_steps", C.c_void_p), ("adam_nranges", c_i32),
+        ("clip_max_norm", C.c_void_p), ("clip_record", C.c_void_p), ("clip_scratch", C.c_void_p),
     ]
 
 
@@ -111,6 +113,13 @@ _SIGNATURES = {
                                                P, P]),
     "mms_adam_flat_step": (c_i32, [P, P, P, P, c_i64, P, c_f32, c_f32, c_f32, c_f32, P, P, P]),
     "mms_adam_ranges_step": (c_i32, [P, P, P, P, P, c_i32, P, P, c_f32, c_f32, c_f32, c_f32, P, P, P]),
+    "mms_grad_norm": (c_i32, [P, c_i64, P, c_i32, P, P, P, P]),
+    "mms_adam_flat_clip_step": (c_i32, [P, P, P, P, c_i64, P, c_f32, c_f32, c_f32, c_f32, P, P, P, P]),
+    "mms_adam_ranges_clip_step": (c_i32, [P, P, P, P, P, c_i32, P, P, c_f32, c_f32, c_f32, c_f32, P, P, P, P]),
+    "mms_peer_grad_norm": (c_i32, [P, P, c_i32, c_i32, c_i32, c_i64, P, c_i32, P, P, P, P, P]),
+    "mms_peer_allreduce_adam_clip": (c_i32, [P, P, P, c_i32, c_i32, c_i32, P, P, c_i64, P, c_f32, c_f32, c_f32, c_f32, P, P, P, P, P]),
+    "mms_peer_allreduce_adam_ranges_clip": (c_i32, [P, P, P, c_i32, c_i32, c_i32, P, P, P, c_i32, P, P, c_f32, c_f32, c_f32, c_f32,
+                                                    P, P, P, P, P]),
     "mms_cnngru_train_step": (c_i32, [C.POINTER(CnnGruDesc), P, P, P, P, P, P, P, P, P, P, P, P, P,
                                       c_f32, c_f32, c_f32, c_f32, P, P, P]),
     "mms_batch_gather": (c_i32, [P, P, P, P, c_i64, c_i64, c_i32, P, P, c_i32, P, P]),

@@ -22,7 +22,7 @@ int cuda_fail(cudaError_t e, const char* what, const char* file, int line) {
 
 using namespace mms;
 
-extern "C" int mms_version(void) { return 103; }
+extern "C" int mms_version(void) { return 104; }
 
 extern "C" const char* mms_last_error(void) { return g_error; }
 

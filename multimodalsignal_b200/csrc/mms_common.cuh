@@ -231,6 +231,87 @@ __device__ __forceinline__ float adam_update(float pi, float gsum, float& mi, fl
     return pi - c.step_size * (mi / (sqrtf(vi) / c.bc2_sqrt + eps));
 }
 
+// ---- gradient-norm clipping (torch.nn.utils.clip_grad_norm_, norm_type 2; grad_clip.cu, peer.cu) ----------------------
+// The norm kernels stride over the virtual index space of an AdamRanges table (the ranges laid end to end, as in
+// adam_ranges_kernel), so the element -> thread map, and with it the float64 sum, depends only on the concatenated ranges and
+// the grid size, which grad_norm_blocks fixes from the element count: the norm is bit-reproducible, and the same whether the
+// trainable elements are listed per segment or per tensor.  Each CTA writes one float64 partial; the last CTA to arrive adds
+// them in CTA order.
+constexpr int GRAD_NORM_MAX_CTAS = 128;
+struct ClipScratch {                       // mms_cnngru_desc.clip_scratch, MMS_GRAD_CLIP_SCRATCH_BYTES, zero-initialised
+    float norm;                            // this step's total norm before clipping (fp32)
+    float coef;                            // clamp(max_norm / (norm + 1e-6), max = 1), what the clipped Adam multiplies by
+    uint32_t arrived;                      // CTAs done (the last one resets it)
+    uint32_t pad;
+    double partial[GRAD_NORM_MAX_CTAS];
+};
+static_assert(sizeof(ClipScratch) == MMS_GRAD_CLIP_SCRATCH_BYTES, "ClipScratch layout");
+
+static inline int grad_norm_blocks(int64_t n) {
+    const int64_t b = (n + 1023) / 1024;
+    return (int)(b < 1 ? 1 : (b > GRAD_NORM_MAX_CTAS ? GRAD_NORM_MAX_CTAS : b));
+}
+
+// torch's coefficient bit for bit: max_norm / t is Tensor.__rtruediv__ = t.reciprocal() * max_norm, and torch.clamp(max=1)
+// keeps a NaN (fminf would not)
+__device__ __forceinline__ float clip_coef(float norm, float max_norm) {
+    const float c = __fmul_rn(__frcp_rn(__fadd_rn(norm, 1e-6f)), max_norm);
+    return c > 1.f ? 1.f : c;
+}
+
+// Block-reduces `sumsq` (every thread of the CTA calls it), publishes the CTA's partial and, in the last CTA to arrive,
+// writes the norm and the coefficient and adds this step to the record: [0] sum of the finite norms, [1] their maximum,
+// [2] steps with coef < 1, [3] steps with a non-finite norm, [4] steps.  No CTA waits for another.  True in the one thread
+// that finished the step.
+__device__ __forceinline__ bool grad_norm_finish(double sumsq, ClipScratch* cs, const float* __restrict__ max_norm_dev,
+                                                 double* record) {
+    __shared__ double s_w[32];
+    sumsq = warp_sum(sumsq);
+    if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = sumsq;
+    __syncthreads();
+    if (threadIdx.x != 0) return false;
+    double s = 0.0;
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += s_w[w];
+    cs->partial[blockIdx.x] = s;
+    __threadfence();
+    if (atomicAdd(&cs->arrived, 1u) != gridDim.x - 1) return false;
+    __threadfence();
+    const volatile double* part = cs->partial;
+    double total = 0.0;
+    for (int b = 0; b < (int)gridDim.x; ++b) total += part[b];
+    const float norm = (float)sqrt(total);
+    const float coef = clip_coef(norm, *max_norm_dev);
+    cs->norm = norm;
+    cs->coef = coef;
+    cs->arrived = 0u;
+    if (record) {
+        if (isfinite(norm)) {
+            record[0] += (double)norm;
+            record[1] = fmax(record[1], (double)norm);
+        } else {
+            record[3] += 1.0;
+        }
+        if (coef < 1.f) record[2] += 1.0;
+        record[4] += 1.0;
+    }
+    return true;
+}
+
+// adam_update with the gradient scaled first: torch clips p.grad in place, and Adam adds wd * p to the ROUNDED product
+// (__fmul_rn is never contracted into the FMA that follows).  coef == 1 gives adam_update's result bit for bit.
+__device__ __forceinline__ void adam_update_clipped(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
+                                                    float* __restrict__ v, int64_t i, float coef, const AdamCoef c, float beta1,
+                                                    float beta2, float eps, float wd) {
+    const float pi = p[i];
+    const float gi = __fmul_rn(g[i], coef) + wd * pi;
+    const float mi = beta1 * m[i] + (1.f - beta1) * gi;
+    const float vi = beta2 * v[i] + (1.f - beta2) * gi * gi;
+    m[i] = mi;
+    v[i] = vi;
+    const float denom = sqrtf(vi) / c.bc2_sqrt + eps;
+    p[i] = pi - c.step_size * (mi / denom);
+}
+
 #endif  // __CUDACC__
 
 }  // namespace mms

@@ -44,6 +44,11 @@ int launch_adam(float*, const float*, float*, float*, int64_t, const float*, flo
                 cudaStream_t);
 int launch_adam_ranges(float*, const float*, float*, float*, const AdamRanges&, int64_t*, const float*, float, float, float, float,
                        int64_t*, int32_t*, cudaStream_t);
+int launch_grad_norm(const float*, const AdamRanges&, const float*, double*, void*, cudaStream_t);
+int launch_adam_clip(float*, const float*, float*, float*, int64_t, const float*, float, float, float, float, int64_t*, int32_t*,
+                     const float*, cudaStream_t);
+int launch_adam_ranges_clip(float*, const float*, float*, float*, const AdamRanges&, int64_t*, const float*, float, float, float,
+                            float, int64_t*, int32_t*, const float*, cudaStream_t);
 int launch_chan_dx(const float*, const float*, const float*, int, int, int, float*, cudaStream_t);
 bool conv_fused_supported(const float*, int, int, int);
 bool conv_bwd_supported(const float*, int, int, int);
@@ -1475,6 +1480,28 @@ extern "C" int mms_cnngru_train_step(const mms_cnngru_desc* d, const float* x, c
     }
     rc = model_backward(d, x, params, bn_buffers, workspace, w.dlogits, grads, nullptr, st, 7, fuse_head, zero_bwd);        // trainer.py:148
     if (rc) return rc;
+    if (d->clip_max_norm) {
+        // clip_grad_norm_ over the trainable elements: the Adam ranges, or every non-empty segment (never the padding between them)
+        AdamRanges nr;
+        if (by_range) {
+            nr = ranges;
+        } else {
+            nr.n = 0;
+            for (int sg = 0; sg < po.nseg; ++sg)
+                if (po.size[sg] > 0) {
+                    nr.off[nr.n] = po.off[sg]; nr.cnt[nr.n] = po.size[sg]; nr.slot[nr.n] = 0;
+                    ++nr.n;
+                }
+        }
+        rc = launch_grad_norm(grads, nr, d->clip_max_norm, d->clip_record, d->clip_scratch, st);
+        if (rc) return rc;
+        const float* coef = reinterpret_cast<const float*>(d->clip_scratch) + 1;
+        if (by_range)
+            return launch_adam_ranges_clip(params, grads, exp_avg, exp_avg_sq, ranges, d->adam_steps, lr_dev, beta1, beta2, eps,
+                                           weight_decay, step_dev, scratch_dev, coef, st);
+        return launch_adam_clip(params, grads, exp_avg, exp_avg_sq, po.total, lr_dev, beta1, beta2, eps, weight_decay, step_dev,
+                                scratch_dev, coef, st);
+    }
     if (by_range)
         return launch_adam_ranges(params, grads, exp_avg, exp_avg_sq, ranges, d->adam_steps, lr_dev, beta1, beta2, eps, weight_decay,
                                   step_dev, scratch_dev, st);

@@ -118,14 +118,17 @@ __global__ void __launch_bounds__(256) peer_allreduce_f64_kernel(const PeerPtrs 
 // the same launch, so nothing depends on co-residency); the last CTA to finish runs the closing barrier.
 // RANGES: only the elements of `r` are summed and updated, range k with its own step count steps[r.slot[k]] (see
 // adam_ranges_kernel); otherwise the whole buffer with *step_dev.
-template <bool RANGES>
+// CLIP: the summed gradient is scaled by *coef_dev (mms_peer_grad_norm) before the update, rounded before + wd * p.
+template <bool RANGES, bool CLIP = false>
 __device__ __forceinline__ void peer_adam_body(float* __restrict__ p, const PeerPtrs& pp, float* __restrict__ m, float* __restrict__ v,
                                                int64_t n, const AdamRanges* r, int64_t* steps, const float* __restrict__ lr_dev,
                                                float beta1, float beta2, float eps, float wd, int64_t* step_dev, int world, int rank,
-                                               int base, uint32_t* epoch_dev, uint32_t* done_dev, uint64_t timeout_ns) {
+                                               int base, uint32_t* epoch_dev, uint32_t* done_dev, uint64_t timeout_ns,
+                                               const float* __restrict__ coef_dev = nullptr) {
     const int tid = threadIdx.x;
     const uint32_t e = *epoch_dev + 1;
     const float lr = *lr_dev;
+    const float coef = CLIP ? *coef_dev : 1.f;
     __shared__ AdamCoef s_c[RANGES ? MMS_MAX_ADAM_RANGES : 1];
     if (RANGES)
         for (int k = tid; k < r->n; k += blockDim.x) s_c[k] = adam_coef(steps[r->slot[k]], lr, beta1, beta2);
@@ -144,6 +147,7 @@ __device__ __forceinline__ void peer_adam_body(float* __restrict__ p, const Peer
                 const int64_t i = r->off[k] + j;
                 float g = 0.f;
                 for (int q = 0; q < world; ++q) g += ld_relaxed_sys_f(reinterpret_cast<const float*>(pp.buf[q]) + i);
+                if (CLIP) g = __fmul_rn(g, coef);
                 float mi = m[i], vi = v[i];
                 p[i] = adam_update(p[i], g, mi, vi, ck, beta1, beta2, eps, wd);
                 m[i] = mi;
@@ -159,6 +163,7 @@ __device__ __forceinline__ void peer_adam_body(float* __restrict__ p, const Peer
                 const float4 x = ld_relaxed_sys_f4(reinterpret_cast<const float*>(pp.buf[q]) + 4 * i4);
                 g.x += x.x; g.y += x.y; g.z += x.z; g.w += x.w;
             }
+            if (CLIP) { g.x = __fmul_rn(g.x, coef); g.y = __fmul_rn(g.y, coef); g.z = __fmul_rn(g.z, coef); g.w = __fmul_rn(g.w, coef); }
             float4 pv = reinterpret_cast<float4*>(p)[i4], mv = reinterpret_cast<float4*>(m)[i4], vv = reinterpret_cast<float4*>(v)[i4];
             float* gp = &g.x; float* pq = &pv.x; float* mq = &mv.x; float* vq = &vv.x;
 #pragma unroll
@@ -171,6 +176,7 @@ __device__ __forceinline__ void peer_adam_body(float* __restrict__ p, const Peer
             for (int64_t i = (n4 << 2) + tid; i < n; i += blockDim.x) {
                 float g = 0.f;
                 for (int q = 0; q < world; ++q) g += ld_relaxed_sys_f(reinterpret_cast<const float*>(pp.buf[q]) + i);
+                if (CLIP) g = __fmul_rn(g, coef);
                 p[i] = adam_update(p[i], g, m[i], v[i], c, beta1, beta2, eps, wd);
             }
         }
@@ -214,6 +220,59 @@ __global__ void __launch_bounds__(256) peer_allreduce_adam_ranges_kernel(float* 
                                                                          uint64_t timeout_ns) {
     peer_adam_body<true>(p, pp, m, v, 0, &r, steps, lr_dev, beta1, beta2, eps, wd, step_dev, world, rank, base, epoch_dev, done_dev,
                          timeout_ns);
+}
+
+__global__ void __launch_bounds__(256) peer_allreduce_adam_clip_kernel(float* __restrict__ p, const PeerPtrs pp, float* __restrict__ m,
+                                                                       float* __restrict__ v, int64_t n, const float* __restrict__ lr_dev,
+                                                                       float beta1, float beta2, float eps, float wd, int64_t* step_dev,
+                                                                       int world, int rank, int base, uint32_t* epoch_dev,
+                                                                       uint32_t* done_dev, uint64_t timeout_ns,
+                                                                       const float* __restrict__ coef_dev) {
+    peer_adam_body<false, true>(p, pp, m, v, n, nullptr, nullptr, lr_dev, beta1, beta2, eps, wd, step_dev, world, rank, base, epoch_dev,
+                                done_dev, timeout_ns, coef_dev);
+}
+
+__global__ void __launch_bounds__(256) peer_allreduce_adam_ranges_clip_kernel(float* __restrict__ p, const PeerPtrs pp,
+                                                                              float* __restrict__ m, float* __restrict__ v,
+                                                                              const __grid_constant__ AdamRanges r, int64_t* steps,
+                                                                              const float* __restrict__ lr_dev, float beta1, float beta2,
+                                                                              float eps, float wd, int64_t* step_dev, int world, int rank,
+                                                                              int base, uint32_t* epoch_dev, uint32_t* done_dev,
+                                                                              uint64_t timeout_ns, const float* __restrict__ coef_dev) {
+    peer_adam_body<true, true>(p, pp, m, v, 0, &r, steps, lr_dev, beta1, beta2, eps, wd, step_dev, world, rank, base, epoch_dev,
+                               done_dev, timeout_ns, coef_dev);
+}
+
+// The norm of the world's summed gradient over the virtual index space of `r` (grad_norm_kernel, grad_clip.cu), every element
+// summed over the ranks in rank order with the fp32 additions of peer_adam_body, so that every rank forms the same norm and
+// coefficient.  CTA 0 signals "this rank's gradient is complete" on words [base, base + world) with its own epoch; every CTA
+// waits for the peers on the rank's own pad.  No closing barrier: the clipped Adam kernel that follows signals again and ends
+// with the barrier after which the gradient buffers may be overwritten.
+__global__ void __launch_bounds__(256) peer_grad_norm_kernel(const PeerPtrs pp, int world, int rank, int base,
+                                                             const __grid_constant__ AdamRanges r, const float* __restrict__ max_norm_dev,
+                                                             double* record, ClipScratch* cs, uint32_t* epoch_dev, uint64_t timeout_ns) {
+    const int tid = threadIdx.x;
+    const uint32_t e = *epoch_dev + 1;
+    if (blockIdx.x == 0) peer_signal(pp, world, rank, base, e, tid);
+    peer_wait(pp, world, rank, base, e, tid, timeout_ns);
+    __syncthreads();
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x, gt = (int64_t)blockIdx.x * blockDim.x + tid;
+    double s = 0.0;
+    int64_t vbase = 0;
+    for (int k = 0; k < r.n; ++k) {
+        int64_t j = (gt - vbase) % stride;
+        if (j < 0) j += stride;
+        for (; j < r.cnt[k]; j += stride) {
+            const int64_t i = r.off[k] + j;
+            float g = 0.f;
+            for (int q = 0; q < world; ++q) g += ld_relaxed_sys_f(reinterpret_cast<const float*>(pp.buf[q]) + i);
+            const double x = (double)g;
+            s += x * x;
+        }
+        vbase += r.cnt[k];
+    }
+    // the last CTA to arrive advances the epoch: every CTA read it before it arrived
+    if (grad_norm_finish(s, cs, max_norm_dev, record)) *epoch_dev = e;
 }
 
 static int fill_peer(PeerPtrs* pp, const void* const* bufs_host, void* const* signals_host, int world) {
@@ -309,5 +368,88 @@ extern "C" int mms_peer_allreduce_adam_ranges(float* params, const void* const* 
                                                               weight_decay, step_dev, world, rank, signal_base, epoch_dev,
                                                               scratch2_dev + 1, peer_timeout_ns());
     MMS_LAUNCH_CHECK("peer_allreduce_adam_ranges_kernel");
+    return MMS_OK;
+}
+
+namespace mms {
+int clip_ranges_from_host(const int64_t* ranges_host, int32_t nranges, int64_t n, AdamRanges* r);     // grad_clip.cu
+}
+
+extern "C" int mms_peer_grad_norm(const void* const* grads_host, void* const* signals_host, int32_t world, int32_t rank,
+                                  int32_t signal_base, int64_t n, const int64_t* ranges_host, int32_t nranges, const float* max_norm,
+                                  double* record, void* clip_scratch, uint32_t* norm_epoch_dev, mms_stream_t stream) {
+    MMS_REQUIRE(grads_host && signals_host && max_norm && clip_scratch && norm_epoch_dev && rank >= 0 && rank < world && signal_base >= 0,
+                "peer_grad_norm: bad arguments");
+    MMS_REQUIRE((reinterpret_cast<uintptr_t>(clip_scratch) & 7) == 0, "peer_grad_norm: clip_scratch must be 8-byte aligned");
+    AdamRanges r;
+    int rc = clip_ranges_from_host(ranges_host, nranges, n, &r);
+    if (rc) return rc;
+    PeerPtrs pp;
+    rc = fill_peer(&pp, grads_host, signals_host, world);
+    if (rc) return rc;
+    int64_t cnt = 0;
+    for (int k = 0; k < r.n; ++k) cnt += r.cnt[k];
+    cudaStream_t st = (cudaStream_t)stream;
+    MMS_PROF_BEGIN(st);
+    peer_grad_norm_kernel<<<grad_norm_blocks(cnt), 256, 0, st>>>(pp, world, rank, signal_base, r, max_norm, record,
+                                                                 reinterpret_cast<ClipScratch*>(clip_scratch), norm_epoch_dev,
+                                                                 peer_timeout_ns());
+    MMS_LAUNCH_CHECK("peer_grad_norm_kernel");
+    return MMS_OK;
+}
+
+extern "C" int mms_peer_allreduce_adam_clip(float* params, const void* const* grads_host, void* const* signals_host, int32_t world,
+                                            int32_t rank, int32_t signal_base, float* exp_avg, float* exp_avg_sq, int64_t n,
+                                            const float* lr_dev, float beta1, float beta2, float eps, float weight_decay,
+                                            int64_t* step_dev, uint32_t* epoch_dev, uint32_t* scratch2_dev, const float* coef_dev,
+                                            mms_stream_t stream) {
+    MMS_REQUIRE(params && grads_host && signals_host && exp_avg && exp_avg_sq && lr_dev && step_dev && epoch_dev && scratch2_dev &&
+                    coef_dev && rank >= 0 && rank < world && n > 0 && signal_base >= 0,
+                "peer_allreduce_adam_clip: bad arguments");
+    MMS_REQUIRE(((reinterpret_cast<uintptr_t>(params) | reinterpret_cast<uintptr_t>(exp_avg) | reinterpret_cast<uintptr_t>(exp_avg_sq)) & 15) == 0,
+                "peer_allreduce_adam_clip: buffers must be 16-byte aligned");
+    PeerPtrs pp;
+    int rc = fill_peer(&pp, grads_host, signals_host, world);
+    if (rc) return rc;
+    for (int i = 0; i < world; ++i)
+        MMS_REQUIRE((reinterpret_cast<uintptr_t>(pp.buf[i]) & 15) == 0, "peer_allreduce_adam_clip: gradient buffers must be 16-byte aligned");
+    int blocks = (int)((n / 4 + 255) / 256);
+    if (blocks > 64) blocks = 64;
+    if (blocks < 1) blocks = 1;
+    cudaStream_t st = (cudaStream_t)stream;
+    MMS_PROF_BEGIN(st);
+    peer_allreduce_adam_clip_kernel<<<blocks, 256, 0, st>>>(params, pp, exp_avg, exp_avg_sq, n, lr_dev, beta1, beta2, eps, weight_decay,
+                                                            step_dev, world, rank, signal_base, epoch_dev, scratch2_dev + 1,
+                                                            peer_timeout_ns(), coef_dev);
+    MMS_LAUNCH_CHECK("peer_allreduce_adam_clip_kernel");
+    return MMS_OK;
+}
+
+extern "C" int mms_peer_allreduce_adam_ranges_clip(float* params, const void* const* grads_host, void* const* signals_host, int32_t world,
+                                                   int32_t rank, int32_t signal_base, float* exp_avg, float* exp_avg_sq,
+                                                   const int64_t* ranges_host, int32_t nranges, int64_t* steps_dev, const float* lr_dev,
+                                                   float beta1, float beta2, float eps, float weight_decay, int64_t* step_dev,
+                                                   uint32_t* epoch_dev, uint32_t* scratch2_dev, const float* coef_dev,
+                                                   mms_stream_t stream) {
+    MMS_REQUIRE(params && grads_host && signals_host && exp_avg && exp_avg_sq && steps_dev && lr_dev && step_dev && epoch_dev &&
+                    scratch2_dev && coef_dev && rank >= 0 && rank < world && signal_base >= 0,
+                "peer_allreduce_adam_ranges_clip: bad arguments");
+    AdamRanges r;
+    int rc = adam_ranges_from_host(ranges_host, nranges, INT64_MAX / 2, &r);
+    if (rc) return rc;
+    PeerPtrs pp;
+    rc = fill_peer(&pp, grads_host, signals_host, world);
+    if (rc) return rc;
+    int64_t n = 0;
+    for (int k = 0; k < r.n; ++k) n += r.cnt[k];
+    int blocks = (int)((n + 255) / 256);
+    if (blocks > 64) blocks = 64;
+    if (blocks < 1) blocks = 1;
+    cudaStream_t st = (cudaStream_t)stream;
+    MMS_PROF_BEGIN(st);
+    peer_allreduce_adam_ranges_clip_kernel<<<blocks, 256, 0, st>>>(params, pp, exp_avg, exp_avg_sq, r, steps_dev, lr_dev, beta1, beta2,
+                                                                   eps, weight_decay, step_dev, world, rank, signal_base, epoch_dev,
+                                                                   scratch2_dev + 1, peer_timeout_ns(), coef_dev);
+    MMS_LAUNCH_CHECK("peer_allreduce_adam_ranges_clip_kernel");
     return MMS_OK;
 }

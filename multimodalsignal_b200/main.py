@@ -47,6 +47,7 @@ WEIGHTS_DECAY = 1e-4
 USE_CLASS_WEIGHTS = False                     # class-weighted CrossEntropyLoss, 'balanced' weights (never enabled upstream, SURVEY D9)
 ATTRIBUTION_STEPS = 0                         # > 0: integrated-gradients channel attribution of each fold's test set, this many steps
 MC_DROPOUT_SAMPLES = 0                        # > 0: MC-dropout uncertainty of each fold's test set, this many samples per window
+GRAD_CLIP_NORM = None                         # a number: clip the gradient to this total 2-norm before every Adam step (clip_grad_norm_)
 ALL_SUBJECTS = [f"S{i}" for i in range(2, 18) if i != 12]
 CONCURRENT_FOLDS = int(os.environ.get("MMS_CONCURRENT_FOLDS", "1"))     # folds interleaved per GPU (new; 1 = the reference's loop)
 
@@ -68,7 +69,8 @@ def folds_for_rank(n_folds: int, rank: int, world: int):
 def trainer_config():
     return {'trainer': {'epochs': EPOCHS, 'learning_rate': LEARNING_RATE,
                         'early_stopping': {'enabled': True, 'patience': PATIENCE, 'delta': 0},
-                        'weight_decay': WEIGHTS_DECAY, 'use_class_weights': USE_CLASS_WEIGHTS}}
+                        'weight_decay': WEIGHTS_DECAY, 'use_class_weights': USE_CLASS_WEIGHTS,
+                        'grad_clip_norm': GRAD_CLIP_NORM}}
 
 
 def run_fold_async(fold_index, subject_to_test, run_output_dir, all_channel_names, subject_streams=None, stream=None,

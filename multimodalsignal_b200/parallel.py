@@ -94,6 +94,7 @@ class DataParallelTrainStep:
         opt.grads = grads
         self.signals = self._alloc(256, torch.int32, dev)                   # this rank's signal pad
         self.epoch = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.norm_epoch = torch.zeros(1, dtype=torch.int32, device=dev)      # mms_peer_grad_norm's own epoch (clipping)
         self.scratch2 = torch.zeros(2, dtype=torch.int32, device=dev)
         if self.peer == "symm":
             import torch.distributed as dist
@@ -147,6 +148,26 @@ class DataParallelTrainStep:
         yield
         self._bwd(4, x)
         _, grads, sig = self._peer_tables()
+        if o.max_grad_norm is not None:
+            # clip_grad_norm_ on the summed gradient: every rank forms the same norm from the peers' buffers, on pad words
+            # [2 world, 3 world) with its own epoch (the Adam kernel below uses [0, 2 world) and self.epoch)
+            nt = o.norm_table(self._table)
+            check(self.lib.mms_peer_grad_norm(grads, sig, self.world, self.rank, 2 * self.world, self.flat.numel(), nt, len(nt) // 3,
+                                              ptr(o.clip_max_norm), ptr(o.clip_record), ptr(o.clip_scratch), ptr(self.norm_epoch),
+                                              stream()))
+            yield
+            if self._table is None:
+                check(self.lib.mms_peer_allreduce_adam_clip(ptr(self.flat), grads, sig, self.world, self.rank, 0, ptr(o.exp_avg),
+                                                            ptr(o.exp_avg_sq), self.flat.numel(), ptr(o.lr_dev), g['betas'][0],
+                                                            g['betas'][1], g['eps'], g['weight_decay'], ptr(o.step_dev), ptr(self.epoch),
+                                                            ptr(self.scratch2), ptr(o.clip_coef), stream()))
+            else:
+                check(self.lib.mms_peer_allreduce_adam_ranges_clip(ptr(self.flat), grads, sig, self.world, self.rank, 0, ptr(o.exp_avg),
+                                                                   ptr(o.exp_avg_sq), self._table, len(self._table) // 3,
+                                                                   ptr(o.tensor_steps), ptr(o.lr_dev), g['betas'][0], g['betas'][1],
+                                                                   g['eps'], g['weight_decay'], ptr(o.step_dev), ptr(self.epoch),
+                                                                   ptr(self.scratch2), ptr(o.clip_coef), stream()))
+            return
         if self._table is None:
             check(self.lib.mms_peer_allreduce_adam(ptr(self.flat), grads, sig, self.world, self.rank, 0, ptr(o.exp_avg), ptr(o.exp_avg_sq),
                                                    self.flat.numel(), ptr(o.lr_dev), g['betas'][0], g['betas'][1], g['eps'],
@@ -166,7 +187,7 @@ class DataParallelTrainStep:
         mask, table = self.opt.plan()
         self.desc.frozen_segments = mask
         self._table = table
-        return mask, None if table is None else tuple(table)
+        return mask, None if table is None else tuple(table), self.opt.max_grad_norm is not None
 
     def run_peer(self):
         """One step on the static inputs ``self.x`` / ``self.y`` (graph replay after the first call of each freeze plan)."""
@@ -228,7 +249,7 @@ class DataParallelTrainStep:
         yield self.red1
         self._bwd(4, x)
         yield self.opt.grads                                     # ONE flat gradient all-reduce (~0.5 MB)
-        self.opt.flat_step(self.flat)                            # trainer.py:149
+        self.opt.flat_step(self.flat)                            # trainer.py:149 (clips the summed gradient if the optimizer does)
 
     def __call__(self, x, y):
         if self.peer is not None:

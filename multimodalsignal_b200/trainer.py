@@ -10,6 +10,7 @@ device (the reference syncs twice per step through ``loss.item()``, trainer.py:1
 from __future__ import annotations
 
 import contextlib
+import math
 import os
 import ctypes as C
 import threading
@@ -189,6 +190,24 @@ def capture_graph(enqueue):
     return graph
 
 
+def check_max_grad_norm(max_norm, norm_type=2.0):
+    """``max_norm`` as a float, after the checks of the clipping this package implements: ``norm_type`` 2 only
+    (``NotImplementedError`` otherwise), ``max_norm`` finite and > 0 (``ValueError`` otherwise)."""
+    try:
+        nt = float(norm_type)
+    except (TypeError, ValueError):
+        nt = None
+    if nt != 2.0:
+        raise NotImplementedError(f"gradient clipping: only norm_type 2 is implemented, got {norm_type!r}")
+    try:
+        v = float(max_norm)
+    except (TypeError, ValueError):
+        raise ValueError(f"gradient clipping: max_norm must be a number, got {max_norm!r}") from None
+    if not math.isfinite(v) or v <= 0.0:
+        raise ValueError(f"gradient clipping: max_norm must be finite and > 0, got {max_norm!r}")
+    return v
+
+
 class FlatAdam(torch.optim.Optimizer):
     """``torch.optim.Adam(model.parameters(), lr, weight_decay)`` (reference trainer.py:68) over
     the model's flat parameter buffer: one kernel for all 30 tensors.  It is a real
@@ -198,9 +217,18 @@ class FlatAdam(torch.optim.Optimizer):
     Frozen parameters follow torch: a tensor that is not updated (``step()``: no ``.grad``; ``flat_step()`` and the fused
     steps: ``requires_grad`` False) keeps its value, its moments and its step count, and on unfreezing continues from
     them.  The per-tensor step counts (``tensor_steps``) are used from the first step that leaves a tensor out; until then
-    every tensor's count is ``step_dev`` and the single whole-buffer kernel runs."""
+    every tensor's count is ``step_dev`` and the single whole-buffer kernel runs.
 
-    def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0):
+    ``max_grad_norm`` (None: off) clips the gradient before every update, as
+    ``torch.nn.utils.clip_grad_norm_(params, max_grad_norm)`` between ``backward()`` and ``step()`` would: the total 2-norm
+    of the gradient of the tensors being updated, and ``coef = min(max_grad_norm / (norm + 1e-6), 1)`` on the gradient
+    Adam reads (DESIGN.md, gradient-norm clipping).  ``step()``, ``flat_step()``, ``FusedTrainStep`` and the data-parallel
+    steps all clip.  The flat gradient buffer ``grads`` keeps the UNCLIPPED gradient.  ``grad_norm`` is a one-element device
+    tensor holding the last update's norm before clipping; ``clip_record`` (float64 [5], device) adds up, per update, the
+    finite norms, their maximum, the clipped updates (coef < 1), the non-finite norms and the updates -- zero it with
+    ``reset_clip_record()``.  ``set_max_grad_norm`` changes the threshold with a device copy: captured graphs keep working."""
+
+    def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0, max_grad_norm=None, norm_type=2.0):
         params = [p for p in model.parameters()]
         super().__init__(params, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
         self.model = model
@@ -215,6 +243,50 @@ class FlatAdam(torch.optim.Optimizer):
         self._per_tensor = False            # tensor_steps in use (some step has left a tensor out)
         self._tables = {}                   # ranges -> HOST int64 [n][3] table (kept alive for the library)
         self._lr_on_device = float(lr)
+        self.clip_max_norm = torch.zeros(1, dtype=torch.float32, device=flat.device)
+        self.clip_record = torch.zeros(5, dtype=torch.float64, device=flat.device)
+        self.clip_scratch = torch.zeros(_ext.GRAD_CLIP_SCRATCH_BYTES // 4, dtype=torch.float32, device=flat.device)
+        self.grad_norm = self.clip_scratch[0:1]          # written by the norm kernel of every clipped update
+        self.clip_coef = self.clip_scratch[1:2]
+        self.max_grad_norm = None
+        self._norm_tables = {}
+        if max_grad_norm is not None:
+            self.set_max_grad_norm(max_grad_norm, norm_type)
+
+    def set_max_grad_norm(self, max_norm, norm_type=2.0):
+        """Clip to ``max_norm`` from the next update on (None: stop clipping).  A stream-ordered copy to the device value the
+        kernels read, so a captured CUDA graph picks it up without re-capture."""
+        if max_norm is None:
+            self.max_grad_norm = None
+            return
+        v = check_max_grad_norm(max_norm, norm_type)
+        self.clip_max_norm.fill_(v)
+        self.max_grad_norm = v
+
+    def reset_clip_record(self):
+        self.clip_record.zero_()
+
+    @staticmethod
+    def clip_summary(record):
+        """``clip_record`` read back to the host (five numbers) as a dict: mean and max of the finite norms (NaN without
+        one), clipped / non-finite / total update counts."""
+        s, mx, clipped, nonfinite, n = (float(v) for v in record)
+        finite = n - nonfinite
+        return {'mean': s / finite if finite > 0 else float('nan'), 'max': mx if finite > 0 else float('nan'),
+                'clipped': int(clipped), 'nonfinite': int(nonfinite), 'steps': int(n)}
+
+    def norm_table(self, table):
+        """The HOST range table the norm is taken over: the Adam range table of the update (``plan()``), or, when the
+        update covers the whole buffer, one range per non-empty segment -- never the padding between segments.  Both list
+        the same elements in the same order, so the norm has the same bits either way."""
+        if table is not None:
+            return table
+        t = self._norm_tables.get(None)
+        if t is None:
+            offs, sizes, _ = self.model._layout()
+            rows = [(o, n, 0) for o, n in zip(offs, sizes) if n]
+            t = self._norm_tables[None] = (C.c_int64 * (3 * len(rows)))(*[v for r in rows for v in r])
+        return t
 
     def sync_lr(self):
         lr = float(self.param_groups[0]['lr'])
@@ -260,6 +332,20 @@ class FlatAdam(torch.optim.Optimizer):
         self.sync_lr()
         g = self.param_groups[0]
         _, table = self.plan(trainable)
+        if self.max_grad_norm is not None:
+            nt = self.norm_table(table)
+            check(lib.mms_grad_norm(ptr(self.grads), flat.numel(), nt, len(nt) // 3, ptr(self.clip_max_norm), ptr(self.clip_record),
+                                    ptr(self.clip_scratch), stream()))
+            if table is None:
+                check(lib.mms_adam_flat_clip_step(ptr(flat), ptr(self.grads), ptr(self.exp_avg), ptr(self.exp_avg_sq), flat.numel(),
+                                                  ptr(self.lr_dev), g['betas'][0], g['betas'][1], g['eps'], g['weight_decay'],
+                                                  ptr(self.step_dev), ptr(self.scratch), ptr(self.clip_coef), stream()))
+            else:
+                check(lib.mms_adam_ranges_clip_step(ptr(flat), ptr(self.grads), ptr(self.exp_avg), ptr(self.exp_avg_sq), table,
+                                                    len(table) // 3, ptr(self.tensor_steps), ptr(self.lr_dev),
+                                                    g['betas'][0], g['betas'][1], g['eps'], g['weight_decay'], ptr(self.step_dev),
+                                                    ptr(self.scratch), ptr(self.clip_coef), stream()))
+            return
         if table is None:
             check(lib.mms_adam_flat_step(ptr(flat), ptr(self.grads), ptr(self.exp_avg), ptr(self.exp_avg_sq), flat.numel(),
                                          ptr(self.lr_dev), g['betas'][0], g['betas'][1], g['eps'], g['weight_decay'],
@@ -277,6 +363,10 @@ class FlatAdam(torch.optim.Optimizer):
         desc.adam_ranges_host = None if table is None else C.addressof(table)
         desc.adam_steps = None if table is None else self.tensor_steps.data_ptr()
         desc.adam_nranges = 0 if table is None else len(table) // 3
+        clip = self.max_grad_norm is not None
+        desc.clip_max_norm = self.clip_max_norm.data_ptr() if clip else None
+        desc.clip_record = self.clip_record.data_ptr() if clip else None
+        desc.clip_scratch = self.clip_scratch.data_ptr() if clip else None
 
 
 def class_weight_tensor(weight, num_classes, device):
@@ -395,7 +485,7 @@ class FusedTrainStep:
         self.opt.sync_lr()
         self.calls += 1
         mask, table = self.opt.plan()
-        key = (mask, None if table is None else tuple(table))
+        key = (mask, None if table is None else tuple(table), self.opt.max_grad_norm is not None)
         self.opt.set_plan(self.desc, (mask, table))
         if not self.use_graph or key not in self._eager_done:
             self._eager_done.add(key)
@@ -620,6 +710,10 @@ class Trainer:
     of this trainer's work is issued on."""
 
     def __init__(self, model, fold_output_dir: Path, config, stream=None):
+        # refuse a bad clipping setting before anything is written or allocated
+        grad_clip_norm = config['trainer'].get('grad_clip_norm')
+        if grad_clip_norm is not None:
+            grad_clip_norm = check_max_grad_norm(grad_clip_norm)
         self.model, self.fold_dir, self.config = model, Path(fold_output_dir), config
         self.fold_dir.mkdir(parents=True, exist_ok=True)
         self.log_file = self.fold_dir / 'training_log.txt'
@@ -643,13 +737,16 @@ class Trainer:
 
         with self._on_stream():
             self.model.to(self.device)
-            self.optimizer = FlatAdam(self.model, lr=self.learning_rate, weight_decay=self.weight_decay)
+            # gradient-norm clipping (torch.nn.utils.clip_grad_norm_ before every Adam step); None: off
+            self.grad_clip_norm = grad_clip_norm
+            self.optimizer = FlatAdam(self.model, lr=self.learning_rate, weight_decay=self.weight_decay, max_grad_norm=grad_clip_norm)
             nc = model.num_classes
             self._eval_conf = torch.zeros(nc * nc, dtype=torch.int64, device=self.device)
             self._eval_loss = torch.zeros(1, dtype=torch.float64, device=self.device)
             self._train_loss = torch.zeros(1, dtype=torch.float64, device=self.device)
         self._host_conf = torch.zeros(nc * nc, dtype=torch.int64).pin_memory()
         self._host_loss = torch.zeros(2, dtype=torch.float64).pin_memory()       # [0] training sum, [1] evaluation sum
+        self._host_clip = torch.zeros(5, dtype=torch.float64).pin_memory() if grad_clip_norm is not None else None
         self.criterion = CrossEntropyLoss()
         self.scheduler = ReduceLROnPlateau(self.optimizer, mode='min', factor=0.1, patience=3)
         self.early_stopping = None
@@ -758,11 +855,15 @@ class Trainer:
         from .dataset import DeviceBatchLoader
         self.model.train()
         self._train_loss.zero_()
+        if self._host_clip is not None:
+            self.optimizer.reset_clip_record()
         if isinstance(train_loader, DeviceBatchLoader):
             self._train_epoch_device(train_loader)
         else:
             self._train_epoch_host(train_loader)
         self._host_loss[0:1].copy_(self._train_loss, non_blocking=True)
+        if self._host_clip is not None:                  # read back behind the same event as the loss
+            self._host_clip.copy_(self.optimizer.clip_record, non_blocking=True)
         return self._event()
 
     def train(self, train_loader, val_loader):
@@ -801,6 +902,8 @@ class Trainer:
                       f"验证损失: {val_loss:.4f} | "
                       f"验证Acc: {val_acc:.4f} | "
                       f"验证F1: {val_f1:.4f}")
+            if self._host_clip is not None:
+                self._log_clipping()
             stop = False
             if self.early_stopping:
                 with self._on_stream():
@@ -817,6 +920,15 @@ class Trainer:
             with self._on_stream():
                 self.model.load_state_dict(torch.load(self.early_stopping.checkpoint_path, weights_only=True))
         self._log(f"--- 训练完成 --- 总训练时长: {time.time() - self.total_start_time:.2f}秒")
+
+    def _log_clipping(self):
+        """The epoch's gradient-norm line (``grad_clip_norm``), plus a warning when a norm was not finite."""
+        r = FlatAdam.clip_summary(self._host_clip)
+        self._log(f"Gradient norm before clipping: mean {r['mean']:.4f} | max {r['max']:.4f} | "
+                  f"clipped {r['clipped']} of {r['steps']} steps")
+        if r['nonfinite']:
+            self._log(f"Warning: the gradient norm was not finite in {r['nonfinite']} of {r['steps']} steps; "
+                      "clipping such a gradient makes the parameters NaN (as torch's clip_grad_norm_ does)")
 
     def _flush_checkpoints(self):
         writer = getattr(self.model, "_checkpoint_writer", None)

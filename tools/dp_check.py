@@ -1,6 +1,8 @@
 """torchrun entry: real NCCL data-parallel steps (SyncBN + one flat gradient all-reduce) on WORLD_SIZE GPUs
 must equal the single-device full-batch step.  Used by tests/test_gpu_parallel.py (needs >= 2 GPUs) and by hand:
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 tools/dp_check.py
+--peer: the symmetric-memory exchange with the peer kernels; --clip: gradient-norm clipping (FlatAdam max_grad_norm) on
+every rank and on the reference step.
 """
 import os
 import sys
@@ -40,7 +42,8 @@ def main():
     b = B // world
     m = model()
     peer = "symm" if "--peer" in sys.argv else None      # symmetric memory + the peer kernels instead of NCCL all-reduces
-    step = DataParallelTrainStep(m, FlatAdam(m, lr=1e-3, weight_decay=1e-4), b, B, T, rank=rank, peer=peer)
+    clip = 0.05 if "--clip" in sys.argv else None        # well below the gradient norm of this batch: every step clips
+    step = DataParallelTrainStep(m, FlatAdam(m, lr=1e-3, weight_decay=1e-4, max_grad_norm=clip), b, B, T, rank=rank, peer=peer)
     losses = []
     for _ in range(3 if peer is None else 5):      # peer mode: eager step, graph capture, replays
         step(x[rank * b:(rank + 1) * b], y[rank * b:(rank + 1) * b])
@@ -48,13 +51,17 @@ def main():
     ok = True
     if rank == 0:
         ref = model()
-        ref_step = FusedTrainStep(ref, FlatAdam(ref, lr=1e-3, weight_decay=1e-4), B, T, use_graph=False)
+        ref_step = FusedTrainStep(ref, FlatAdam(ref, lr=1e-3, weight_decay=1e-4, max_grad_norm=clip), B, T, use_graph=False)
         ref_losses = []
         for _ in range(len(losses)):
             ref_step(x, y)
             ref_losses.append(ref_step.last_loss())
         np.testing.assert_allclose(losses, ref_losses, atol=2e-5)
-        np.testing.assert_allclose(losses[:3], z["adam_losses"][:3], atol=1e-4)
+        if clip is None:
+            np.testing.assert_allclose(losses[:3], z["adam_losses"][:3], atol=1e-4)
+        else:
+            assert ref_step.opt.clip_coef.item() < 1.0 and step.opt.clip_coef.item() < 1.0
+            np.testing.assert_allclose(step.opt.grad_norm.item(), ref_step.opt.grad_norm.item(), rtol=1e-4)
         ref_sd = ref.state_dict()
         for k, v in m.state_dict().items():
             if v.numel():
