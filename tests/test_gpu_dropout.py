@@ -85,10 +85,10 @@ def test_port_matches_dropout_apply_bit_for_bit(p, base):
 
 
 # ------------------------------------------------------------------------------------------------ b. the whole step
-def _state(C, nc, H, layers, seed):
+def _state(C, nc, H, layers, seed, O=32):
     """Reference-shaped parameters (oracle/cpu_port.make_state) with non-trivial BatchNorm affine values."""
     from oracle import cpu_port
-    p, bufs = cpu_port.make_state(C=C, num_classes=nc, H=H, layers=layers, seed=seed)
+    p, bufs = cpu_port.make_state(C=C, num_classes=nc, cnn_out=O, H=H, layers=layers, seed=seed)
     g = torch.Generator().manual_seed(seed + 100)
     for k in ("cnn_encoder.1", "cnn_encoder.5"):
         p[f"{k}.weight"] = p[f"{k}.weight"] + 0.1 * torch.randn(p[f"{k}.weight"].shape, generator=g)
@@ -96,9 +96,10 @@ def _state(C, nc, H, layers, seed):
     return p, bufs
 
 
-def _model(p, bufs, C, nc, H, layers, dropout):
+def _model(p, bufs, C, nc, H, layers, dropout, O=32, attention=True):
     from multimodalsignal_b200.models import CnnGruAttentionModel
-    m = CnnGruAttentionModel(C, nc, gru_hidden_size=H, gru_num_layers=layers, dropout=dropout)
+    m = CnnGruAttentionModel(C, nc, cnn_out_channels=O, gru_hidden_size=H, gru_num_layers=layers, dropout=dropout,
+                             attention=attention)
     sd = dict(p)
     sd.update(bufs)
     sd["cnn_encoder.1.num_batches_tracked"] = torch.zeros((), dtype=torch.int64)
@@ -191,44 +192,50 @@ def _run_fused(m, x, y, head_fused):
     return got, int(step.desc.rng_seed), offset
 
 
-# B, C, T, H, layers, p, num_classes, options: the path each reaches (model.cu)
+# B, C, T, O, H, layers, p, num_classes, options: the path each reaches (model.cu)
 STEP_CASES = {
     # M = 320 < TC_MIN_ROWS: separate dropout pass, SIMT products, forward skinny product on the dropped tensor, skinny
     # drop-on-C in the backward, head_fwd2
-    "b8_t640": (8, 6, 640, 64, 2, 0.5, 2, {}),
+    "b8_t640": (8, 6, 640, 32, 64, 2, 0.5, 2, {}),
     # the bench configuration: tcgen05 A-operand dropout (forward), skinny drop-on-A (forward), epilogue dropout (backward)
-    "b64_t3840": (64, 6, 3840, 64, 2, 0.5, 2, {}),
+    "b64_t3840": (64, 6, 3840, 32, 64, 2, 0.5, 2, {}),
     # the same with the fusions off: separate pass, gemm_nn + dropout_rows
-    "b64_t3840_unfused": (64, 6, 3840, 64, 2, 0.5, 2, {"DROP_FUSED": 0, "GEMM_SKINNY": 0}),
+    "b64_t3840_unfused": (64, 6, 3840, 32, 64, 2, 0.5, 2, {"DROP_FUSED": 0, "GEMM_SKINNY": 0}),
     # H = 128: N = 384 split into tiles
-    "b16_h128": (16, 6, 3840, 128, 2, 0.5, 2, {}),
+    "b16_h128": (16, 6, 3840, 32, 128, 2, 0.5, 2, {}),
     # H = 32, 3 classes, p = 0.2
-    "b16_h32_c3": (16, 8, 3840, 32, 2, 0.2, 3, {}),
+    "b16_h32_c3": (16, 8, 3840, 32, 32, 2, 0.2, 3, {}),
     # two sites: layer 0 by a separate pass, layer 1 on the A operand
-    "b8_l3": (8, 6, 3840, 64, 3, 0.5, 2, {}),
+    "b8_l3": (8, 6, 3840, 32, 64, 3, 0.5, 2, {}),
     # B > 256: skinny refused -> forward gemm_nt on the dropped tensor, backward gemm_nn + dropout_rows; M = 6321 on tcgen05
-    "b301_t336": (301, 3, 336, 64, 2, 0.5, 2, {}),
+    "b301_t336": (301, 3, 336, 32, 64, 2, 0.5, 2, {}),
     # odd L = 63, p = 0.8 (scale 5)
-    "b5_t1004_p08": (5, 6, 1004, 64, 2, 0.8, 2, {}),
+    "b5_t1004_p08": (5, 6, 1004, 32, 64, 2, 0.8, 2, {}),
     # one layer: the head site only
-    "b8_l1": (8, 6, 640, 64, 1, 0.5, 2, {}),
+    "b8_l1": (8, 6, 640, 32, 64, 1, 0.5, 2, {}),
+    # O = 64 (per-layer BN-folded encoder backward), four GRU sites at offsets l * 2^40 on tcgen05 (M = 3840), 8 classes
+    "b16_o64_l5_c8": (16, 6, 3840, 64, 64, 5, 0.5, 8, {}),
+    # O = 16 at H = 128: bottom-layer weight gradient with N2 = 16 on the SIMT TN product, in tn_split's row halves
+    "b16_o16_h128": (16, 6, 3840, 16, 128, 2, 0.5, 3, {}),
+    # eight layers at M = 320: seven GRU sites on the separate pass and the SIMT products
+    "b8_t640_l8": (8, 6, 640, 32, 64, 8, 0.5, 2, {}),
 }
 
 
 @pytest.mark.parametrize("case", list(STEP_CASES))
 def test_dropout_step_vs_float64_oracle_with_drawn_masks(case):
     from multimodalsignal_b200.synth import synthetic_windows
-    B, C, T, H, layers, p, nc, opts = STEP_CASES[case]
-    params, bufs = _state(C, nc, H, layers, seed=20 + C + H)
+    B, C, T, O, H, layers, p, nc, opts = STEP_CASES[case]
+    params, bufs = _state(C, nc, H, layers, seed=20 + C + H, O=O)
     x, y = synthetic_windows(B, C, T, seed=7 + B, num_classes=nc)
     xt, yt = torch.from_numpy(x), torch.from_numpy(y)
     p64 = {k: v.double() for k, v in params.items()}
     runs = []
     with _options(opts):
-        runs.append(("autograd",) + _run_autograd(_model(params, bufs, C, nc, H, layers, p), xt.cuda(), yt.cuda()))
+        runs.append(("autograd",) + _run_autograd(_model(params, bufs, C, nc, H, layers, p, O=O), xt.cuda(), yt.cuda()))
         for head_fused in (1, 0):
             runs.append((f"fused_step/HEAD_FUSED={head_fused}",)
-                        + _run_fused(_model(params, bufs, C, nc, H, layers, p), xt.cuda(), yt.cuda(), head_fused))
+                        + _run_fused(_model(params, bufs, C, nc, H, layers, p, O=O), xt.cuda(), yt.cuda(), head_fused))
     assert len({(seed, off) for _, _, seed, off in runs}) == len(runs)      # three different streams
     for name, got, seed, offset in runs:
         masks = _masks(B, T, H, layers, p, seed, offset)
@@ -244,7 +251,7 @@ def test_wrong_masks_are_caught():
     tolerance of the oracle run with the masks of the next offset, with the layer mask's direction halves swapped, and
     without the head mask."""
     from multimodalsignal_b200.synth import synthetic_windows
-    B, C, T, H, layers, p, nc, _ = STEP_CASES["b64_t3840"]
+    B, C, T, _, H, layers, p, nc, _ = STEP_CASES["b64_t3840"]
     params, bufs = _state(C, nc, H, layers, seed=20 + C + H)
     x, y = synthetic_windows(B, C, T, seed=7 + B, num_classes=nc)
     xt, yt = torch.from_numpy(x), torch.from_numpy(y)

@@ -18,13 +18,14 @@ pytestmark = pytest.mark.gpu
 LOGIT_ATOL = 1e-4
 
 
-def make_model(C_, nc=2, H=64, layers=2, attention=True, seed=0, p=0.5):
+def make_model(C_, nc=2, H=64, layers=2, attention=True, seed=0, p=0.5, O=32):
     """Random weights and random BatchNorm running statistics / affine parameters (eval BatchNorm is a non-trivial map)."""
     from multimodalsignal_b200.models import CnnGruAttentionModel
     torch.manual_seed(seed)
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        m = CnnGruAttentionModel(C_, nc, gru_hidden_size=H, gru_num_layers=layers, dropout=p, attention=attention)
+        m = CnnGruAttentionModel(C_, nc, cnn_out_channels=O, gru_hidden_size=H, gru_num_layers=layers, dropout=p,
+                                 attention=attention)
     g = torch.Generator().manual_seed(seed + 1000)
     with torch.no_grad():
         for bn in (m.cnn_encoder[1], m.cnn_encoder[5]):
@@ -94,10 +95,25 @@ CASES = [  # B, C, T, H, layers, nc, attention, samples
     (64, 6, 3840, 128, 2, 2, True, 32),
 ]
 
+# cnn_out_channels O != 32: the per-window encoder workspace and the bottom layer's input projection (K = O)
+CNN_WIDTH_CASES = [  # O, B, C, T, H, layers, nc, attention, samples
+    (16, 8, 6, 3840, 64, 2, 3, True, 16),    # 128 sample rows
+    (64, 6, 6, 3840, 64, 3, 5, True, 8),     # a middle layer on the sample rows
+]
+
 
 @pytest.mark.parametrize("B,C_,T,H,layers,nc,attention,samples", CASES)
 def test_every_sample_matches_oracle(B, C_, T, H, layers, nc, attention, samples):
-    m = make_model(C_, nc=nc, H=H, layers=layers, attention=attention, seed=B + T + H)
+    _check_every_sample(B, C_, T, H, layers, nc, attention, samples)
+
+
+@pytest.mark.parametrize("O,B,C_,T,H,layers,nc,attention,samples", CNN_WIDTH_CASES)
+def test_every_sample_matches_oracle_other_cnn_widths(O, B, C_, T, H, layers, nc, attention, samples):
+    _check_every_sample(B, C_, T, H, layers, nc, attention, samples, O=O)
+
+
+def _check_every_sample(B, C_, T, H, layers, nc, attention, samples, O=32):
+    m = make_model(C_, nc=nc, H=H, layers=layers, attention=attention, seed=B + T + H, O=O)
     x = make_x(B, C_, T, seed=B + layers)
     res = run(m, x, samples)
     assert res.offset == 0 and res.seed == 1234
